@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the nabo cell-projection hot path on B200 (contract: see task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--metric ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--metric ...] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 100 000 target cells mapped onto a 100 000-cell
 reference, 50 PCs, k = 30.  One *step* = one pass of the hot path over one batch of target
@@ -68,7 +68,17 @@ def parse():
                          "whole waves of the persistent candidate kernel; 5 batches = 1.14 M targets)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the modified-Canberra measurement")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work per cpu_baseline sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (neighbour indices and "
+                         "distances, SNN counts and weights, per-reference scores) as DIR/<name>.npy in float32 / "
+                         "float64, at most 64 MB in all: a fixed, seeded sample of target rows when the whole output "
+                         "is larger (DIR/rows.npy lists them).  Default workload only")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "config2" or a.shard != "targets"):
+        ap.error("--dump-outputs covers the default workload (--impl b200 --workload config2 --shard targets)")
+    return a
 
 
 WORKLOAD = "config2: {nq} target x {nr} reference cells, {g} PCs, k={k}, {metric}"
@@ -93,6 +103,28 @@ def canberra_roofline(g, n, m, kernel_ms):
                                  "note": "5 FP ops per (pair, dimension) of the full metric; the count bound prunes "
                                          "~98 % of it before the FP32 pipe, so achieved / peak is not a fraction of a roof"},
             "traffic": None}
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, out, budget=DUMP_BYTES, suffix=""):
+    """Write the arrays of one mapping step (`out`: name -> host array; "scores" per reference cell, the others per
+    target row) as path/<name><suffix>.npy.  Integers are stored exactly as float64 (indices) or float32 (counts).
+    When the per-target arrays do not fit in `budget` bytes, only a sample of target rows drawn with a fixed seed is
+    written; rows.npy holds the row numbers, so that two runs with the same arguments give the same files."""
+    exact = {np.dtype(np.int32): np.float64, np.dtype(np.int64): np.float64, np.dtype(np.uint8): np.float32}
+    out = {name: np.ascontiguousarray(v, dtype=exact.get(v.dtype, v.dtype)) for name, v in out.items()}
+    per_row = [name for name in out if name != "scores"]
+    n = out[per_row[0]].shape[0]
+    row_bytes = 8 + sum(out[name][:1].nbytes for name in per_row)           # + the row number itself
+    keep = min(n, max(0, budget - out["scores"].nbytes - 4096) // row_bytes)   # 4 KB for the .npy headers
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    out.update({name: out[name][rows] for name in per_row}, rows=rows.astype(np.float64))
+    os.makedirs(path, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(path, name + suffix + ".npy"), v, allow_pickle=False)
+    return keep, n
 
 
 def load_peaks():
@@ -665,7 +697,7 @@ def run_b200(a):
         sc = core.scores_finalize(score_acc, N)
         return idx, dst, cnt, w, sc, (r[2] if stats else None)
 
-    def timed(metric, steps, warmup, e2e=False):
+    def timed(metric, steps, warmup, e2e=False, keep_last=False):
         for _ in range(warmup):
             if e2e:
                 host_step(metric)
@@ -676,7 +708,7 @@ def run_b200(a):
             dist.barrier()
         torch.cuda.synchronize()
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
-        kern_ms, launches, fallback = [], 0, 0
+        kern_ms, launches, fallback, last = [], 0, 0, None
         sampler = ClockSampler(local)
         sampler.start()
         t0 = time.perf_counter()
@@ -685,6 +717,8 @@ def run_b200(a):
             ev[i][0].record()
             if e2e:
                 host_step(metric)
+            elif keep_last and i == steps - 1:
+                last = step(metric, tgt)
             else:
                 step(metric, tgt)
             ev[i][1].record()
@@ -693,6 +727,8 @@ def run_b200(a):
         if world > 1:
             dist.barrier()
         clocks = sampler.stop()
+        if last is not None:
+            last = {name: x.cpu().numpy() for name, x in zip(("idx", "dist", "counts", "weights", "scores"), last)}
         if not e2e:
             # kernel timing pass: the same steps again with the library's per-stage CUDA events (recorded on the
             # launch stream around the candidate kernel).  Kept out of the timed region because reading the
@@ -709,7 +745,7 @@ def run_b200(a):
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return {"ms_total": float(t.item()), "kern_ms": kern_ms, "launches": launches, "fallback": fallback,
-                "clocks": clocks, "wall_s": wall}
+                "clocks": clocks, "wall_s": wall, "last": last}
 
     SCORE_LAUNCHES = 3          # memset of the accumulator, score_accumulate_kernel, score_finalize_kernel
 
@@ -717,7 +753,7 @@ def run_b200(a):
         """Public host-buffer API: pinned host targets in, pinned host results out (copies pipelined)."""
         core.map_cells_host(tgt_pin, ref, ref_knn, k, metric=metric, dist_factor=0.25, mode=a.engine)
 
-    main = timed(a.metric, a.steps, a.warmup)
+    main = timed(a.metric, a.steps, a.warmup, keep_last=bool(a.dump_outputs))
     e2e = timed(a.metric, max(3, a.steps // 2), 2, e2e=True)
     ms_step = main["ms_total"] / a.steps
     value = world * N / (ms_step / 1e3)
@@ -808,6 +844,9 @@ def run_b200(a):
                                           "(C port of the reference loops, %d host threads)" % (n, N, M, dt, threads)}
     elif rank == 0:
         line["cpu_baseline"] = None
+    if a.dump_outputs:
+        # every rank maps its own targets: one file set per rank when there are several, sharing the size budget
+        dump_outputs(a.dump_outputs, main["last"], DUMP_BYTES // world, "" if world == 1 else "_rank%d" % rank)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:

@@ -1,4 +1,5 @@
-"""bench.py contract on the GPU: one JSON line with the metric, the end-to-end arm, the roofline and the CPU baseline."""
+"""bench.py contract on the GPU: one JSON line with the metric, the end-to-end arm, the roofline and the CPU baseline;
+--dump-outputs writes what the timed path computed."""
 import json
 import os
 import subprocess
@@ -10,10 +11,11 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_bench_line_has_the_contract_keys():
+def test_bench_line_has_the_contract_keys(tmp_path):
+    dump = str(tmp_path / "outputs")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "3", "--warmup", "3",
                           "--n-ref", "30000", "--n-query", "30000", "--cpu-seconds", "1", "--no-config5",
-                          "--ref-rows-per-gpu", "300000", "--ref-batch", "60000"],
+                          "--ref-rows-per-gpu", "300000", "--ref-batch", "60000", "--dump-outputs", dump],
                          capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-3000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
@@ -39,3 +41,18 @@ def test_bench_line_has_the_contract_keys():
     assert set(("knn_candidates", "knn_rerank", "exchange", "merge", "snn", "scores")) <= set(rs["stage_ms"])
     assert line["score_determinism"]["bit_identical_single_vs_target_sharded_vs_reference_sharded"] is True
     assert line["projection"]["config1"]["mma"]["ms"] > 0 and line["projection"]["config5_slice"]["mma"]["fp64_tflops"] > 1
+    # --dump-outputs: the last timed step's arrays, whole at this size, equal to the same path run here
+    import numpy as np
+    import torch
+    from nabo_b200 import core, synth
+    got = {f[:-4]: np.load(os.path.join(dump, f), allow_pickle=False) for f in os.listdir(dump)}
+    assert sorted(got) == ["counts", "dist", "idx", "rows", "scores", "weights"]
+    assert np.array_equal(got["rows"], np.arange(30000))
+    ref = torch.from_numpy(synth.pc_mixture(30000, 50, seed=1)).cuda()
+    tgt = torch.from_numpy(synth.pc_mixture(30000, 50, seed=101)).cuda()
+    ref_knn, _ = core.knn(ref, ref, 30, "euclidean", drop_first=True, mode="fast")
+    idx, dst = core.knn(tgt, ref, 30, "euclidean", mode="fast")
+    cnt, w = core.snn_weights(idx, ref_knn, 30)
+    sc = core.scores_finalize(core.score_accumulate(idx, cnt, 30000, 30), 30000)
+    for name, x in (("idx", idx), ("dist", dst), ("counts", cnt), ("weights", w), ("scores", sc)):
+        assert got[name].dtype in (np.float32, np.float64) and np.array_equal(got[name], x.cpu().numpy()), name
