@@ -36,7 +36,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(objdir, exist_ok=True)
     common = [nvcc, *ARCH_FLAGS, "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr", "-Xptxas", "-v" if verbose else "-O3"]
-    common += os.environ.get("NABO_NVCC_EXTRA", "").split()      # development switches (e.g. -DNABO_CBS_STATS)
+    common += os.environ.get("NABO_NVCC_EXTRA", "").split()      # development switches (e.g. -DNABO_CBS_PROF)
     objs = []
     procs = []
     for src in sources():

@@ -31,19 +31,6 @@
 #include "ptx.cuh"
 #include "select.cuh"
 
-#ifndef NABO_CBS_NBINS
-#define NABO_CBS_NBINS 32
-#endif
-#ifndef NABO_CBS_RT
-#define NABO_CBS_RT 128
-#endif
-#ifndef NABO_CBS_DUAL
-#define NABO_CBS_DUAL 1              // two work-list entries per lane and evaluation pass when more than 32 are left
-#endif
-#ifndef NABO_CBS_SLEEP_NS
-#define NABO_CBS_SLEEP_NS 400        // suspend-time hint of the tile waits (0 = plain polling)
-#endif
-
 namespace cbs {
 
 #ifdef NABO_CBS_PROF       // development cycle accounting of a busy warp's sweep (tools/probe_cb_prof.py):
@@ -64,15 +51,13 @@ __device__ unsigned long long g_cbs_prof[12];
 
 using namespace sel;   // make_key, compact_select, compact_sort_inline
 
-constexpr int NBINS = NABO_CBS_NBINS;     // value bins per dimension
-constexpr int RT = NABO_CBS_RT;           // references per tile (64 or 128)
+constexpr int NBINS = 32;                 // value bins per dimension
+constexpr int RT = 128;                   // references per tile
 constexpr int WPT = RT / 32;              // words per tile
 constexpr int T64 = RT / 64;              // 64-reference blocks of the FP32 copy per tile
-// cumulative planes per (dimension, word): NBINS + 1, padded so that a (dimension) row of WPT words is a multiple
-// of 16 bytes (bulk copies) - the pad planes are never read
-constexpr int NPL = (WPT % 4 == 0) ? NBINS + 1 : ((NBINS + 1 + 1) & ~1);
-static_assert(RT == 64 || RT == 128, "tile = 64 or 128 references");
-static_assert(NBINS >= 2 && NBINS <= 128 && (WPT * NPL) % 4 == 0, "plane rows must be multiples of 16 bytes");
+constexpr int NPL = NBINS + 1;            // cumulative planes per (dimension, word)
+static_assert((WPT * NPL) % 4 == 0, "plane rows must be multiples of 16 bytes (bulk copies)");
+constexpr int SLEEP_NS = 400;             // suspend-time hint of the tile waits
 constexpr int NW = 12;                    // warps per CTA
 constexpr int QB = NW * 32;               // queries a CTA handles per round (at most)
 constexpr int NTHREADS = NW * 32;
@@ -347,12 +332,12 @@ sliced_kernel(const Params p) {
     const int kprime = p.kprime;
 
     // dense FP32 evaluation of the first n work-list entries of the current tile.  A lane takes TWO entries per pass
-    // (NABO_CBS_DUAL) when more than 32 are left: the two dependency chains (load, rcp, select, add) interleave, and a
+    // when more than 32 are left: the two dependency chains (load, rcp, select, add) interleave, and a
     // warp's sweep is latency-bound.  A pass then adds at most 64 keys to one query, so the buffers are kept at or
     // below CAP - 64 (dual passes are used only when kprime + trig_extra allows that).
     CBS_PROF_DECL
     const int trig = min(CAP - 32, kprime + p.trig_extra);
-    const bool dual_ok = NABO_CBS_DUAL && trig <= CAP - 64;
+    const bool dual_ok = trig <= CAP - 64;
     auto compact_due = [&]() {
         // compacting earlier than the buffer limit (kprime + trig_extra keys) keeps tau closer to the true running
         // K'-th best score: a stale threshold lets proportionally more pairs through to the dense evaluation
@@ -363,7 +348,7 @@ sliced_kernel(const Params p) {
             need &= need - 1;
             int nc;
             float nt;
-            compact_select<4>(gbuf + (size_t)src * CAP, s_cnt[src], lane, kprime, trig - 4 > kprime ? trig - 4 : kprime, hist, nc, nt);
+            compact_select(gbuf + (size_t)src * CAP, s_cnt[src], lane, kprime, trig - 4 > kprime ? trig - 4 : kprime, hist, nc, nt);
             if (lane == src) { s_cnt[lane] = nc; s_tau[lane] = nt; }
             __syncwarp();
             CBS_PROF_COUNT(9, 1)
@@ -443,7 +428,7 @@ sliced_kernel(const Params p) {
             // no group for this warp in this round: keep the tile ring moving
             for (int j = 0; j < n_tiles; ++j, ++t) {
                 const uint32_t s = t % p.stages, use = t / p.stages;
-                ptx::mbar_wait_hint(&bars->full[s], use & 1, NABO_CBS_SLEEP_NS);
+                ptx::mbar_wait_hint(&bars->full[s], use & 1, SLEEP_NS);
                 release_tile(t, s);
             }
             continue;
@@ -462,7 +447,7 @@ sliced_kernel(const Params p) {
         for (int jl = 0; jl < n_tiles; ++jl, ++t) {
             const int j = tile0 + jl;
             const uint32_t s = t % p.stages, use = t / p.stages;
-            ptx::mbar_wait_hint(&bars->full[s], use & 1, NABO_CBS_SLEEP_NS);   // sleep, do not poll: 10 % of the issue slots went here
+            ptx::mbar_wait_hint(&bars->full[s], use & 1, SLEEP_NS);   // sleep, do not poll: 10 % of the issue slots went here
             CBS_PROF_COUNT(7, 1)
             CBS_PROF(0)
             const unsigned char* stage = smem + p.stage_off + (size_t)s * p.stage_bytes;
@@ -601,7 +586,7 @@ sliced_kernel(const Params p) {
             uint32_t ks[4], kpl[4];
             int nc;
             float nt;
-            compact_sort_inline<4>(gbuf + (size_t)src * CAP, n, lane, kprime, ks, kpl, nc, nt);
+            compact_sort_inline(gbuf + (size_t)src * CAP, n, lane, kprime, ks, kpl, nc, nt);
             const long long qg = (long long)group * 32 + src;
             if (qg < p.n_query) {
 #pragma unroll

@@ -618,15 +618,6 @@ int nabo_knn_exact_launch_ex(const double* q, int ldq, const double* r, int ldr,
     return 0;
 }
 
-#ifndef NABO_RR_HIST
-#define NABO_RR_HIST 1         // development switches of the re-rank kernel (A/B builds)
-#endif
-#ifndef NABO_RR_SCRAMBLE
-#define NABO_RR_SCRAMBLE 1
-#endif
-#ifndef NABO_RR_FUSED
-#define NABO_RR_FUSED 1
-#endif
 // ------------------------------------------------------------------ exact re-rank of candidates
 // One warp per query.  cand (n_query x n_cand) holds LOCAL reference indices, -1 = empty,
 // all distinct.  With a certificate (NaboCert.kind != 0) the kernel also proves that no
@@ -717,8 +708,6 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
     const double* x = q + (long long)qi * ldq;
     double nq = 0.0;
     if (METRIC == NABO_COSINE) nq = seq_sqnorm(x, g);
-    // FROM_BUF: final K' selection of the query's candidate buffer (what tc::emit_kernel does otherwise): the 128
-    // keys are sorted by score in registers, element u * 32 + lane of the sorted list ends up in kpl[u]
     // FROM_BUF: final K' selection of the query's candidate buffer (what tc::emit_kernel does otherwise).  One
     // histogram pass over the scores finds the bin that holds the K'-th best key; the keys of lower bins and the best
     // of that bin (ranked by pairwise comparison) are the K' candidates, the threshold is the largest kept score.
@@ -741,7 +730,7 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
         uint32_t* hist = reinterpret_cast<uint32_t*>(smem + hist_off) + warp * 256;
         int bin[4], cut_bin, kept;
         bool reach;
-        sel::histogram_cut<4>(fv, n, lane, cb.kprime, hist, bin, cut_bin, kept, reach);
+        sel::histogram_cut(fv, n, lane, cb.kprime, hist, bin, cut_bin, kept, reach);
         // keys of the cut bin beyond the K' needed: ranked among themselves (score, then buffer position), so that
         // exactly K' stay - every extra candidate is a 400-byte row gather from HBM once the reference outgrows L2
         const int c_cut = reach ? (int)hist[cut_bin] : 0;
@@ -753,7 +742,7 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
             atomicAdd(&g_rr_stats[4], (unsigned long long)(reach ? c_cut - need : 0));
         }
 #endif
-        if (NABO_RR_HIST && (!reach || c_cut <= 48)) {
+        if (!reach || c_cut <= 48) {
             int rank[4] = {0, 0, 0, 0};
             if (reach && c_cut > need) {
 #pragma unroll
@@ -789,7 +778,7 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
             uint32_t ks[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) ks[u] = u * 32 + lane < n ? float_to_sortable(fv[u]) : 0xffffffffu;
-            sel::sortn<4>(ks, kpl, lane);
+            sel::sortn(ks, kpl, lane);
             nc = n < cb.kprime ? n : cb.kprime;
             const int e = cb.kprime - 1;                      // kprime <= 64
             const uint32_t ts = __shfl_sync(0xffffffffu, (e >> 5) ? ks[1] : ks[0], e & 31);
@@ -813,7 +802,7 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
     const double* xq = xw ? xw : x;
     int jj[4];
     int n_slots = 0;
-    const bool scramble = NABO_RR_SCRAMBLE && (long long)n_ref * ldr * 8 > (96ll << 20);
+    const bool scramble = (long long)n_ref * ldr * 8 > (96ll << 20);
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
         const int c = u * 32 + lane;
@@ -834,7 +823,7 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
         if (__any_sync(0xffffffffu, j >= 0)) n_slots = u + 1;
     }
     double accs[4] = {0.0, 0.0, 0.0, 0.0};
-    if (METRIC == NABO_MOD_CANBERRA || !NABO_RR_FUSED) {
+    if (METRIC == NABO_MOD_CANBERRA) {
         // the FP64 division sits under a divergent branch: slot by slot, so that a slot with few lanes costs few divisions
 #pragma unroll
         for (int u = 0; u < 4; ++u)

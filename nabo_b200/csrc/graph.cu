@@ -230,25 +230,6 @@ rs_scatter_kernel(const uint32_t* __restrict__ keys, const uint32_t* __restrict_
     }
 }
 
-// One stable 8-bit LSD pass over (keys, vals): used by the score reduction below and by the locality ordering of
-// the tensor-core candidate pass (keys = cluster ids, one pass).  scratch: 256 * nblocks + 256 uint32.
-size_t nabo_radix_pass_scratch_bytes(long long n) {
-    const size_t nblocks = (size_t)((n + RS_BLOCK - 1) / RS_BLOCK);
-    return nabo_align_up(256 * nblocks * sizeof(uint32_t), 256) + 256 * sizeof(uint32_t) + 256;
-}
-int nabo_radix_pass_launch(const uint32_t* keys, const uint32_t* vals, int n, int shift, void* scratch,
-                           uint32_t* out_keys, uint32_t* out_vals, cudaStream_t st) {
-    if (n <= 0) return 0;
-    const int nblocks = (n + RS_BLOCK - 1) / RS_BLOCK;
-    uint32_t* hist = (uint32_t*)scratch;
-    uint32_t* totals = (uint32_t*)((char*)scratch + nabo_align_up(256 * (size_t)nblocks * sizeof(uint32_t), 256));
-    rs_hist_kernel<<<nblocks, RS_THREADS, 0, st>>>(keys, n, shift, hist, nblocks);
-    rs_scan_rows_kernel<<<256, 256, 0, st>>>(hist, nblocks, totals);
-    rs_scatter_kernel<<<nblocks, RS_THREADS, 0, st>>>(keys, vals, n, shift, hist, totals, nblocks, out_keys, out_vals);
-    NABO_LAUNCH_CHECK("radix pass");
-    return 0;
-}
-
 // ------------------------------------------------------------------ mapping scores
 __global__ void __launch_bounds__(256)
 score_edges_kernel(const int32_t* __restrict__ tgt_knn, const uint8_t* __restrict__ counts,

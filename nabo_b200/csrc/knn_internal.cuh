@@ -131,9 +131,6 @@ int nabo_cbs_split(int n_query, int n_ref, int k, int drop_first);
 int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                         double f, const uint8_t* mask, int drop_first, int n_split, float* rt, void* extra,
                         size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st);
-size_t nabo_radix_pass_scratch_bytes(long long n);
-int nabo_radix_pass_launch(const uint32_t* keys, const uint32_t* vals, int n, int shift, void* scratch,
-                           uint32_t* out_keys, uint32_t* out_vals, cudaStream_t st);
 int nabo_tau_min_launch(float* tau, int n_query, int n_split, cudaStream_t st);
 
 size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric);

@@ -1,4 +1,4 @@
-// Per-query running top-K' selection over a 128-entry key buffer in global memory (L2 resident):
+// Per-query running top-K' selection over a CAP-entry key buffer in global memory (L2 resident):
 // shared by the tensor-core candidate kernel (tc_candidates.cu) and the bit-sliced Canberra kernel
 // (canberra_sliced.cu).  All routines are warp-cooperative; `lane` is the caller's lane id.
 #pragma once
@@ -6,8 +6,8 @@
 
 namespace sel {
 
-constexpr int CAP = 128;   // keys per query buffer of the default instantiations (KPL = 4 keys per lane);
-                           // the tensor-core pass uses KPL = 8 (256 keys): compactions are a quarter as frequent
+constexpr int CAP = 128;        // keys per query buffer
+constexpr int KPL = CAP / 32;   // keys per lane: element i = u * 32 + lane sits in slot u of its lane
 
 // buffer key = raw float bits of the score (high word) | local reference index (low word);
 // the compaction routines convert to an order-preserving integer when they load a key
@@ -16,7 +16,7 @@ __device__ __forceinline__ unsigned long long make_key(float score, uint32_t col
 }
 
 // ---- warp-cooperative compaction entirely in registers -----------------------------------
-// The 128 keys of one query are spread 4 per lane (element i = u*32 + lane) and sorted by
+// The CAP keys of one query are spread KPL per lane (element i = u*32 + lane) and sorted by
 // score with a bitonic network: strides >= 32 are register-to-register, smaller strides are
 // shuffles.  Only the score is compared (ties keep an arbitrary member; everything dropped
 // still has score >= the new threshold, which is all the certificate needs).
@@ -26,7 +26,6 @@ __device__ __forceinline__ void cex(uint32_t& s0, uint32_t& p0, uint32_t& s1, ui
     if (sw) { uint32_t t = s0; s0 = s1; s1 = t; t = p0; p0 = p1; p1 = t; }
 }
 
-template <int KPL>
 __device__ __forceinline__ void sortn(uint32_t (&s)[KPL], uint32_t (&pl)[KPL], int lane) {
 #pragma unroll
     for (int size = 2; size <= 32 * KPL; size <<= 1) {
@@ -57,13 +56,11 @@ __device__ __forceinline__ void sortn(uint32_t (&s)[KPL], uint32_t (&pl)[KPL], i
         }
     }
 }
-__device__ __forceinline__ void sort128(uint32_t (&s)[4], uint32_t (&pl)[4], int lane) { sortn<4>(s, pl, lane); }
 
 // Exact compaction: sort lane `src`'s buffer (n live keys), keep the kprime best at the front of the
 // buffer.  New count / threshold come back through nc / nt (valid on every lane); s / pl hold the sorted
 // keys.  Force-inlined where the caller consumes s / pl (the per-item final emit) so that the arrays
 // stay in registers; compact_select uses the out-of-line wrapper below as its rare fallback.
-template <int KPL>
 __device__ __forceinline__ void compact_sort_inline(unsigned long long* gbuf, int n, int lane, int kprime,
                                                     uint32_t (&s)[KPL], uint32_t (&pl)[KPL], int& nc, float& nt) {
     __syncwarp();            // the owner's appends (plain global stores) are ordered before our loads
@@ -74,7 +71,7 @@ __device__ __forceinline__ void compact_sort_inline(unsigned long long* gbuf, in
         s[u] = i < n ? float_to_sortable(__uint_as_float((uint32_t)(kv >> 32))) : 0xffffffffu;
         pl[u] = (uint32_t)kv;
     }
-    sortn<KPL>(s, pl, lane);
+    sortn(s, pl, lane);
     nc = n < kprime ? n : kprime;
 #pragma unroll
     for (int u = 0; u < KPL; ++u) {
@@ -92,10 +89,9 @@ __device__ __forceinline__ void compact_sort_inline(unsigned long long* gbuf, in
     __syncwarp();
 }
 
-template <int KPL>
 static __device__ __noinline__ void compact_sort(unsigned long long* gbuf, int n, int lane, int kprime, int& nc, float& nt) {
     uint32_t s[KPL], pl[KPL];
-    compact_sort_inline<KPL>(gbuf, n, lane, kprime, s, pl, nc, nt);
+    compact_sort_inline(gbuf, n, lane, kprime, s, pl, nc, nt);
 }
 
 // Cheap running compaction: one 256-bin histogram pass over the scores of the buffer finds a
@@ -105,7 +101,6 @@ static __device__ __noinline__ void compact_sort(unsigned long long* gbuf, int n
 // ("everything rejected or dropped has score >= tau") holds without an exact selection.
 // If the cut keeps more than max_keep keys (ties, duplicates) the exact sort takes over.
 // hist: 256 counters of this warp in shared memory.
-template <int KPL>
 static __device__ __noinline__ void compact_select(unsigned long long* gbuf, int n, int lane, int kprime, int max_keep,
                                             uint32_t* hist, int& nc, float& nt) {
     __syncwarp();
@@ -168,7 +163,7 @@ static __device__ __noinline__ void compact_select(unsigned long long* gbuf, int
         kept = __shfl_sync(0xffffffffu, k_at, owner);
     }
     if ((int)kept > max_keep) {
-        compact_sort<KPL>(gbuf, n, lane, kprime, nc, nt);
+        compact_sort(gbuf, n, lane, kprime, nc, nt);
         return;
     }
     // stream-compact the kept keys to the front (all keys are in registers: in-place is safe)
@@ -194,7 +189,6 @@ static __device__ __noinline__ void compact_select(unsigned long long* gbuf, int
 // The histogram cut of compact_select on keys already in registers: bin[u] of every live key and the cut bin with
 // at least kprime keys at or below it (kept = how many).  reach = false when n < kprime (keep everything).
 // fv[u] of element i = u * 32 + lane, live iff i < n.  hist: 256 counters of this warp in shared memory.
-template <int KPL>
 __device__ __forceinline__ void histogram_cut(const float (&fv)[KPL], int n, int lane, int kprime, uint32_t* hist,
                                               int (&bin)[KPL], int& cut_bin, int& kept, bool& reach_out) {
     float flo = CUDART_INF_F, fhi = -CUDART_INF_F;

@@ -28,7 +28,6 @@
 #include "select.cuh"
 
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 namespace tc {
 
@@ -37,35 +36,21 @@ constexpr int NQ = 3;               // query tiles per work item
 constexpr int NTHREADS = 512;
 constexpr int N_EPI_WARPS = 4 * NQ;  // warps 0..11: epilogue (TMEM lane quarter = warp % 4)
 constexpr int PRODUCER_WARP = 12;    // highest warp ids on their schedulers: the arbiter favours them,
-constexpr int MMA_WARP0 = 13;        // so the single-thread producer / issuers are never starved;
-                                     // warps 13..15: one MMA issuer per query tile (no polling loop)
+constexpr int MMA_WARP = 13;         // so the single-thread producer / issuer are never starved
 constexpr int TMEM_WARP = 12;
-#ifndef NABO_TC_KPL
-#define NABO_TC_KPL 4                // measured with 8 (256-key buffers, a quarter of the compactions): candidate kernel
-#endif                               // 3.78 -> 4.51 ms at 100 k x 100 k (staler thresholds, 2 KB per query in L2) and the
-constexpr int KPL = NABO_TC_KPL;     // final selection 0.17 -> 1.8 ms; it only pays for K' > 56 (k = 60: 55 -> 7.4 ms)
+constexpr int KPL = 4;               // keys per lane.  Measured with 8 (256-key buffers, a quarter of the compactions):
+                                     // candidate kernel 3.78 -> 4.51 ms at 100 k x 100 k (staler thresholds, 2 KB per
+                                     // query in L2) and the final selection 0.17 -> 1.8 ms; it only pays for K' > 56
+                                     // (k = 60: 55 -> 7.4 ms)
 constexpr int CAP = 32 * KPL;        // candidate buffer entries per query
+static_assert(CAP == sel::CAP, "the fused re-rank (exact.cu) reads the candidate buffers with sel::CAP keys per query");
 constexpr int CHUNK = 32;           // columns per tcgen05.ld
 constexpr int MAX_KPRIME = 96;      // K' lists go to the re-rank, which takes at most 128 candidates per query
-#ifndef NABO_TC_ROTATE
-#define NABO_TC_ROTATE 1
-#endif
-#ifndef NABO_TC_PIPE
-#define NABO_TC_PIPE 0
-#endif
-#ifndef NABO_TC_SLEEP_NS
-#define NABO_TC_SLEEP_NS 2000        // suspend-time hint of the producer's mbarrier waits (0 = plain polling)
-#endif
-#ifndef NABO_TC_EPI_SLEEP_NS
-#define NABO_TC_EPI_SLEEP_NS 0       // suspend-time hint of the epilogue warps' wait for an accumulator (0 = plain polling)
-#endif
-#ifndef NABO_TC_UNIFORM_HIT
-#define NABO_TC_UNIFORM_HIT 0
-#endif
-// accumulators in TMEM (128 columns each).  ROTATE: the NQ query tiles share NQ + 1 buffers in a fixed
-// rotation (job n = tile * NQ + q uses buffer n % 4), so the MMAs of a warpgroup's next tile run while it is
-// still reading the current one; otherwise one private buffer per query tile (MMA and epilogue alternate).
-constexpr int NACC = NABO_TC_ROTATE ? 4 : NQ;
+constexpr int SLEEP_NS = 2000;      // suspend-time hint of the producer's mbarrier waits
+// accumulators in TMEM (128 columns each): the NQ query tiles share NQ + 1 buffers in a fixed rotation
+// (job n = tile * NQ + q uses buffer n % 4), so the MMAs of a warpgroup's next tile run while it is still
+// reading the current one
+constexpr int NACC = 4;
 
 __host__ __device__ inline int kp_for(int g) { return (3 * g + 3 + 15) / 16 * 16; }
 __host__ __device__ inline size_t tile_bytes(int kp) { return (size_t)TILE * kp * 2; }
@@ -138,20 +123,18 @@ __global__ void scale_kernel(const unsigned int* __restrict__ maxq_bits, const u
 // (core matrices of 8 rows x 16 B, K-chunk-major: SBO = 128 B, LBO = TILE*16 B).  The chunks that hold the norm
 // columns 3g .. 3g+2 of a reference row need the whole ||r~||^2: they are written after the partial sums of the
 // row's threads have met in shared memory (fixed order: deterministic).
-// perm (or NULL): packed row i holds input row perm[i] (locality order, see order_* below)
 constexpr int PACK_SPLIT = 4;
 template <bool IS_QUERY>
 __global__ void __launch_bounds__(TILE * PACK_SPLIT)
 pack_kernel(const double* __restrict__ x, int ld, int n, int g, int kp, const double* __restrict__ norms2,
-            const double* __restrict__ scal, const uint8_t* __restrict__ mask, const uint32_t* __restrict__ perm,
-            __half* __restrict__ out, double* __restrict__ qn2_out) {
+            const double* __restrict__ scal, const uint8_t* __restrict__ mask, __half* __restrict__ out,
+            double* __restrict__ qn2_out) {
     __shared__ double part[PACK_SPLIT][TILE];
     const int r = threadIdx.x & (TILE - 1);
     const int c = threadIdx.x / TILE;                 // warp-uniform
-    const long long prow = (long long)blockIdx.x * TILE + r;
+    const long long row = (long long)blockIdx.x * TILE + r;
     __half* tile = out + (size_t)blockIdx.x * TILE * kp;
-    const bool live = prow < n;
-    const long long row = live && perm ? (long long)perm[prow] : prow;
+    const bool live = row < n;
     const double sc = scal[0];
     const bool cosine = scal[3] != 0.0;
     double mul = sc;
@@ -238,109 +221,19 @@ pack_kernel(const double* __restrict__ x, int ld, int n, int g, int kp, const do
     if (IS_QUERY && c == 0 && live && qn2_out) qn2_out[row] = n2_row;
 }
 
-// ------------------------------------------------------------------ locality order
-// A query's threshold tau is only as tight as the best K' references it has met so far, and while it is loose
-// nearly every 32 x 32 warp chunk holds some score below some lane's tau and takes the append path.  Both
-// operands are therefore packed in LOCALITY ORDER - sorted by the nearest of N_CEN centroids (rows sampled from
-// the reference; leading min(g, 64) coordinates, FP32; one stable radix pass) - and every work item starts its
-// sweep at the reference tiles of its own queries' cluster: the neighbours arrive first, tau is final after a
-// few percent of the sweep, and the remaining tiles cost the no-hit path only.  All pairs are still evaluated on
-// the tensor cores; results do not change (the exact re-rank orders by (distance, index) of the ORIGINAL rows).
-constexpr int N_CEN = 64;
-constexpr int CEN_DIMS = 64;
-
-__global__ void centroid_gather_kernel(const double* __restrict__ r, int ld, int n_ref, int gs, int cosine,
-                                       float* __restrict__ cen) {
-    const int c = blockIdx.x, k = threadIdx.x;
-    const long long row = (long long)c * n_ref / N_CEN;
-    const double* p = r + row * ld;
-    __shared__ float inv;
-    if (k == 0) {
-        inv = 1.f;
-        if (cosine) {
-            double s = 0.0;
-            for (int i = 0; i < gs; ++i) s = fma(p[i], p[i], s);
-            inv = s > 0.0 ? (float)(1.0 / sqrt(s)) : 0.f;
-        }
-    }
-    __syncthreads();
-    if (k < gs) cen[c * CEN_DIMS + k] = (float)p[k] * inv;
-}
-
-__global__ void __launch_bounds__(256)
-cluster_assign_kernel(const double* __restrict__ x, int ld, int n, int gs, int cosine, const float* __restrict__ cen,
-                      uint32_t* __restrict__ cl, uint32_t* __restrict__ iota) {
-    __shared__ float sc[N_CEN * CEN_DIMS];
-    for (int i = threadIdx.x; i < N_CEN * CEN_DIMS; i += blockDim.x) sc[i] = cen[i];
-    __syncthreads();
-    const int row = blockIdx.x * blockDim.x + threadIdx.x;
-    if (row >= n) return;
-    const double* p = x + (long long)row * ld;
-    float inv = 1.f;
-    if (cosine) {
-        float s = 0.f;
-        for (int k = 0; k < gs; ++k) { const float v = (float)p[k]; s = fmaf(v, v, s); }
-        inv = s > 0.f ? rsqrtf(s) : 0.f;
-    }
-    float acc[N_CEN];
-#pragma unroll
-    for (int c = 0; c < N_CEN; ++c) acc[c] = 0.f;
-    for (int k = 0; k < gs; ++k) {
-        const float v = (float)p[k] * inv;
-#pragma unroll
-        for (int c = 0; c < N_CEN; ++c) { const float d = v - sc[c * CEN_DIMS + k]; acc[c] = fmaf(d, d, acc[c]); }
-    }
-    int best = 0;
-    float bd = CUDART_INF_F;
-#pragma unroll
-    for (int c = 0; c < N_CEN; ++c)
-        if (acc[c] < bd) { bd = acc[c]; best = c; }            // NaN rows stay in cluster 0
-    cl[row] = (uint32_t)best;
-    iota[row] = (uint32_t)row;
-}
-
-// first[c] = first sorted position holding a cluster id >= c (c = 0 .. N_CEN)
-__global__ void cluster_first_kernel(const uint32_t* __restrict__ sorted_cl, int n, int* __restrict__ first) {
-    const int c = threadIdx.x;
-    if (c > N_CEN) return;
-    int lo = 0, hi = n;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if (sorted_cl[mid] < (uint32_t)c) lo = mid + 1; else hi = mid;
-    }
-    first[c] = lo;
-}
-
-// start tile of every work item = where the cluster of its middle query begins in the sorted reference
-__global__ void item_start_kernel(const uint32_t* __restrict__ sorted_cl_q, int n_query, const int* __restrict__ first_r,
-                                  int n_items, int n_rtiles, int* __restrict__ start) {
-    const int it = blockIdx.x * blockDim.x + threadIdx.x;
-    if (it >= n_items) return;
-    long long mid = (long long)it * NQ * TILE + NQ * TILE / 2;
-    if (mid >= n_query) mid = n_query - 1;
-    int t = first_r[sorted_cl_q[mid]] / TILE;
-    start[it] = t < n_rtiles ? t : n_rtiles - 1;
-}
-
 // ------------------------------------------------------------------ the candidate kernel
 struct Params {
     const __half* qa;       // packed queries  [n_qtiles_padded][TILE*kp]
     const __half* rb;       // packed references [n_rtiles][TILE*kp]
     int n_query, n_ref, kp, n_items, n_rtiles, stages, kprime, kc_out, soft;
-    int signal_round;       // MODE 0: > 0 = every CTA signals the dependent launch after its signal_round-th item (0 = never)
+    int signal_round;       // > 0 = every CTA signals the dependent launch after its signal_round-th item (0 = never;
+                            // always 0 when n_split > 1)
     int n_split;            // reference ranges per query item (work item = n_items x n_split, see nabo_tc_split)
     unsigned long long* cand_buf;   // [work item][NQ*TILE][CAP]: every (query, reference range) owns CAP keys
     int* cand_cnt;          // [work item][NQ*TILE] live keys of each buffer when its sweep ended
     float* cand_tau;        // [work item][NQ*TILE] running threshold when its sweep ended
     int32_t* cand_idx;      // [n_query][n_split][kc_out]      (written by emit_kernel)
     float* cert_tau;        // [n_split][n_query]              (written by emit_kernel)
-    const uint32_t* perm_q; // packed query row -> input row (NULL = identity)
-    const uint32_t* perm_r; // packed reference row -> input row (NULL = identity)
-    const int* item_start;  // first reference tile of every item's sweep (NULL = 0; unsplit kernel only)
-    // balanced last wave (MODE 2): the first n_full items run whole, one per CTA and round; the remaining bal_rem
-    // items are cut into reference pieces so that all CTAs finish together (see work_piece below)
-    int n_full, bal_rem, bal_share, bal_p;      // bal_p > 0: bal_p aligned pieces per item; 0: contiguous ranges
-    int dbg;                // NABO_TC_DBG bit mask for timing experiments (0 in production): 1 = skip the final emit
     size_t a_off, b_off, sort_off, bar_off;
 };
 
@@ -351,7 +244,7 @@ struct Barriers {
     uint32_t tmem_base;
 };
 
-using namespace sel;   // make_key, sort128, compact_sort(_inline), compact_select (select.cuh)
+using namespace sel;   // make_key, compact_sort_inline, compact_select (select.cuh)
 
 #ifdef NABO_TC_STATS       // development counters (tools/probe_tc_stats.py): [0] warp chunks, [1] warp chunks with a hit,
 __device__ unsigned long long g_tc_stats[12];  // [2] lanes with a hit, [3] keys appended, [4] running compactions,
@@ -399,24 +292,6 @@ __device__ __forceinline__ void filter_chunk(const uint32_t (&vr)[32], uint32_t 
         if ((threadIdx.x & 31) == 0) TC_STAT(3, na);
     }
 #endif
-#if NABO_TC_UNIFORM_HIT
-    // warp-uniform branches only (no divergence / reconvergence barriers): a group of 8 columns is appended with
-    // predicated stores whenever ANY lane holds a score below its threshold in it
-    if (__any_sync(0xffffffffu, m < tau)) {
-#pragma unroll
-        for (int gi = 0; gi < 4; ++gi) {
-            if (__any_sync(0xffffffffu, g4[gi] < tau)) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    if (v[8 * gi + i] < tau) {
-                        mybuf[cnt] = make_key(v[8 * gi + i], col0 + 8 * gi + i);
-                        ++cnt;
-                    }
-                }
-            }
-        }
-    }
-#else
     if (m < tau) {
 #pragma unroll
         for (int gi = 0; gi < 4; ++gi) {
@@ -432,90 +307,30 @@ __device__ __forceinline__ void filter_chunk(const uint32_t (&vr)[32], uint32_t 
             }
         }
     }
-#endif
 }
 
-// Work enumeration.  MODE 0: one work item per query item (whole reference sweep, cyclic from the item's start
-// tile).  MODE 1: few items - every item's reference range is cut into n_split equal pieces, each a work item.
-// MODE 2: more items than CTAs and a last wave that would leave SMs idle - the first n_full (a multiple of the grid)
-// items run whole, the other bal_rem items are cut so that every CTA gets the same number of reference tiles:
-//   bal_p > 0 (last wave less than half full): bal_p aligned pieces per item, piece s = tiles [s share, (s+1) share);
-//   bal_p = 0: the tail is one sequence of bal_rem * n_rtiles tiles, CTA c takes [c share, (c+1) share) - up to two
-//              pieces (end of one item, start of the next); an item is cut into at most three pieces.
-// Every piece has its own buffer `slot`, K' list and threshold (segment `seg` of its item); the re-rank takes the
-// union of the lists and the smallest threshold.  Returns false when CTA `c` has no r-th work item.
-template <int MODE>
-__device__ __forceinline__ bool work_piece(const Params& p, int c, int r, int& slot, int& qitem, int& seg, int& j0,
-                                           int& j1, int& start) {
-    start = 0;
-    if (MODE == 0) {
-        slot = c + r * (int)gridDim.x;
+// Work enumeration: the reference range of every query item is cut into n_split equal pieces, each a work item with
+// its own buffer `slot`, K' list and threshold; the re-rank takes the union of the lists and the smallest threshold.
+// CTA c takes the slots c, c + grid, c + 2 grid, ...  Returns false when CTA `c` has no r-th work item.
+// SPLIT = false is the n_split = 1 case (the whole reference), compiled on its own: the general form in the unsplit
+// kernel measured 3.59 -> 3.72 ms at 100 k x 100 k, k = 30 (B200, 1 000 W power limit).
+template <bool SPLIT>
+__device__ __forceinline__ bool work_piece(const Params& p, int c, int r, int& slot, int& qitem, int& j0, int& j1) {
+    slot = c + r * (int)gridDim.x;
+    if (!SPLIT) {
         if (slot >= p.n_items) return false;
-        qitem = slot; seg = 0; j0 = 0; j1 = p.n_rtiles;
-        if (p.item_start) start = p.item_start[slot];
+        qitem = slot; j0 = 0; j1 = p.n_rtiles;
         return true;
     }
-    if (MODE == 1) {
-        slot = c + r * (int)gridDim.x;
-        if (slot >= p.n_items * p.n_split) return false;
-        qitem = slot / p.n_split;
-        seg = slot - qitem * p.n_split;
-        j0 = (int)((long long)p.n_rtiles * seg / p.n_split);
-        j1 = (int)((long long)p.n_rtiles * (seg + 1) / p.n_split);
-        return true;
-    }
-    const int rounds_full = p.n_full / (int)gridDim.x;
-    if (r < rounds_full) {
-        slot = c + r * (int)gridDim.x;
-        qitem = slot; seg = 0; j0 = 0; j1 = p.n_rtiles;
-        return true;
-    }
-    const int tr = r - rounds_full;                     // 0 or 1: piece of the tail
-    if (p.bal_p > 0) {
-        if (tr > 0 || c >= p.bal_rem * p.bal_p) return false;
-        const int i = c / p.bal_p;
-        seg = c - i * p.bal_p;
-        j0 = seg * p.bal_share;
-        j1 = min(p.n_rtiles, j0 + p.bal_share);
-        if (j0 >= j1) return false;
-        qitem = p.n_full + i;
-        slot = p.n_full + i * NABO_TC_MAX_SPLIT + seg;
-        return true;
-    }
-    if (tr > 1) return false;
-    const long long total = (long long)p.bal_rem * p.n_rtiles;
-    const long long lo = (long long)c * p.bal_share, hi = min(total, lo + p.bal_share);
-    if (lo >= hi) return false;
-    int i = (int)(lo / p.n_rtiles);
-    long long a = lo, b = min(hi, (long long)(i + 1) * p.n_rtiles);
-    if (tr == 1) {
-        if (b >= hi) return false;                      // the range does not reach into the next item
-        ++i; a = b; b = hi;
-    }
-    qitem = p.n_full + i;
-    seg = c - (int)(((long long)i * p.n_rtiles) / p.bal_share);
-    j0 = (int)(a - (long long)i * p.n_rtiles);
-    j1 = (int)(b - (long long)i * p.n_rtiles);
-    slot = p.n_full + i * NABO_TC_MAX_SPLIT + seg;
+    if (slot >= p.n_items * p.n_split) return false;
+    qitem = slot / p.n_split;
+    const int seg = slot - qitem * p.n_split;
+    j0 = (int)((long long)p.n_rtiles * seg / p.n_split);
+    j1 = (int)((long long)p.n_rtiles * (seg + 1) / p.n_split);
     return true;
 }
-// number of pieces item i of the tail is cut into (MODE 2)
-__device__ __forceinline__ int tail_pieces(const Params& p, int i) {
-    if (p.bal_p > 0) {
-        int n = 0;
-        for (int s_ = 0; s_ < p.bal_p; ++s_) n += (s_ * p.bal_share < p.n_rtiles) ? 1 : 0;
-        return n;
-    }
-    const long long first = ((long long)i * p.n_rtiles) / p.bal_share;
-    const long long last = ((long long)(i + 1) * p.n_rtiles - 1) / p.bal_share;
-    return (int)(last - first + 1);
-}
-__device__ __forceinline__ int sweep_tile(int jj, int start, int n_rtiles) {
-    const int j = jj + start;
-    return j >= n_rtiles ? j - n_rtiles : j;
-}
 
-template <int KSTEPS, int MODE>   // K steps of 16 known at compile time (0 = runtime loop); MODE: see work_piece
+template <int KSTEPS, bool SPLIT>   // K steps of 16 known at compile time (0 = runtime loop); SPLIT: see work_piece
 __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     Barriers* bars = reinterpret_cast<Barriers*>(smem + p.bar_off);
@@ -525,9 +340,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
 
     if (threadIdx.x == 0) {
         ptx::mbar_init(&bars->a_full, 1);
-        const int n_issuers = NABO_TC_ROTATE ? 1 : NQ;
-        ptx::mbar_init(&bars->a_empty, n_issuers);
-        for (int s = 0; s < 4; ++s) { ptx::mbar_init(&bars->b_full[s], 1); ptx::mbar_init(&bars->b_empty[s], n_issuers); }
+        ptx::mbar_init(&bars->a_empty, 1);
+        for (int s = 0; s < 4; ++s) { ptx::mbar_init(&bars->b_full[s], 1); ptx::mbar_init(&bars->b_empty[s], 1); }
         for (int q = 0; q < NACC; ++q) { ptx::mbar_init(&bars->acc_full[q], 1); ptx::mbar_init(&bars->acc_empty[q], 4); }
         ptx::fence_barrier_init();
     }
@@ -542,9 +356,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
         if (lane == 0) {
             uint32_t t = 0, it = 0;
             for (int wr = 0;; ++wr, ++it) {
-                int w, item, seg, j0, j1, start;
-                if (!work_piece<MODE>(p, blockIdx.x, wr, w, item, seg, j0, j1, start)) break;
-                ptx::mbar_wait_hint(&bars->a_empty, (it & 1) ^ 1, NABO_TC_SLEEP_NS);
+                int w, item, j0, j1;
+                if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
+                ptx::mbar_wait_hint(&bars->a_empty, (it & 1) ^ 1, SLEEP_NS);
                 ptx::mbar_arrive_expect_tx(&bars->a_full, NQ * a_tile_bytes);
                 for (int q = 0; q < NQ; ++q) {
                     const char* src = reinterpret_cast<const char*>(p.qa) + (size_t)(item * NQ + q) * a_tile_bytes;
@@ -554,17 +368,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                 }
                 for (int j = j0; j < j1; ++j, ++t) {
                     const uint32_t s = t % p.stages, use = t / p.stages;
-                    ptx::mbar_wait_hint(&bars->b_empty[s], (use & 1) ^ 1, NABO_TC_SLEEP_NS);   // far ahead of the consumers
+                    ptx::mbar_wait_hint(&bars->b_empty[s], (use & 1) ^ 1, SLEEP_NS);   // far ahead of the consumers
                     ptx::mbar_arrive_expect_tx(&bars->b_full[s], a_tile_bytes);
-                    const char* src = reinterpret_cast<const char*>(p.rb) + (size_t)sweep_tile(j, start, p.n_rtiles) * a_tile_bytes;
+                    const char* src = reinterpret_cast<const char*>(p.rb) + (size_t)j * a_tile_bytes;
                     char* dst = reinterpret_cast<char*>(smem + p.b_off) + (size_t)s * a_tile_bytes;
                     for (uint32_t o = 0; o < a_tile_bytes; o += 8192)
                         ptx::bulk_g2s(dst + o, src + o, min(8192u, a_tile_bytes - o), &bars->b_full[s]);
                 }
             }
         }
-#if NABO_TC_ROTATE
-    } else if (warp == MMA_WARP0) {
+    } else if (warp == MMA_WARP) {
         // ===================== MMA issuer: one warp, jobs in a fixed rotation =====================
         // Job n = (reference tile, query tile q = n % NQ) accumulates into buffer n % 4.  With one buffer more
         // than there are warpgroups, the MMAs of job n start as soon as the warpgroup of job n - 4 (the
@@ -579,12 +392,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
             const uint64_t bd0 = ptx::make_smem_desc(ptx::smem_u32(smem + p.b_off), lbo, sbo);
             uint32_t t = 0, it = 0, n = 0;
             for (int wr = 0;; ++wr, ++it) {
-                int w, item, seg, j0, j1, start;
-                if (!work_piece<MODE>(p, blockIdx.x, wr, w, item, seg, j0, j1, start)) break;
+                int w, item, j0, j1;
+                if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
                 ptx::mbar_wait(&bars->a_full, it & 1);
                 for (int j = j0; j < j1; ++j, ++t) {
                     const uint32_t s = t % p.stages, use = t / p.stages;
                     ptx::mbar_wait(&bars->b_full[s], use & 1);
+                    // descriptors differ only in the start-address field (16-byte units): one K step = 2 * LBO
                     const uint64_t bd1 = bd0 + (uint64_t)((s * a_tile_bytes) >> 4);
 #pragma unroll
                     for (int q = 0; q < NQ; ++q, ++n) {
@@ -615,53 +429,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                 }
             }
         }
-#else
-    } else if (warp >= MMA_WARP0 && warp < MMA_WARP0 + NQ) {
-        // ===================== MMA issuers: one thread per query tile =====================
-        // Each issuer sleeps on its own accumulator's mbarrier (hardware wake-up, no polling loop), so a
-        // warpgroup that is busy compacting never delays the other two; the tensor pipe interleaves the
-        // three instruction streams.  An operand stage is released when all NQ issuers have consumed it.
-        // The whole warp runs the loop so that descriptor arithmetic stays in the uniform datapath (no
-        // per-instruction R2UR traffic); only the elected lane issues tcgen05.mma / commit.
-        {
-            const int q = warp - MMA_WARP0;
-            const uint32_t idesc = ptx::make_idesc_f16(TILE, TILE);
-            const uint32_t lbo = TILE * 16, sbo = 128;
-            const uint32_t d_tmem = tmem_base + q * TILE;
-            const uint64_t ad0 = ptx::make_smem_desc(ptx::smem_u32(smem + p.a_off) + q * a_tile_bytes, lbo, sbo);
-            const uint64_t bd0 = ptx::make_smem_desc(ptx::smem_u32(smem + p.b_off), lbo, sbo);
-            uint32_t t = 0, it = 0;
-            for (int wr = 0;; ++wr, ++it) {
-                int w, item, seg, j0, j1, start;
-                if (!work_piece<MODE>(p, blockIdx.x, wr, w, item, seg, j0, j1, start)) break;
-                ptx::mbar_wait(&bars->a_full, it & 1);
-                for (int j = j0; j < j1; ++j, ++t) {
-                    const uint32_t s = t % p.stages, use = t / p.stages;
-                    ptx::mbar_wait(&bars->acc_empty[q], (t & 1) ^ 1);
-                    ptx::mbar_wait(&bars->b_full[s], use & 1);
-                    ptx::tc_fence_after();
-                    // descriptors differ only in the start-address field (16-byte units): one K step = 2 * LBO
-                    const uint64_t bd1 = bd0 + (uint64_t)((s * a_tile_bytes) >> 4);
-                    if (ptx::elect_one()) {
-                        if (KSTEPS > 0) {
-#pragma unroll
-                            for (int ks = 0; ks < KSTEPS; ++ks)
-                                ptx::mma_f16_ss(d_tmem, ad0 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4), idesc,
-                                                ks > 0 ? 1u : 0u);
-                        } else {
-                            for (int ks = 0; ks < ksteps; ++ks)
-                                ptx::mma_f16_ss(d_tmem, ad0 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4), idesc,
-                                                ks > 0 ? 1u : 0u);
-                        }
-                        ptx::mma_commit(&bars->acc_full[q]);
-                        ptx::mma_commit(&bars->b_empty[s]);
-                        if (j == j1 - 1) ptx::mma_commit(&bars->a_empty);
-                    }
-                    __syncwarp();
-                }
-            }
-        }
-#endif
     } else if (warp < N_EPI_WARPS) {
         // ===================== epilogue: fused top-K' selection =====================
         const int q = warp >> 2;                           // query tile of this warpgroup
@@ -673,33 +440,20 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
         uint32_t* hist = reinterpret_cast<uint32_t*>(smem + p.sort_off) + (size_t)warp * 256;
         TC_DECL;
         for (int wr = 0;; ++wr) {
-            int w, item, seg, j0, j1, start;
-            if (!work_piece<MODE>(p, blockIdx.x, wr, w, item, seg, j0, j1, start)) break;
+            int w, item, j0, j1;
+            if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
             unsigned long long* mybuf = p.cand_buf + ((size_t)w * NQ * TILE + slot) * CAP;
-#ifdef NABO_TC_DBG_NOHIT
-            float tau = -CUDART_INF_F;              // timing experiment: nothing is ever appended (results invalid)
-#else
             float tau = CUDART_INF_F;
-#endif
             int cnt = 0;
             TC_CLK(t_item);
             for (int j = j0; j < j1; ++j, ++t) {
-#if NABO_TC_ROTATE
                 const uint32_t job = t * NQ + q, buf = job & 3, acc_par = (job >> 2) & 1;
-#else
-                const uint32_t buf = q, acc_par = t & 1;
-#endif
                 const uint32_t taddr0 = tlane0 + buf * TILE;
                 TC_CLK(t_w);
-#if NABO_TC_EPI_SLEEP_NS
-                ptx::mbar_wait_hint(&bars->acc_full[buf], acc_par, NABO_TC_EPI_SLEEP_NS);
-#else
                 ptx::mbar_wait(&bars->acc_full[buf], acc_par);
-#endif
                 ptx::tc_fence_after();
                 TC_CLK_ADD(7, t_w);
-                const int jt = sweep_tile(j, start, p.n_rtiles);  // the reference tile this sweep position holds
-                NABO_DEV_ASSERT(jt >= 0 && jt < p.n_rtiles);
+                NABO_DEV_ASSERT(j >= 0 && j < p.n_rtiles);
                 // the compaction of every lane whose buffer passed `lim` (soft limit once per tile, after the
                 // accumulator has been handed back; hard limit otherwise: the next chunk may append 32 more)
                 auto compact_over = [&](int lim) {
@@ -713,35 +467,12 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                         const int n = __shfl_sync(0xffffffffu, cnt, src);
                         int nc;
                         float nt;
-                        compact_select<KPL>(gb, n, lane, p.kprime, p.soft - 8, hist, nc, nt);
+                        compact_select(gb, n, lane, p.kprime, p.soft - 8, hist, nc, nt);
                         if (lane == src) { cnt = nc; tau = nt; }
                         if (lane == 0) TC_STAT(4, 1);
                     }
                     TC_CLK_ADD(5, t_c);
                 };
-                auto release_acc = [&]() {      // accumulator fully read: hand it back to the MMA warp
-                    ptx::tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) ptx::mbar_arrive(&bars->acc_empty[buf]);
-                };
-#if NABO_TC_PIPE
-                // two register sets: the tcgen05.ld of the next chunk is in flight while the current one is filtered
-                uint32_t va[32], vb[32];
-                ptx::tmem_ld_32x32(taddr0, va);
-                ptx::tmem_ld_wait();
-#pragma unroll 1
-                for (int c = 0; c < TILE / CHUNK; c += 2) {
-                    ptx::tmem_ld_32x32(taddr0 + (c + 1) * CHUNK, vb);
-                    filter_chunk(va, (uint32_t)(jt * TILE + c * CHUNK), tau, mybuf, cnt TC_PASS);
-                    compact_over(CAP - CHUNK);
-                    ptx::tmem_ld_wait();
-                    if (c + 2 < TILE / CHUNK) ptx::tmem_ld_32x32(taddr0 + (c + 2) * CHUNK, va);
-                    else release_acc();
-                    filter_chunk(vb, (uint32_t)(jt * TILE + (c + 1) * CHUNK), tau, mybuf, cnt TC_PASS);
-                    compact_over(c + 2 < TILE / CHUNK ? CAP - CHUNK : p.soft);
-                    if (c + 2 < TILE / CHUNK) ptx::tmem_ld_wait();
-                }
-#else
 #pragma unroll 1
                 for (int c = 0; c < TILE / CHUNK; ++c) {
                     uint32_t vr[32];
@@ -749,13 +480,16 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                     ptx::tmem_ld_32x32(taddr0 + c * CHUNK, vr);
                     ptx::tmem_ld_wait();
                     TC_CLK_ADD(8, t_l);
-                    if (c == TILE / CHUNK - 1) release_acc();
+                    if (c == TILE / CHUNK - 1) {        // accumulator fully read: hand it back to the MMA warp
+                        ptx::tc_fence_before();
+                        __syncwarp();
+                        if (lane == 0) ptx::mbar_arrive(&bars->acc_empty[buf]);
+                    }
                     TC_CLK(t_f);
-                    filter_chunk(vr, (uint32_t)(jt * TILE + c * CHUNK), tau, mybuf, cnt TC_PASS);
+                    filter_chunk(vr, (uint32_t)(j * TILE + c * CHUNK), tau, mybuf, cnt TC_PASS);
                     TC_CLK_ADD(6, t_f);
                     compact_over(c == TILE / CHUNK - 1 ? p.soft : CAP - CHUNK);
                 }
-#endif
             }
             // item done: leave the buffer as it is; emit_kernel makes the final selection of every (query, range)
             // at full occupancy instead of 32 serial sorts per warp here, with the tensor pipe idle meanwhile
@@ -765,7 +499,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
             TC_CLK_ADD(9, t_e);
             TC_CLK_ADD(10, t_item);
             TC_FLUSH;
-            if (MODE == 0 && p.signal_round == wr + 1) {
+            if (!SPLIT && p.signal_round == wr + 1) {
                 // the full waves are done on this CTA: its buffers, counts and thresholds are in global memory
                 // (fence), the 12 epilogue warps meet on a named barrier, one thread lets the dependent grid - the
                 // re-rank of those queries - start while the last, partly filled wave is still running
@@ -781,60 +515,33 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
 }
 
 // Final selection: one warp per (query, reference range).  Sorts the buffer the sweep left behind, emits the K'
-// best as reference rows of the INPUT order (perm_r) into the query's INPUT row (perm_q) and the threshold every
-// other reference of the range is at or above.
-template <int MODE, bool PERM>     // PERM: operands were packed in locality order (perm_q / perm_r map back to input rows)
+// best reference rows and the threshold every other reference of the range is at or above.
 __global__ void __launch_bounds__(256)
-emit_kernel(const Params p, int n_slots_items, int n_seg) {
+emit_kernel(const Params p) {
     const int lane = threadIdx.x & 31;
     const long long wq = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);          // (buffer slot, query of the item)
-    if (wq >= (long long)n_slots_items * NQ * TILE) return;
+    if (wq >= (long long)p.n_items * p.n_split * NQ * TILE) return;
     const int w = (int)(wq / (NQ * TILE)), slot = (int)(wq - (long long)w * NQ * TILE);
-    int item, seg = 0, n_empty_after = 0;       // n_empty_after: segments of this query that hold nothing (MODE 2)
-    bool exists = true;
-    if (MODE == 0) {
-        item = w;
-    } else if (MODE == 1) {
-        item = w / n_seg;
-        seg = w - item * n_seg;
-    } else if (w < p.n_full) {
-        item = w;
-        n_empty_after = n_seg - 1;               // a whole item: segments 1.. stay empty
-    } else {
-        const int t = w - p.n_full, i = t / NABO_TC_MAX_SPLIT;
-        seg = t - i * NABO_TC_MAX_SPLIT;
-        item = p.n_full + i;
-        exists = seg < tail_pieces(p, i);
-    }
-    const long long qp = (long long)item * NQ * TILE + slot;                       // packed position
-    if (qp >= p.n_query || seg >= n_seg) return;
-    const long long qg = PERM ? (long long)p.perm_q[qp] : qp;                     // input row
-    if (!exists) {                               // no such piece: an empty list that rejected nothing
-        for (int i = lane; i < p.kc_out; i += 32) p.cand_idx[(qg * n_seg + seg) * p.kc_out + i] = -1;
-        if (lane == 0) p.cert_tau[(long long)seg * p.n_query + qg] = CUDART_INF_F;
-        return;
-    }
+    const int item = w / p.n_split, seg = w - item * p.n_split;
+    const long long qg = (long long)item * NQ * TILE + slot;                       // query row
+    if (qg >= p.n_query) return;
     const int n = p.cand_cnt[wq];
     const float old_tau = p.cand_tau[wq];
     NABO_DEV_ASSERT(n >= 0 && n <= CAP);
     uint32_t ks[KPL], kpl[KPL];
     int nc;
     float nt;
-    compact_sort_inline<KPL>(p.cand_buf + (size_t)wq * CAP, n, lane, p.kprime, ks, kpl, nc, nt);
+    compact_sort_inline(p.cand_buf + (size_t)wq * CAP, n, lane, p.kprime, ks, kpl, nc, nt);
 #pragma unroll
     for (int u = 0; u < 4; ++u) {                 // kc_out <= 128
         const int i = u * 32 + lane;
         if (i < p.kc_out) {
             int32_t id = -1;
-            if (i < nc && kpl[u] < (uint32_t)p.n_ref) id = PERM ? (int32_t)p.perm_r[kpl[u]] : (int32_t)kpl[u];
-            p.cand_idx[(qg * n_seg + seg) * p.kc_out + i] = id;
+            if (i < nc && kpl[u] < (uint32_t)p.n_ref) id = (int32_t)kpl[u];
+            p.cand_idx[(qg * p.n_split + seg) * p.kc_out + i] = id;
         }
     }
     if (lane == 0) p.cert_tau[(long long)seg * p.n_query + qg] = n >= p.kprime ? nt : old_tau;
-    for (int e = 1; e <= n_empty_after; ++e) {
-        for (int i = lane; i < p.kc_out; i += 32) p.cand_idx[(qg * n_seg + e) * p.kc_out + i] = -1;
-        if (lane == 0) p.cert_tau[(long long)e * p.n_query + qg] = CUDART_INF_F;
-    }
 }
 
 }  // namespace tc
@@ -856,42 +563,6 @@ int nabo_tc_kprime(int k, int drop_first) {
     int kprime = ksel + (ksel / 4 > 8 ? ksel / 4 : 8);
     if (kprime > tc::MAX_KPRIME) kprime = tc::MAX_KPRIME;
     return kprime;
-}
-
-// NABO_TC_ORDER=1 switches the locality order on.  Measured on B200 (tools/probe_tc_scan.py, probe_tc_stats.py):
-// it cuts the warp chunks that take the append path from 70 % to 8 % at 100 k x 100 k and the appends per query
-// from 506 to 373, but the kernel is bound by the TMEM read-out (64 B/clk/SM) plus the compactions, not by the
-// hit path, so the candidate pass gains 4 % there and the ten extra launches cost as much; off by default.
-static bool nabo_tc_order_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("NABO_TC_ORDER");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v != 0;
-}
-
-// NABO_TC_BALANCE=1 switches the balanced last wave (MODE 2) on.  Measured on B200 (tools/probe_fast.py): correct
-// (tests/test_gpu_tc.py::test_balanced_last_wave_equals_exact) but not a gain - at 100 k x 100 k the pieces start with
-// a cold threshold (candidate kernel 3.79 -> 4.24 ms) and the re-rank walks three K' lists per query (0.87 -> 1.43 ms);
-// at 200 k x 1.25 M the kernel gains 3 % and the re-rank loses as much.  Off by default.
-// NABO_TC_TAIL_OVERLAP=0 keeps the candidate pass one launch (no re-rank of the full waves under the last wave).
-static bool nabo_tc_tail_overlap_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("NABO_TC_TAIL_OVERLAP");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v != 0;
-}
-
-static bool nabo_tc_balance_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("NABO_TC_BALANCE");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v != 0;
 }
 
 static int tc_grid(int n_items) {
@@ -942,11 +613,6 @@ size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_fi
     b += nabo_align_up((size_t)n_items * NABO_TC_MAX_SPLIT * tc::NQ * tc::TILE * (tc::CAP * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
     b += nabo_align_up((size_t)n_query * kprime * 4 * NABO_TC_MAX_SPLIT, 256);   // candidate indices (per reference range)
     b += nabo_align_up((size_t)n_query * 4 * NABO_TC_MAX_SPLIT, 256) + nabo_align_up((size_t)n_query * 4, 256);   // cert tau, fail rows
-    // locality order: cluster ids + row numbers (in / sorted) of both operands, radix scratch, centroids, tables
-    b += 4 * (nabo_align_up((size_t)n_query * 4, 256) + nabo_align_up((size_t)n_ref * 4, 256));
-    b += nabo_align_up(nabo_radix_pass_scratch_bytes(n_query > n_ref ? n_query : n_ref), 256);
-    b += nabo_align_up((size_t)tc::N_CEN * tc::CEN_DIMS * 4, 256) + nabo_align_up((size_t)(tc::N_CEN + 1) * 4, 256) +
-         nabo_align_up((size_t)n_items * 4, 256);
     b += 4096;
     return b;
 }
@@ -957,12 +623,11 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
                        int metric, const uint8_t* mask, int drop_first, int* n_split_io, NaboArena& ar, int32_t** cand_idx_out,
                        int* kprime_out, float** cert_tau_out, double** qn2_out, double** scal_out, int* launches,
                        NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out, NaboTailSplit* tail) {
-    // raw_out != NULL: when every query has ONE buffer in input order (MODE 0, no locality order, K' <= 64, 128-key
-    // buffers) the final selection is left to the re-rank kernel: raw_out is filled and no emit kernel runs.
-    // *n_split_io in: reference pieces per item when there are few items (nabo_tc_split), or 0 = one piece and no
-    // balancing of the last wave (the public candidate entry point: one K' list per query); out: K' lists per query
+    // raw_out != NULL: when every query has ONE buffer (no reference split, K' <= 64) the final selection is left to
+    // the re-rank kernel: raw_out is filled and no emit kernel runs.
+    // *n_split_io in: reference pieces per item when there are few items (nabo_tc_split), or 0 = one piece (the
+    // public candidate entry point: one K' list per query); out: K' lists per query
     int n_split = *n_split_io;
-    const bool may_balance = n_split >= 1;
     const int kp = tc::kp_for(g);
     const tc::SmemPlan pl = tc::plan_smem(kp);
     const size_t tb = tc::tile_bytes(kp);
@@ -971,161 +636,86 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
     const int kprime = nabo_tc_kprime(k, drop_first);
     if (n_split < 1 || n_split > NABO_TC_MAX_SPLIT) n_split = 1;
-    const int grid_all = tc_grid(n_items * n_split);
-    // MODE 2 (see work_piece): more items than CTAs, a last wave between 5 % and 90 % full, room for three K' lists
-    int mode = n_split > 1 ? 1 : 0, n_full = n_items, bal_rem = 0, bal_share = 0, bal_p = 0;
-    if (mode == 0 && may_balance && n_items > grid_all && 3 * kprime <= 128 && n_rtiles >= 96 && nabo_tc_balance_enabled()) {
-        const int rem = n_items % grid_all;
-        if (rem > 0 && rem * 20 >= grid_all && rem * 10 <= grid_all * 9) {
-            mode = 2;
-            n_full = n_items - rem;
-            bal_rem = rem;
-            if (rem * 2 >= grid_all) {                       // contiguous ranges, <= 3 pieces per item
-                bal_p = 0;
-                bal_share = (int)(((long long)rem * n_rtiles + grid_all - 1) / grid_all);
-            } else {                                     // aligned pieces
-                bal_p = grid_all / rem < NABO_TC_MAX_SPLIT ? grid_all / rem : NABO_TC_MAX_SPLIT;
-                bal_share = (n_rtiles + bal_p - 1) / bal_p;
-            }
-        }
-    }
-    const int n_seg = mode == 2 ? NABO_TC_MAX_SPLIT : n_split;
-    const int n_slot_items = mode == 2 ? n_full + bal_rem * NABO_TC_MAX_SPLIT : n_items * n_split;
+    const int grid = tc_grid(n_items * n_split);
 
     __half* qa = (__half*)ar.take<char>((size_t)n_qtiles * tb);
     __half* rb = (__half*)ar.take<char>((size_t)n_rtiles * tb);
     double* qnorm = ar.take<double>(n_query);
     double* qn2 = ar.take<double>(n_query);
     double* rnorm = ar.take<double>(n_ref);
-    const size_t n_slots = (size_t)n_slot_items * tc::NQ * tc::TILE;
+    const size_t n_slots = (size_t)n_items * n_split * tc::NQ * tc::TILE;
     unsigned long long* cbuf = ar.take<unsigned long long>(n_slots * tc::CAP);
     int* ccnt = ar.take<int>(n_slots);
     float* ctau = ar.take<float>(n_slots);
-    int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_seg);
-    float* tau = ar.take<float>((size_t)n_query * n_seg);
+    int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_split);
+    float* tau = ar.take<float>((size_t)n_query * n_split);
     double* scal = ar.take<double>(4);
     unsigned int* maxbits = ar.take<unsigned int>(2);
     if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the tensor-core pass");
-
-    // locality order (see order kernels above): only worth its ~10 small launches on a real sweep
-    const bool ordered = mode == 0 && n_rtiles >= 64 && nabo_tc_order_enabled();
-    uint32_t *perm_q = nullptr, *perm_r = nullptr;
-    int* item_start = nullptr;
-    if (ordered) {
-        uint32_t* cl_q = ar.take<uint32_t>(n_query);
-        uint32_t* io_q = ar.take<uint32_t>(n_query);
-        uint32_t* scl_q = ar.take<uint32_t>(n_query);
-        perm_q = ar.take<uint32_t>(n_query);
-        uint32_t* cl_r = ar.take<uint32_t>(n_ref);
-        uint32_t* io_r = ar.take<uint32_t>(n_ref);
-        uint32_t* scl_r = ar.take<uint32_t>(n_ref);
-        perm_r = ar.take<uint32_t>(n_ref);
-        char* rscratch = ar.take<char>(nabo_radix_pass_scratch_bytes(n_query > n_ref ? n_query : n_ref));
-        float* cen = ar.take<float>((size_t)tc::N_CEN * tc::CEN_DIMS);
-        int* first_r = ar.take<int>(tc::N_CEN + 1);
-        item_start = ar.take<int>(n_items);
-        if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the tensor-core pass");
-        const int gs = g < tc::CEN_DIMS ? g : tc::CEN_DIMS;
-        const int cosine = metric == NABO_COSINE ? 1 : 0;
-        tc::centroid_gather_kernel<<<tc::N_CEN, tc::CEN_DIMS, 0, st>>>(r, ldr, n_ref, gs, cosine, cen);
-        tc::cluster_assign_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(q, ldq, n_query, gs, cosine, cen, cl_q, io_q);
-        tc::cluster_assign_kernel<<<(n_ref + 255) / 256, 256, 0, st>>>(r, ldr, n_ref, gs, cosine, cen, cl_r, io_r);
-        NABO_LAUNCH_CHECK("tc order kernels");
-        int rc = nabo_radix_pass_launch(cl_q, io_q, n_query, 0, rscratch, scl_q, perm_q, st);
-        if (rc) return rc;
-        rc = nabo_radix_pass_launch(cl_r, io_r, n_ref, 0, rscratch, scl_r, perm_r, st);
-        if (rc) return rc;
-        tc::cluster_first_kernel<<<1, 128, 0, st>>>(scl_r, n_ref, first_r);
-        tc::item_start_kernel<<<(n_items + 127) / 128, 128, 0, st>>>(scl_q, n_query, first_r, n_items, n_rtiles, item_start);
-        NABO_LAUNCH_CHECK("tc order kernels");
-        *launches += 11;
-    }
 
     NABO_CUDA(cudaMemsetAsync(maxbits, 0, 2 * sizeof(unsigned int), st));
     tc::norms_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(q, ldq, n_query, g, qnorm, maxbits);
     tc::norms_kernel<<<(n_ref + 255) / 256, 256, 0, st>>>(r, ldr, n_ref, g, rnorm, maxbits + 1);
     tc::scale_kernel<<<1, 1, 0, st>>>(maxbits, maxbits + 1, metric == NABO_COSINE ? 1 : 0, scal);
-    tc::pack_kernel<true><<<n_qtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(q, ldq, n_query, g, kp, qnorm, scal, nullptr, perm_q, qa, qn2);
-    tc::pack_kernel<false><<<n_rtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(r, ldr, n_ref, g, kp, rnorm, scal, mask, perm_r, rb, nullptr);
+    tc::pack_kernel<true><<<n_qtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(q, ldq, n_query, g, kp, qnorm, scal, nullptr, qa, qn2);
+    tc::pack_kernel<false><<<n_rtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(r, ldr, n_ref, g, kp, rnorm, scal, mask, rb, nullptr);
     NABO_LAUNCH_CHECK("tc pack kernels");
     tm.end(3);
 
     tc::Params p;
     p.qa = qa; p.rb = rb;
     p.n_query = n_query; p.n_ref = n_ref; p.kp = kp; p.n_items = n_items; p.n_rtiles = n_rtiles;
-    p.signal_round = 0;
     p.stages = pl.stages; p.kprime = kprime; p.kc_out = kprime; p.n_split = n_split;
-    p.n_full = n_full; p.bal_rem = bal_rem; p.bal_share = bal_share; p.bal_p = bal_p;
     p.cand_buf = cbuf; p.cand_cnt = ccnt; p.cand_tau = ctau; p.cand_idx = cand; p.cert_tau = tau;
-    p.perm_q = perm_q; p.perm_r = perm_r; p.item_start = item_start;
-    {
-        const char* e = getenv("NABO_TC_DBG");
-        p.dbg = e ? atoi(e) : 0;
-    }
     p.a_off = pl.a_off; p.b_off = pl.b_off; p.sort_off = pl.sort_off; p.bar_off = pl.bar_off;
     p.soft = tc::CAP - tc::CHUNK - 16 > kprime ? tc::CAP - tc::CHUNK - 16 : kprime;
-    {
-        const char* e = getenv("NABO_TC_SOFT");      // development: compaction trigger (keys in the buffer at a tile end)
-        if (e && atoi(e) >= kprime + 8 && atoi(e) <= tc::CAP - tc::CHUNK) p.soft = atoi(e);
+    // Partly filled last wave (see NaboTailSplit): every CTA signals after its last full-wave item when the caller can
+    // use the gap - the fused re-rank path only, at least two waves, at least 16 SMs idle in the last one.
+    const bool fused = raw_out && n_split == 1 && kprime <= 64;
+    const int rem_items = n_items % grid;
+    const bool tail_applies = tail && fused && n_items > grid && rem_items > 0 && grid - rem_items >= 16;
+    const bool overlap = tail_applies && !tail->dry;
+    p.signal_round = overlap ? n_items / grid : 0;
+    if (tail) {
+        tail->applies = tail_applies ? 1 : 0;
+        tail->rows_full = overlap ? (n_items - rem_items) * tc::NQ * tc::TILE : 0;
     }
-#define NABO_TC_LAUNCH1(KS, MD)                                                                                    \
+#define NABO_TC_LAUNCH1(KS, SPLIT)                                                                                 \
     do {                                                                                                           \
-        NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, MD>,                                              \
+        NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, SPLIT>,                                           \
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.total));               \
-        tc::candidates_kernel<KS, MD><<<grid, tc::NTHREADS, pl.total, st>>>(p);                                    \
+        tc::candidates_kernel<KS, SPLIT><<<grid, tc::NTHREADS, pl.total, st>>>(p);                                 \
     } while (0)
 #define NABO_TC_LAUNCH(KS)                                                                                         \
     do {                                                                                                           \
-        if (mode == 1) NABO_TC_LAUNCH1(KS, 1);                                                                     \
-        else if (mode == 2) NABO_TC_LAUNCH1(KS, 2);                                                                \
-        else NABO_TC_LAUNCH1(KS, 0);                                                                               \
+        if (n_split > 1) NABO_TC_LAUNCH1(KS, true);                                                                \
+        else NABO_TC_LAUNCH1(KS, false);                                                                           \
     } while (0)
-    // Partly filled last wave (see NaboTailSplit): every CTA signals after its last full-wave item when the caller can
-    // use the gap - the fused re-rank path only (one buffer per query, input order), at least two waves, at least
-    // 16 SMs idle in the last one.
-    const bool fused = raw_out && mode == 0 && !perm_q && kprime <= 64 && tc::CAP == 128;
-    const int grid = grid_all;
-    const int rem_items = n_items % grid_all;
-    if (tail) tail->rows_full = 0, tail->applies = 0;
-    bool split_tail = tail && fused && n_items > grid_all && rem_items > 0 && grid_all - rem_items >= 16 &&
-                      nabo_tc_tail_overlap_enabled();
-    if (split_tail) {
-        tail->applies = 1;
-        if (tail->dry) split_tail = false;
-    }
-    if (split_tail) {
-        p.signal_round = n_items / grid_all;
-        tail->rows_full = (n_items - rem_items) * tc::NQ * tc::TILE;
-    }
     if (kp == 160) NABO_TC_LAUNCH(10);        // g = 50 (BASELINE configs 2-5)
     else if (kp == 80) NABO_TC_LAUNCH(5);     // g = 25 (config 1)
     else NABO_TC_LAUNCH(0);
 #undef NABO_TC_LAUNCH1
 #undef NABO_TC_LAUNCH
     NABO_LAUNCH_CHECK("candidates_kernel");
-    if (!split_tail) tm.end(0);    // the final selection below is timed with the re-rank stage; with a dependent launch the
+    if (!overlap) tm.end(0);       // the final selection below is timed with the re-rank stage; with a dependent launch the
                                    // caller ends the stage after that launch (nothing may sit between the two kernels)
-    if (raw_out) raw_out->buf = nullptr;
-    if (raw_out && mode == 0 && !perm_q && kprime <= 64 && tc::CAP == 128) {
+    if (fused) {
         raw_out->buf = cbuf; raw_out->cnt = ccnt; raw_out->tau = ctau; raw_out->kprime = kprime;
         *cand_idx_out = cand; *kprime_out = kprime; *cert_tau_out = tau; *qn2_out = qn2; *scal_out = scal;
         *launches += 6;
         *n_split_io = 1;
         return 0;
     }
-    const unsigned egrid = (unsigned)((n_slots + 7) / 8);
-    if (mode == 0 && perm_q) tc::emit_kernel<0, true><<<egrid, 256, 0, st>>>(p, n_slot_items, n_seg);
-    else if (mode == 0) tc::emit_kernel<0, false><<<egrid, 256, 0, st>>>(p, n_slot_items, n_seg);
-    else if (mode == 1) tc::emit_kernel<1, false><<<egrid, 256, 0, st>>>(p, n_slot_items, n_seg);
-    else tc::emit_kernel<2, false><<<egrid, 256, 0, st>>>(p, n_slot_items, n_seg);
+    if (raw_out) raw_out->buf = nullptr;
+    tc::emit_kernel<<<(unsigned)((n_slots + 7) / 8), 256, 0, st>>>(p);
     NABO_LAUNCH_CHECK("emit_kernel");
     *launches += 1;
-    if (n_seg > 1) {
-        int rc = nabo_tau_min_launch(tau, n_query, n_seg, st);
+    if (n_split > 1) {
+        int rc = nabo_tau_min_launch(tau, n_query, n_split, st);
         if (rc) return rc;
         *launches += 1;
     }
-    *n_split_io = n_seg;
+    *n_split_io = n_split;
     *cand_idx_out = cand; *kprime_out = kprime; *cert_tau_out = tau; *qn2_out = qn2; *scal_out = scal;
     *launches += 6;
     return 0;

@@ -23,6 +23,5 @@ for n, m in shapes:
     ms = a.elapsed_time(b) / 3
     waves = -(-(-(-n // 384)) // 148)
     jobs = waves * 3 * -(-m // 128)
-    print("k=%d %s order=%s  %7d x %7d: %.3f ms  %.3e pairs/s  %.3f us per (128x128) job on the critical SM" % (
-        k, os.path.basename(os.environ.get("NABO_B200_LIB", "product")), os.environ.get("NABO_TC_ORDER", "1"), n, m, ms,
-        n * m / ms * 1e3, ms * 1e3 / jobs))
+    print("k=%d %s  %7d x %7d: %.3f ms  %.3e pairs/s  %.3f us per (128x128) job on the critical SM" % (
+        k, os.path.basename(os.environ.get("NABO_B200_LIB", "product")), n, m, ms, n * m / ms * 1e3, ms * 1e3 / jobs))
