@@ -92,6 +92,7 @@ int nabo_knn(const double* q, int ldq, const double* r, int ldr, int n_query, in
  * out_tau (n_query) = score threshold every non-candidate is at or above (+inf = no
  * reference was rejected); optional out_qn2 (n_query) and out_scal (4 doubles: scale,
  * 1/scale, max scaled reference norm, cosine flag) are what the certificate uses.
+ * Takes 1 <= g <= 128 and k + drop_first + 8 <= 96; NABO_EUNSUPPORTED otherwise.
  * nabo_knn(mode = NABO_MODE_FAST) = this + nabo_rerank_exact + certificate + fallback. */
 int nabo_knn_candidates_width(int k, int drop_first);
 size_t nabo_knn_candidates_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first);

@@ -108,7 +108,7 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
     int kprime = 0, launches = 0;
     NaboCandBuf raw;
     raw.buf = nullptr;
-    int n_split = nabo_tc_split(n_query, n_ref);              // > 1 only when there are fewer query items than SMs
+    int n_split = nabo_tc_split(n_query, n_ref, g);              // > 1 only when there are fewer query items than SMs
     while (n_split > 1 && n_split * nabo_tc_kprime(k, drop_first) > 128) --n_split;     // the re-rank takes <= 128 candidates
     // the failure list first: the re-rank of the full waves may start while the candidate pass is still running
     int* fail_rows = ar.take<int>(n_query);

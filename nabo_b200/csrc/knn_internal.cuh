@@ -107,7 +107,7 @@ bool nabo_tc_supported(int g, int k, int drop_first);
 int nabo_tc_kprime(int k, int drop_first);
 size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first);
 #define NABO_TC_MAX_SPLIT 3
-int nabo_tc_split(int n_query, int n_ref);
+int nabo_tc_split(int n_query, int n_ref, int g);
 int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                        int metric, const uint8_t* mask, int drop_first, int* n_split_io, NaboArena& ar, int32_t** cand_idx_out,
                        int* kprime_out, float** cert_tau_out, double** qn2_out, double** scal_out, int* launches,

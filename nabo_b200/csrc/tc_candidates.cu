@@ -16,6 +16,10 @@
 //   warp 12  TMEM allocator, then TMA producer: A tiles once per item, B (reference) tiles through a ring
 //   warp 13  MMA issuer: the three query tiles rotate over FOUR accumulators, so the MMAs of a warpgroup's
 //            next tile run while it still reads the current one (warps 14-15 idle)
+// Wide plan (53 <= g <= 128, where three query tiles and two whole reference tiles no longer fit in shared memory):
+// NQ=2 query tiles (epilogue warps 0-7, each warpgroup double-buffered over the four accumulators) and the reference
+// tile streamed through the ring in K-slabs of SLAB K steps - the packed layout is K-chunk-major, so a slab is one
+// contiguous span (see plan_smem).
 // The epilogue keeps, per query, a running threshold tau (register) and a private
 // candidate buffer of CAP keys in L2-resident global memory; a tile chunk is first reduced
 // with FMNMX3 and only chunks holding a score < tau take the append path.  When a buffer
@@ -32,9 +36,8 @@
 namespace tc {
 
 constexpr int TILE = 128;           // rows per operand tile (UMMA M and N)
-constexpr int NQ = 3;               // query tiles per work item
-constexpr int NTHREADS = 512;
-constexpr int N_EPI_WARPS = 4 * NQ;  // warps 0..11: epilogue (TMEM lane quarter = warp % 4)
+constexpr int NTHREADS = 512;        // epilogue: warps 0 .. 4 NQ - 1 (TMEM lane quarter = warp % 4)
+constexpr int MAX_G = 128;           // widest PCA space of the tensor-core pass (certificate constant checked up to here)
 constexpr int PRODUCER_WARP = 12;    // highest warp ids on their schedulers: the arbiter favours them,
 constexpr int MMA_WARP = 13;         // so the single-thread producer / issuer are never starved
 constexpr int TMEM_WARP = 12;
@@ -47,31 +50,58 @@ static_assert(CAP == sel::CAP, "the fused re-rank (exact.cu) reads the candidate
 constexpr int CHUNK = 32;           // columns per tcgen05.ld
 constexpr int MAX_KPRIME = 96;      // K' lists go to the re-rank, which takes at most 128 candidates per query
 constexpr int SLEEP_NS = 2000;      // suspend-time hint of the producer's mbarrier waits
-// accumulators in TMEM (128 columns each): the NQ query tiles share NQ + 1 buffers in a fixed rotation
+// accumulators in TMEM (128 columns each): the NQ query tiles share four buffers in a fixed rotation
 // (job n = tile * NQ + q uses buffer n % 4), so the MMAs of a warpgroup's next tile run while it is still
 // reading the current one
 constexpr int NACC = 4;
+constexpr int MAX_STAGES = 4;        // reference ring stages (b_full / b_empty of Barriers)
+constexpr uint32_t KSTEP_BYTES = TILE * 16 * 2;   // one K step (16 columns) of a packed tile: two 16-byte K chunks
 
 __host__ __device__ inline int kp_for(int g) { return (3 * g + 3 + 15) / 16 * 16; }
 __host__ __device__ inline size_t tile_bytes(int kp) { return (size_t)TILE * kp * 2; }
 
+// The tile plan of a PCA width g - the one place that decides it:
+//   g <= 52       NQ = 3 query tiles, whole reference tiles per ring stage (2 - 4 stages)
+//   53 <= g <= 128  NQ = 2 query tiles, reference slabs of 4 or 2 K steps (16 / 8 KB) per stage: the slab width with
+//                 the most bytes in flight (at most MAX_STAGES stages, at least 2), the wider one on a tie.  Slabs of
+//                 1 K step would never win up to g = 128 (g = 128 leaves 17.5 KB: 2 x 8 KB).
+// stages = 0: no plan fits (g > 128).
 struct SmemPlan {
+    int nq;              // query tiles per work item
+    int slab;            // K steps per reference slab, 0 = whole tiles
     int stages;
+    size_t stage_bytes;
     size_t a_off, b_off, sort_off, bar_off, total;
 };
-inline SmemPlan plan_smem(int kp) {
+inline SmemPlan plan_smem(int g) {
+    const int kp = kp_for(g);
+    const size_t bars = 512;
+    const size_t budget = 227 * 1024 - 1024;   // keep 1 KB for alignment slack
+    auto room = [&](int nq) {                  // what nq query tiles, their warps' histograms and the barriers leave
+        const size_t used = nq * tile_bytes(kp) + (size_t)4 * nq * 256 * 4 + bars;
+        return budget > used ? budget - used : (size_t)0;
+    };
     SmemPlan p;
-    size_t a = NQ * tile_bytes(kp);
-    size_t sort = (size_t)N_EPI_WARPS * 256 * 4;     // per-warp histogram
-    size_t bars = 512;
-    size_t budget = 227 * 1024 - 1024;   // keep 1 KB for alignment slack
-    size_t left = budget > a + sort + bars ? budget - a - sort - bars : 0;
-    p.stages = (int)(left / tile_bytes(kp));
-    if (p.stages > 4) p.stages = 4;
+    p.nq = 3;
+    p.slab = 0;
+    p.stage_bytes = tile_bytes(kp);
+    p.stages = (int)(room(3) / p.stage_bytes);
+    if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
+    if (p.stages < 2) {
+        p.nq = 2;
+        p.stages = 0;
+        for (int slab = 4; slab >= 2 && g <= MAX_G; slab /= 2) {
+            const size_t sb = (size_t)slab * KSTEP_BYTES;
+            int st = (int)(room(2) / sb);
+            if (st > MAX_STAGES) st = MAX_STAGES;
+            if (st >= 2 && st * sb > p.stages * p.stage_bytes) { p.slab = slab; p.stages = st; p.stage_bytes = sb; }
+        }
+    }
+    const size_t a = p.nq * tile_bytes(kp);
     p.a_off = 0;
     p.b_off = a;
-    p.sort_off = a + (size_t)p.stages * tile_bytes(kp);
-    p.bar_off = p.sort_off + sort;
+    p.sort_off = a + (size_t)p.stages * p.stage_bytes;
+    p.bar_off = p.sort_off + (size_t)4 * p.nq * 256 * 4;     // per-warp histogram
     p.total = p.bar_off + bars;
     return p;
 }
@@ -239,7 +269,7 @@ struct Params {
 
 struct Barriers {
     uint64_t a_full, a_empty;
-    uint64_t b_full[4], b_empty[4];
+    uint64_t b_full[MAX_STAGES], b_empty[MAX_STAGES];
     uint64_t acc_full[NACC], acc_empty[NACC];
     uint32_t tmem_base;
 };
@@ -330,18 +360,24 @@ __device__ __forceinline__ bool work_piece(const Params& p, int c, int r, int& s
     return true;
 }
 
-template <int KSTEPS, bool SPLIT>   // K steps of 16 known at compile time (0 = runtime loop); SPLIT: see work_piece
+// KSTEPS: K steps of 16 known at compile time (0 = runtime loop); SPLIT: see work_piece; NQ: query tiles per work item;
+// SLAB: K steps per reference slab (0 = whole reference tiles).  The tile plan (plan_smem) picks NQ and SLAB.
+template <int KSTEPS, bool SPLIT, int NQ = 3, int SLAB = 0>
 __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p) {
+    static_assert(NQ * 4 <= PRODUCER_WARP && (SLAB == 0 || KSTEPS == 0), "tile plan");
+    constexpr int N_EPI_WARPS = 4 * NQ;
     extern __shared__ __align__(1024) uint8_t smem[];
     Barriers* bars = reinterpret_cast<Barriers*>(smem + p.bar_off);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int ksteps = p.kp / 16;
     const uint32_t a_tile_bytes = (uint32_t)tile_bytes(p.kp);
+    const int nslab = SLAB ? (ksteps + SLAB - 1) / SLAB : 1;       // ring stages per reference tile
+    const uint32_t stage_bytes = SLAB ? SLAB * KSTEP_BYTES : a_tile_bytes;
 
     if (threadIdx.x == 0) {
         ptx::mbar_init(&bars->a_full, 1);
         ptx::mbar_init(&bars->a_empty, 1);
-        for (int s = 0; s < 4; ++s) { ptx::mbar_init(&bars->b_full[s], 1); ptx::mbar_init(&bars->b_empty[s], 1); }
+        for (int s = 0; s < MAX_STAGES; ++s) { ptx::mbar_init(&bars->b_full[s], 1); ptx::mbar_init(&bars->b_empty[s], 1); }
         for (int q = 0; q < NACC; ++q) { ptx::mbar_init(&bars->acc_full[q], 1); ptx::mbar_init(&bars->acc_empty[q], 4); }
         ptx::fence_barrier_init();
     }
@@ -366,15 +402,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                     for (uint32_t o = 0; o < a_tile_bytes; o += 8192)
                         ptx::bulk_g2s(dst + o, src + o, min(8192u, a_tile_bytes - o), &bars->a_full);
                 }
-                for (int j = j0; j < j1; ++j, ++t) {
-                    const uint32_t s = t % p.stages, use = t / p.stages;
-                    ptx::mbar_wait_hint(&bars->b_empty[s], (use & 1) ^ 1, SLEEP_NS);   // far ahead of the consumers
-                    ptx::mbar_arrive_expect_tx(&bars->b_full[s], a_tile_bytes);
-                    const char* src = reinterpret_cast<const char*>(p.rb) + (size_t)j * a_tile_bytes;
-                    char* dst = reinterpret_cast<char*>(smem + p.b_off) + (size_t)s * a_tile_bytes;
-                    for (uint32_t o = 0; o < a_tile_bytes; o += 8192)
-                        ptx::bulk_g2s(dst + o, src + o, min(8192u, a_tile_bytes - o), &bars->b_full[s]);
-                }
+                for (int j = j0; j < j1; ++j)
+                    for (int sl = 0; sl < nslab; ++sl, ++t) {
+                        // slab sl: K chunks [2 SLAB sl, 2 SLAB (sl + 1)) of tile j, one contiguous span (the last may be shorter)
+                        const uint32_t s = t % p.stages, use = t / p.stages;
+                        const uint32_t off = sl * stage_bytes, bytes = min(stage_bytes, a_tile_bytes - off);
+                        ptx::mbar_wait_hint(&bars->b_empty[s], (use & 1) ^ 1, SLEEP_NS);   // far ahead of the consumers
+                        ptx::mbar_arrive_expect_tx(&bars->b_full[s], bytes);
+                        const char* src = reinterpret_cast<const char*>(p.rb) + (size_t)j * a_tile_bytes + off;
+                        char* dst = reinterpret_cast<char*>(smem + p.b_off) + (size_t)s * stage_bytes;
+                        for (uint32_t o = 0; o < bytes; o += 8192)
+                            ptx::bulk_g2s(dst + o, src + o, min(8192u, bytes - o), &bars->b_full[s]);
+                    }
             }
         }
     } else if (warp == MMA_WARP) {
@@ -382,7 +421,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
         // Job n = (reference tile, query tile q = n % NQ) accumulates into buffer n % 4.  With one buffer more
         // than there are warpgroups, the MMAs of job n start as soon as the warpgroup of job n - 4 (the
         // PREVIOUS query tile, one reference tile back) has read its accumulator - about a third of a period
-        // before warpgroup q finishes its current tile - so they complete while q is still filtering.
+        // before warpgroup q finishes its current tile - so they complete while q is still filtering.  With NQ = 2
+        // job n - 4 is the SAME query tile two reference tiles back: each warpgroup has a full double buffer.
         // The whole warp runs the loop (descriptor arithmetic in the uniform datapath); only the elected
         // lane issues tcgen05.mma / commit.
         {
@@ -395,38 +435,50 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                 int w, item, j0, j1;
                 if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
                 ptx::mbar_wait(&bars->a_full, it & 1);
-                for (int j = j0; j < j1; ++j, ++t) {
-                    const uint32_t s = t % p.stages, use = t / p.stages;
-                    ptx::mbar_wait(&bars->b_full[s], use & 1);
-                    // descriptors differ only in the start-address field (16-byte units): one K step = 2 * LBO
-                    const uint64_t bd1 = bd0 + (uint64_t)((s * a_tile_bytes) >> 4);
+                for (int j = j0; j < j1; ++j, n += NQ, ++t)
+                    for (int sl = 0; sl < nslab; ++sl) {
+                        // slab sl of reference tile j against every query tile; with slabs the NQ accumulators of tile j
+                        // are all open until its last slab
+                        const uint32_t u = t * nslab + sl, s = u % p.stages, use = u / p.stages;
+                        ptx::mbar_wait(&bars->b_full[s], use & 1);
+                        // descriptors differ only in the start-address field (16-byte units): one K step = 2 * LBO
+                        const uint64_t bd1 = bd0 + (uint64_t)((s * stage_bytes) >> 4);
+                        const int k0 = sl * SLAB;
 #pragma unroll
-                    for (int q = 0; q < NQ; ++q, ++n) {
-                        const uint32_t buf = n & 3;
-                        ptx::mbar_wait(&bars->acc_empty[buf], ((n >> 2) & 1) ^ 1);
-                        ptx::tc_fence_after();
-                        const uint32_t d_tmem = tmem_base + buf * TILE;
-                        const uint64_t ad1 = ad0 + (uint64_t)((q * a_tile_bytes) >> 4);
-                        if (ptx::elect_one()) {
-                            if (KSTEPS > 0) {
+                        for (int q = 0; q < NQ; ++q) {
+                            const uint32_t job = n + q, buf = job & 3;
+                            if (sl == 0) {
+                                ptx::mbar_wait(&bars->acc_empty[buf], ((job >> 2) & 1) ^ 1);
+                                ptx::tc_fence_after();
+                            }
+                            const uint32_t d_tmem = tmem_base + buf * TILE;
+                            const uint64_t ad1 = ad0 + (uint64_t)((q * a_tile_bytes + k0 * KSTEP_BYTES) >> 4);
+                            if (ptx::elect_one()) {
+                                if (SLAB > 0) {
 #pragma unroll
-                                for (int ks = 0; ks < KSTEPS; ++ks)
-                                    ptx::mma_f16_ss(d_tmem, ad1 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4), idesc,
-                                                    ks > 0 ? 1u : 0u);
-                            } else {
-                                for (int ks = 0; ks < ksteps; ++ks)
-                                    ptx::mma_f16_ss(d_tmem, ad1 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4), idesc,
-                                                    ks > 0 ? 1u : 0u);
+                                    for (int ks = 0; ks < SLAB; ++ks)
+                                        if (k0 + ks < ksteps)
+                                            ptx::mma_f16_ss(d_tmem, ad1 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4),
+                                                            idesc, k0 + ks > 0 ? 1u : 0u);
+                                } else if (KSTEPS > 0) {
+#pragma unroll
+                                    for (int ks = 0; ks < KSTEPS; ++ks)
+                                        ptx::mma_f16_ss(d_tmem, ad1 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4), idesc,
+                                                        ks > 0 ? 1u : 0u);
+                                } else {
+                                    for (int ks = 0; ks < ksteps; ++ks)
+                                        ptx::mma_f16_ss(d_tmem, ad1 + ks * ((2 * lbo) >> 4), bd1 + ks * ((2 * lbo) >> 4), idesc,
+                                                        ks > 0 ? 1u : 0u);
+                                }
+                                if (sl == nslab - 1) ptx::mma_commit(&bars->acc_full[buf]);
+                                if (q == NQ - 1) {
+                                    ptx::mma_commit(&bars->b_empty[s]);
+                                    if (j == j1 - 1 && sl == nslab - 1) ptx::mma_commit(&bars->a_empty);
+                                }
                             }
-                            ptx::mma_commit(&bars->acc_full[buf]);
-                            if (q == NQ - 1) {
-                                ptx::mma_commit(&bars->b_empty[s]);
-                                if (j == j1 - 1) ptx::mma_commit(&bars->a_empty);
-                            }
+                            __syncwarp();
                         }
-                        __syncwarp();
                     }
-                }
             }
         }
     } else if (warp < N_EPI_WARPS) {
@@ -516,6 +568,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
 
 // Final selection: one warp per (query, reference range).  Sorts the buffer the sweep left behind, emits the K'
 // best reference rows and the threshold every other reference of the range is at or above.
+template <int NQ>
 __global__ void __launch_bounds__(256)
 emit_kernel(const Params p) {
     const int lane = threadIdx.x & 31;
@@ -548,9 +601,8 @@ emit_kernel(const Params p) {
 
 // ------------------------------------------------------------------ host side
 bool nabo_tc_supported(int g, int k, int drop_first) {
-    if (g < 1) return false;
-    const int kp = tc::kp_for(g);
-    const tc::SmemPlan pl = tc::plan_smem(kp);
+    if (g < 1 || g > tc::MAX_G) return false;
+    const tc::SmemPlan pl = tc::plan_smem(g);
     const int ksel = k + (drop_first ? 1 : 0);
     return pl.stages >= 2 && ksel + 8 <= tc::MAX_KPRIME;
 }
@@ -576,8 +628,9 @@ static int tc_grid(int n_items) {
 // pieces, each a work item of its own with its own K' candidates and threshold: a 20 000-query call keeps
 // 106 SMs busy instead of 53.  The re-rank sees the union of the candidate lists and the smallest threshold
 // (everything a piece rejected scored >= that piece's threshold >= the minimum), so nothing else changes.
-int nabo_tc_split(int n_query, int n_ref) {
-    const int n_items = (n_query + tc::NQ * tc::TILE - 1) / (tc::NQ * tc::TILE);
+int nabo_tc_split(int n_query, int n_ref, int g) {
+    const int nq = tc::plan_smem(g).nq;
+    const int n_items = (n_query + nq * tc::TILE - 1) / (nq * tc::TILE);
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
     int s = n_items > 0 ? tc_grid(1 << 30) / n_items : 1;
     if (s > NABO_TC_MAX_SPLIT) s = NABO_TC_MAX_SPLIT;
@@ -602,15 +655,16 @@ int nabo_tau_min_launch(float* tau, int n_query, int n_split, cudaStream_t st) {
 size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first) {
     const int kp = tc::kp_for(g);
     const size_t tb = tc::tile_bytes(kp);
-    const int n_items = (n_query + tc::NQ * tc::TILE - 1) / (tc::NQ * tc::TILE);
+    const int nq = tc::plan_smem(g).nq;
+    const int n_items = (n_query + nq * tc::TILE - 1) / (nq * tc::TILE);
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
     const int kprime = nabo_tc_kprime(k, drop_first);
     size_t b = 0;
-    b += nabo_align_up((size_t)n_items * tc::NQ * tb, 256);          // packed queries
+    b += nabo_align_up((size_t)n_items * nq * tb, 256);          // packed queries
     b += nabo_align_up((size_t)n_rtiles * tb, 256);                   // packed references
     b += nabo_align_up((size_t)n_query * 8, 256) * 2;                 // q norms, qn2
     b += nabo_align_up((size_t)n_ref * 8, 256);                       // r norms
-    b += nabo_align_up((size_t)n_items * NABO_TC_MAX_SPLIT * tc::NQ * tc::TILE * (tc::CAP * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
+    b += nabo_align_up((size_t)n_items * NABO_TC_MAX_SPLIT * nq * tc::TILE * (tc::CAP * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
     b += nabo_align_up((size_t)n_query * kprime * 4 * NABO_TC_MAX_SPLIT, 256);   // candidate indices (per reference range)
     b += nabo_align_up((size_t)n_query * 4 * NABO_TC_MAX_SPLIT, 256) + nabo_align_up((size_t)n_query * 4, 256);   // cert tau, fail rows
     b += 4096;
@@ -629,10 +683,10 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     // public candidate entry point: one K' list per query); out: K' lists per query
     int n_split = *n_split_io;
     const int kp = tc::kp_for(g);
-    const tc::SmemPlan pl = tc::plan_smem(kp);
+    const tc::SmemPlan pl = tc::plan_smem(g);
     const size_t tb = tc::tile_bytes(kp);
-    const int n_items = (n_query + tc::NQ * tc::TILE - 1) / (tc::NQ * tc::TILE);
-    const int n_qtiles = n_items * tc::NQ;
+    const int n_items = (n_query + pl.nq * tc::TILE - 1) / (pl.nq * tc::TILE);
+    const int n_qtiles = n_items * pl.nq;
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
     const int kprime = nabo_tc_kprime(k, drop_first);
     if (n_split < 1 || n_split > NABO_TC_MAX_SPLIT) n_split = 1;
@@ -643,7 +697,7 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     double* qnorm = ar.take<double>(n_query);
     double* qn2 = ar.take<double>(n_query);
     double* rnorm = ar.take<double>(n_ref);
-    const size_t n_slots = (size_t)n_items * n_split * tc::NQ * tc::TILE;
+    const size_t n_slots = (size_t)n_items * n_split * pl.nq * tc::TILE;
     unsigned long long* cbuf = ar.take<unsigned long long>(n_slots * tc::CAP);
     int* ccnt = ar.take<int>(n_slots);
     float* ctau = ar.take<float>(n_slots);
@@ -678,22 +732,26 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     p.signal_round = overlap ? n_items / grid : 0;
     if (tail) {
         tail->applies = tail_applies ? 1 : 0;
-        tail->rows_full = overlap ? (n_items - rem_items) * tc::NQ * tc::TILE : 0;
+        tail->rows_full = overlap ? (n_items - rem_items) * pl.nq * tc::TILE : 0;
     }
-#define NABO_TC_LAUNCH1(KS, SPLIT)                                                                                 \
+#define NABO_TC_LAUNCH1(KS, SPLIT, NQ, SLAB)                                                                       \
     do {                                                                                                           \
-        NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, SPLIT>,                                           \
+        NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, SPLIT, NQ, SLAB>,                                 \
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.total));               \
-        tc::candidates_kernel<KS, SPLIT><<<grid, tc::NTHREADS, pl.total, st>>>(p);                                 \
+        tc::candidates_kernel<KS, SPLIT, NQ, SLAB><<<grid, tc::NTHREADS, pl.total, st>>>(p);                       \
     } while (0)
-#define NABO_TC_LAUNCH(KS)                                                                                         \
+#define NABO_TC_LAUNCH(KS, NQ, SLAB)                                                                               \
     do {                                                                                                           \
-        if (n_split > 1) NABO_TC_LAUNCH1(KS, true);                                                                \
-        else NABO_TC_LAUNCH1(KS, false);                                                                           \
+        if (n_split > 1) NABO_TC_LAUNCH1(KS, true, NQ, SLAB);                                                      \
+        else NABO_TC_LAUNCH1(KS, false, NQ, SLAB);                                                                 \
     } while (0)
-    if (kp == 160) NABO_TC_LAUNCH(10);        // g = 50 (BASELINE configs 2-5)
-    else if (kp == 80) NABO_TC_LAUNCH(5);     // g = 25 (config 1)
-    else NABO_TC_LAUNCH(0);
+    if (pl.stages < 2) return nabo_set_error(NABO_EUNSUPPORTED, "knn: g=%d outside the tensor-core tile plans", g);
+    if (pl.nq == 2) {                             // 53 <= g <= 128 (wide plan): slabs of 4 or 2 K steps
+        if (pl.slab == 4) NABO_TC_LAUNCH(0, 2, 4);
+        else NABO_TC_LAUNCH(0, 2, 2);
+    } else if (kp == 160) NABO_TC_LAUNCH(10, 3, 0);    // g = 50 (BASELINE configs 2-5)
+    else if (kp == 80) NABO_TC_LAUNCH(5, 3, 0);        // g = 25 (config 1)
+    else NABO_TC_LAUNCH(0, 3, 0);
 #undef NABO_TC_LAUNCH1
 #undef NABO_TC_LAUNCH
     NABO_LAUNCH_CHECK("candidates_kernel");
@@ -707,7 +765,8 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
         return 0;
     }
     if (raw_out) raw_out->buf = nullptr;
-    tc::emit_kernel<<<(unsigned)((n_slots + 7) / 8), 256, 0, st>>>(p);
+    if (pl.nq == 2) tc::emit_kernel<2><<<(unsigned)((n_slots + 7) / 8), 256, 0, st>>>(p);
+    else tc::emit_kernel<3><<<(unsigned)((n_slots + 7) / 8), 256, 0, st>>>(p);
     NABO_LAUNCH_CHECK("emit_kernel");
     *launches += 1;
     if (n_split > 1) {
