@@ -91,7 +91,8 @@ int nabo_rerank_launch(const double* q, int ldq, const double* r, int ldr, int n
                        int32_t* out_idx, double* out_dist, const NaboRoute& route, cudaStream_t st,
                        const NaboCandBuf* from_buf = nullptr, int row0 = 0, bool dependent = false);
 
-// Partly filled last wave of the persistent candidate kernel (tc_candidates.cu): every CTA executes
+// Partly filled last wave of the persistent candidate kernel (tc_candidates.cu; only where it does not cut items at
+// CTA boundaries, i.e. packed references larger than half of L2): every CTA executes
 // griddepcontrol.launch_dependents once its full-wave items are done, so a kernel launched right behind it on the same
 // stream with programmatic stream serialisation - the re-rank of the first rows_full queries - runs while the last wave is
 // still busy, on the SMs that wave leaves idle.  rows_full = 0: nothing to overlap.  When rows_full > 0 the candidate pass

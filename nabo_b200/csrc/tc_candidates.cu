@@ -11,7 +11,9 @@
 // so one tile is one contiguous span and a single cp.async.bulk brings it in.
 //
 // CTA = 512 threads, persistent over work items of NQ=3 query tiles (384 queries) x one range of
-// reference tiles (the whole reference, or a piece of it when there are fewer items than SMs):
+// reference tiles (the whole reference, or a piece of it when there are fewer items than SMs; with more items than SMs
+// the items are dealt out on a line of modelled cost, and an item cut at a CTA boundary is swept as a head on one CTA
+// and a tail that resumes the head's selection state on the next - see sched_bound):
 //   warps 0-11  epilogue: warpgroup w owns query tile w; thread = one query row (TMEM lane)
 //   warp 12  TMEM allocator, then TMA producer: A tiles once per item, B (reference) tiles through a ring
 //   warp 13  MMA issuer: the three query tiles rotate over FOUR accumulators, so the MMAs of a warpgroup's
@@ -59,6 +61,47 @@ constexpr uint32_t KSTEP_BYTES = TILE * 16 * 2;   // one K step (16 columns) of 
 
 __host__ __device__ inline int kp_for(int g) { return (3 * g + 3 + 15) / 16 * 16; }
 __host__ __device__ inline size_t tile_bytes(int kp) { return (size_t)TILE * kp * 2; }
+
+// ------------------------------------------------------------------ schedule of the unsplit sweep
+// Modelled cost of the first x reference tiles of a work item, in tiles of the warm sweep:
+//   F(x) = x + COST_BETA * j0 * ln(1 + x / j0),   j0 = COST_J0 * K' tiles.
+// The log term is the cold start of the running selection: a query appends about K' / i of its i-th reference, so the
+// appends - and the compactions they trigger - of the first x tiles grow as K' ln(x / K').
+// COST_BETA and COST_J0 are fitted to the epilogue cycles per warp-tile by sweep position (-DNABO_TC_STATS,
+// tools/probe_tc_stats.py) at 100 k x 100 k, g = 50, k = 30 (K' = 39) on a B200: see DESIGN 4.1.
+constexpr double COST_BETA = 16.2, COST_J0 = 1.0 / 20;
+__host__ __device__ inline double sweep_cost(int x, int kprime) {
+    const double j0 = COST_J0 * kprime;
+    return x + COST_BETA * j0 * log1p(x / j0);
+}
+
+// McNaughton's wrap-around rule on the cost line: the n_items items lie end to end, CTA ticket c owns [c T, (c + 1) T)
+// with T = n_items F(n_rtiles) / grid.  sched_bound(c) is where that segment starts: items < item and reference tiles
+// [0, tile) of `item` belong to lower tickets (0 <= tile < n_rtiles; the cut is the first whole tile at or past the
+// boundary's cost).  Ticket c therefore runs, in this order,
+//   the HEAD of item i1 = tiles [0, x1)         (x1 > 0; (i1, x1) = sched_bound(c + 1))
+//   the whole items [i0 or i0 + 1, i1)
+//   the TAIL of item i0 = tiles [x0, n_rtiles)  (x0 > 0; (i0, x0) = sched_bound(c)), resuming the head ticket c - 1 left.
+// A head is the first piece of its CTA and waits on nothing; a tail waits only on the next lower ticket.  In model cost
+// a head ends no later than its tail starts: head + tail = one item < T, and a CTA without whole items runs the head of
+// item i0 + 1 first, cut at a larger cost offset than its tail's (T > F(n_rtiles) when grid < n_items).  With
+// grid = n_items every boundary falls on an item: one whole item per CTA.
+__host__ __device__ inline void sched_bound(int b, int n_items, int n_rtiles, int grid, int kprime, int& item, int& tile) {
+    const long long pos = (long long)b * n_items;           // boundary in units of items: pos / grid
+    item = (int)(pos / grid);
+    const int rem = (int)(pos - (long long)item * grid);
+    tile = 0;
+    if (rem == 0) return;
+    const double o = sweep_cost(n_rtiles, kprime) * rem / grid;      // cost into `item`, 0 < o < F(n_rtiles)
+    // smallest x with F(x) >= o: F(lo) < o <= F(hi)
+    int lo = 0, hi = n_rtiles;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (sweep_cost(mid, kprime) >= o) hi = mid; else lo = mid;
+    }
+    tile = hi;
+    if (tile == n_rtiles) { ++item; tile = 0; }
+}
 
 // The tile plan of a PCA width g - the one place that decides it:
 //   g <= 52       NQ = 3 query tiles, whole reference tiles per ring stage (2 - 4 stages)
@@ -256,9 +299,12 @@ struct Params {
     const __half* qa;       // packed queries  [n_qtiles_padded][TILE*kp]
     const __half* rb;       // packed references [n_rtiles][TILE*kp]
     int n_query, n_ref, kp, n_items, n_rtiles, stages, kprime, kc_out, soft;
-    int signal_round;       // > 0 = every CTA signals the dependent launch after its signal_round-th item (0 = never;
-                            // always 0 when n_split > 1)
     int n_split;            // reference ranges per query item (work item = n_items x n_split, see nabo_tc_split)
+    int cut;                // n_split = 1: 1 = the cost-line schedule of sched_bound, 0 = items c, c + grid, ... per CTA c
+    int signal_round;       // > 0 = every CTA signals the dependent launch after its signal_round-th item (0 = never;
+                            // only without cuts and with n_split = 1)
+    unsigned int* ticket;   // n_split = 1: CTA ticket counter, then one flag per item: its head is in global memory
+                            // (zeroed before every launch)
     unsigned long long* cand_buf;   // [work item][NQ*TILE][CAP]: every (query, reference range) owns CAP keys
     int* cand_cnt;          // [work item][NQ*TILE] live keys of each buffer when its sweep ended
     float* cand_tau;        // [work item][NQ*TILE] running threshold when its sweep ended
@@ -272,14 +318,25 @@ struct Barriers {
     uint64_t b_full[MAX_STAGES], b_empty[MAX_STAGES];
     uint64_t acc_full[NACC], acc_empty[NACC];
     uint32_t tmem_base;
+    int ticket;             // n_split = 1: this CTA's ticket c
+    int sched[4];           // n_split = 1: sched_bound of c and of c + 1 (i0, x0, i1, x1)
 };
 
 using namespace sel;   // make_key, compact_sort_inline, compact_select (select.cuh)
 
 #ifdef NABO_TC_STATS       // development counters (tools/probe_tc_stats.py): [0] warp chunks, [1] warp chunks with a hit,
-__device__ unsigned long long g_tc_stats[12];  // [2] lanes with a hit, [3] keys appended, [4] running compactions,
-                                               // cycles per warp: [5] compaction, [6] filter_chunk, [7] wait for the
-                                               // accumulator, [8] tcgen05.ld + wait, [9] final emit, [10] whole item loop
+                           // [2] lanes with a hit, [3] keys appended, [4] running compactions, cycles per warp:
+                           // [5] compaction, [6] filter_chunk, [7] wait for the accumulator, [8] tcgen05.ld + wait,
+                           // [9] final emit, [10] whole item loop; [TC_HIST + b] epilogue cycles of the warp-tiles at
+                           // sweep position 2^b - 1 <= j < 2^(b+1) - 1 of an item, [TC_HIST + 32 + b] their count;
+                           // [TC_TIME + 2 c], [TC_TIME + 2 c + 1] %globaltimer at the start and end of CTA (ticket) c
+constexpr int TC_HIST = 12, TC_TIME = TC_HIST + 64, TC_NSTATS = TC_TIME + 2 * 1024;
+__device__ unsigned long long g_tc_stats[TC_NSTATS];
+__device__ __forceinline__ unsigned long long globaltimer() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
+    return t;
+}
 // accumulated in per-thread registers (tc_loc), flushed with one atomic per counter at the end of an item
 #define TC_STAT(i, v) (tc_loc[i] += (unsigned long long)(v))
 #define TC_CLK(var) const long long var = clock64()
@@ -339,19 +396,40 @@ __device__ __forceinline__ void filter_chunk(const uint32_t (&vr)[32], uint32_t 
     }
 }
 
-// Work enumeration: the reference range of every query item is cut into n_split equal pieces, each a work item with
-// its own buffer `slot`, K' list and threshold; the re-rank takes the union of the lists and the smallest threshold.
-// CTA c takes the slots c, c + grid, c + 2 grid, ...  Returns false when CTA `c` has no r-th work item.
-// SPLIT = false is the n_split = 1 case (the whole reference), compiled on its own: the general form in the unsplit
-// kernel measured 3.59 -> 3.72 ms at 100 k x 100 k, k = 30 (B200, 1 000 W power limit).
+// Work enumeration (the r-th piece of this CTA; false when there is none).  SPLIT: the reference range of every query
+// item is cut into n_split equal pieces, each a work item with its own buffer `slot`, K' list and threshold; the re-rank
+// takes the union of the lists and the smallest threshold; CTA c takes the slots c, c + grid, c + 2 grid, ...
+// SPLIT is a template parameter: one general form for both measured 3.59 -> 3.72 ms in the unsplit kernel at
+// 100 k x 100 k, k = 30 (B200, 1 000 W power limit).
+// SPLIT = false: CTA ticket c runs the pieces of sched_bound (head, whole items, tail; sched = {i0, x0, i1, x1}), or,
+// without cuts (sched[0] = -1 - c), the whole items c, c + grid, c + 2 grid, ...
 template <bool SPLIT>
-__device__ __forceinline__ bool work_piece(const Params& p, int c, int r, int& slot, int& qitem, int& j0, int& j1) {
-    slot = c + r * (int)gridDim.x;
+__device__ __forceinline__ bool work_piece(const Params& p, const int (&sched)[4], int r, int& slot, int& qitem, int& j0,
+                                           int& j1) {
     if (!SPLIT) {
-        if (slot >= p.n_items) return false;
-        qitem = slot; j0 = 0; j1 = p.n_rtiles;
-        return true;
+        const int i0 = sched[0], x0 = sched[1], i1 = sched[2], x1 = sched[3];
+        if (i0 < 0) {
+            slot = qitem = -1 - i0 + r * (int)gridDim.x;
+            j0 = 0; j1 = p.n_rtiles;
+            return slot < p.n_items;
+        }
+        if (x1 > 0 && r-- == 0) {                          // head
+            slot = qitem = i1; j0 = 0; j1 = x1;
+            return true;
+        }
+        const int first = x0 > 0 ? i0 + 1 : i0;
+        j1 = p.n_rtiles;
+        if (r < i1 - first) {                              // whole items
+            slot = qitem = first + r; j0 = 0;
+            return true;
+        }
+        if (x0 > 0 && r == i1 - first) {                   // tail
+            slot = qitem = i0; j0 = x0;
+            return true;
+        }
+        return false;
     }
+    slot = (int)blockIdx.x + r * (int)gridDim.x;
     if (slot >= p.n_items * p.n_split) return false;
     qitem = slot / p.n_split;
     const int seg = slot - qitem * p.n_split;
@@ -380,12 +458,29 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
         for (int s = 0; s < MAX_STAGES; ++s) { ptx::mbar_init(&bars->b_full[s], 1); ptx::mbar_init(&bars->b_empty[s], 1); }
         for (int q = 0; q < NACC; ++q) { ptx::mbar_init(&bars->acc_full[q], 1); ptx::mbar_init(&bars->acc_empty[q], 4); }
         ptx::fence_barrier_init();
+        if (!SPLIT) {
+            // the ticket, not blockIdx.x, orders the CTAs: a lower ticket belongs to a CTA that has already started, so
+            // a tail's wait for its head (ticket c - 1) ends even when only some CTAs of the grid are resident
+            const int c = (int)atomicAdd(p.ticket, 1u);
+            bars->ticket = c;
+            if (p.cut) {
+                sched_bound(c, p.n_items, p.n_rtiles, (int)gridDim.x, p.kprime, bars->sched[0], bars->sched[1]);
+                sched_bound(c + 1, p.n_items, p.n_rtiles, (int)gridDim.x, p.kprime, bars->sched[2], bars->sched[3]);
+            } else {
+                bars->sched[0] = -1 - c;             // items c, c + grid, c + 2 grid, ... (see work_piece)
+                bars->sched[1] = bars->sched[2] = bars->sched[3] = 0;
+            }
+#ifdef NABO_TC_STATS
+            if (c < 1024) g_tc_stats[TC_TIME + 2 * c] = globaltimer();
+#endif
+        }
     }
     if (warp == TMEM_WARP) ptx::tmem_alloc(&bars->tmem_base, 512);
     ptx::tc_fence_before();
     __syncthreads();
     ptx::tc_fence_after();
     const uint32_t tmem_base = bars->tmem_base;
+    const int sched[4] = {bars->sched[0], bars->sched[1], bars->sched[2], bars->sched[3]};
 
     if (warp == PRODUCER_WARP) {
         // ===================== TMA producer =====================
@@ -393,7 +488,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
             uint32_t t = 0, it = 0;
             for (int wr = 0;; ++wr, ++it) {
                 int w, item, j0, j1;
-                if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
+                if (!work_piece<SPLIT>(p, sched, wr, w, item, j0, j1)) break;
                 ptx::mbar_wait_hint(&bars->a_empty, (it & 1) ^ 1, SLEEP_NS);
                 ptx::mbar_arrive_expect_tx(&bars->a_full, NQ * a_tile_bytes);
                 for (int q = 0; q < NQ; ++q) {
@@ -433,7 +528,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
             uint32_t t = 0, it = 0, n = 0;
             for (int wr = 0;; ++wr, ++it) {
                 int w, item, j0, j1;
-                if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
+                if (!work_piece<SPLIT>(p, sched, wr, w, item, j0, j1)) break;
                 ptx::mbar_wait(&bars->a_full, it & 1);
                 for (int j = j0; j < j1; ++j, n += NQ, ++t)
                     for (int sl = 0; sl < nslab; ++sl) {
@@ -493,12 +588,45 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
         TC_DECL;
         for (int wr = 0;; ++wr) {
             int w, item, j0, j1;
-            if (!work_piece<SPLIT>(p, blockIdx.x, wr, w, item, j0, j1)) break;
+            if (!work_piece<SPLIT>(p, sched, wr, w, item, j0, j1)) break;
             unsigned long long* mybuf = p.cand_buf + ((size_t)w * NQ * TILE + slot) * CAP;
             float tau = CUDART_INF_F;
             int cnt = 0;
+            if (!SPLIT && j0 > 0) {
+                // tail: resume the selection state (buffer, count, tau) the head left in global memory.  One thread
+                // waits for the head's flag (acquire), the epilogue warps meet on the named barrier, then read.
+                if (threadIdx.x == 0) {
+                    unsigned int ns = 32, done;
+#ifdef NABO_CHECK
+                    unsigned int spins = 0;
+#endif
+                    while (true) {
+                        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(done) : "l"(p.ticket + 1 + item) : "memory");
+                        if (done) break;
+                        __nanosleep(ns);
+                        if (ns < 1024) ns *= 2;
+                        NABO_DEV_ASSERT(++spins < (1u << 24));      // ~17 s: a schedule bug, not a slow head
+                    }
+                }
+                asm volatile("bar.sync 1, %0;" ::"n"(N_EPI_WARPS * 32) : "memory");
+                cnt = __ldcg(p.cand_cnt + (size_t)w * NQ * TILE + slot);
+                tau = __ldcg(p.cand_tau + (size_t)w * NQ * TILE + slot);
+            }
             TC_CLK(t_item);
+#ifdef NABO_TC_STATS
+            int hb = -1;                       // log2 bucket of the sweep position, its cycles and warp-tiles so far
+            unsigned long long hcyc = 0, hcnt = 0;
+#endif
             for (int j = j0; j < j1; ++j, ++t) {
+#ifdef NABO_TC_STATS
+                const long long t_tile = clock64();
+                const int pos = SPLIT ? j - j0 : j;          // tiles since this selection state started cold
+                const int b = 31 - __clz(pos + 1);
+                if (b != hb) {
+                    if (lane == 0 && hcnt) { atomicAdd(&g_tc_stats[TC_HIST + hb], hcyc); atomicAdd(&g_tc_stats[TC_HIST + 32 + hb], hcnt); }
+                    hb = b; hcyc = 0; hcnt = 0;
+                }
+#endif
                 const uint32_t job = t * NQ + q, buf = job & 3, acc_par = (job >> 2) & 1;
                 const uint32_t taddr0 = tlane0 + buf * TILE;
                 TC_CLK(t_w);
@@ -542,7 +670,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                     TC_CLK_ADD(6, t_f);
                     compact_over(c == TILE / CHUNK - 1 ? p.soft : CAP - CHUNK);
                 }
+#ifdef NABO_TC_STATS
+                hcyc += (unsigned long long)(clock64() - t_tile);
+                ++hcnt;
+#endif
             }
+#ifdef NABO_TC_STATS
+            if (lane == 0 && hcnt) { atomicAdd(&g_tc_stats[TC_HIST + hb], hcyc); atomicAdd(&g_tc_stats[TC_HIST + 32 + hb], hcnt); }
+#endif
             // item done: leave the buffer as it is; emit_kernel makes the final selection of every (query, range)
             // at full occupancy instead of 32 serial sorts per warp here, with the tensor pipe idle meanwhile
             TC_CLK(t_e);
@@ -553,16 +688,27 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
             TC_FLUSH;
             if (!SPLIT && p.signal_round == wr + 1) {
                 // the full waves are done on this CTA: its buffers, counts and thresholds are in global memory
-                // (fence), the 12 epilogue warps meet on a named barrier, one thread lets the dependent grid - the
+                // (fence), the epilogue warps meet on a named barrier, one thread lets the dependent grid - the
                 // re-rank of those queries - start while the last, partly filled wave is still running
                 __threadfence();
                 asm volatile("bar.sync 1, %0;" ::"n"(N_EPI_WARPS * 32) : "memory");
                 if (threadIdx.x == 0) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
             }
+            if (!SPLIT && j1 < p.n_rtiles) {
+                // head: its buffers, counts and thresholds are in global memory (fence), the epilogue warps meet on
+                // the named barrier, one thread publishes the item's flag for the tail on the next ticket
+                __threadfence();
+                asm volatile("bar.sync 1, %0;" ::"n"(N_EPI_WARPS * 32) : "memory");
+                if (threadIdx.x == 0)
+                    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p.ticket + 1 + item), "r"(1u) : "memory");
+            }
         }
     }
     ptx::tc_fence_before();
     __syncthreads();
+#ifdef NABO_TC_STATS
+    if (!SPLIT && threadIdx.x == 0 && bars->ticket < 1024) g_tc_stats[TC_TIME + 2 * bars->ticket + 1] = globaltimer();
+#endif
     if (warp == TMEM_WARP) ptx::tmem_dealloc(tmem_base, 512);
 }
 
@@ -624,6 +770,13 @@ static int tc_grid(int n_items) {
     return n_items < sms ? n_items : sms;
 }
 
+static size_t l2_bytes() {
+    int dev = 0, l2 = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, dev);
+    return (size_t)l2;
+}
+
 // With fewer query items than SMs the reference range of every item is cut into up to NABO_TC_MAX_SPLIT
 // pieces, each a work item of its own with its own K' candidates and threshold: a 20 000-query call keeps
 // 106 SMs busy instead of 53.  The re-rank sees the union of the candidate lists and the smallest threshold
@@ -667,6 +820,7 @@ size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_fi
     b += nabo_align_up((size_t)n_items * NABO_TC_MAX_SPLIT * nq * tc::TILE * (tc::CAP * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
     b += nabo_align_up((size_t)n_query * kprime * 4 * NABO_TC_MAX_SPLIT, 256);   // candidate indices (per reference range)
     b += nabo_align_up((size_t)n_query * 4 * NABO_TC_MAX_SPLIT, 256) + nabo_align_up((size_t)n_query * 4, 256);   // cert tau, fail rows
+    b += nabo_align_up((size_t)(3 + n_items) * 4, 256);              // norm maxima, CTA ticket, head flags
     b += 4096;
     return b;
 }
@@ -704,10 +858,10 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_split);
     float* tau = ar.take<float>((size_t)n_query * n_split);
     double* scal = ar.take<double>(4);
-    unsigned int* maxbits = ar.take<unsigned int>(2);
+    unsigned int* maxbits = ar.take<unsigned int>(3 + (size_t)n_items);    // 2 norm maxima, CTA ticket, head flags
     if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the tensor-core pass");
 
-    NABO_CUDA(cudaMemsetAsync(maxbits, 0, 2 * sizeof(unsigned int), st));
+    NABO_CUDA(cudaMemsetAsync(maxbits, 0, (3 + (size_t)n_items) * sizeof(unsigned int), st));
     tc::norms_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(q, ldq, n_query, g, qnorm, maxbits);
     tc::norms_kernel<<<(n_ref + 255) / 256, 256, 0, st>>>(r, ldr, n_ref, g, rnorm, maxbits + 1);
     tc::scale_kernel<<<1, 1, 0, st>>>(maxbits, maxbits + 1, metric == NABO_COSINE ? 1 : 0, scal);
@@ -720,14 +874,24 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     p.qa = qa; p.rb = rb;
     p.n_query = n_query; p.n_ref = n_ref; p.kp = kp; p.n_items = n_items; p.n_rtiles = n_rtiles;
     p.stages = pl.stages; p.kprime = kprime; p.kc_out = kprime; p.n_split = n_split;
-    p.cand_buf = cbuf; p.cand_cnt = ccnt; p.cand_tau = ctau; p.cand_idx = cand; p.cert_tau = tau;
+    p.cand_buf = cbuf; p.cand_cnt = ccnt; p.cand_tau = ctau; p.cand_idx = cand; p.cert_tau = tau; p.ticket = maxbits + 2;
     p.a_off = pl.a_off; p.b_off = pl.b_off; p.sort_off = pl.sort_off; p.bar_off = pl.bar_off;
     p.soft = tc::CAP - tc::CHUNK - 16 > kprime ? tc::CAP - tc::CHUNK - 16 : kprime;
-    // Partly filled last wave (see NaboTailSplit): every CTA signals after its last full-wave item when the caller can
-    // use the gap - the fused re-rank path only, at least two waves, at least 16 SMs idle in the last one.
+    // Cut items at CTA boundaries only when the last wave would be partly filled and the packed reference fits in half of
+    // L2 (the other half holds the candidate buffers of the running items, 57 MB at g <= 52).  The cuts put the CTAs'
+    // sweeps out of step by up to an item.  Measured on a B200 (1 000 W power limit) at the two ends only: at 100 k x 100 k,
+    // g = 50 (31 MB packed) the cuts take the candidate kernel from 3.62 to 3.25 ms; at 500 k x 2 M cosine, g = 50 (625 MB
+    // packed) they took the kNN from 3.9e12 to 3.3e12 pairs/s (-18 %; the SM clock under the power cap fell from 1.52 to
+    // 1.30 GHz: the CTAs no longer share the reference tiles they read from HBM).  Between about 63 and 625 MB the half-L2
+    // line is a reasoned choice, not a measured one.  Without cuts every CTA c sweeps the items c, c + grid, ... (contiguous
+    // blocks of whole items measured 2 % slower at 500 k x 2 M), as it does for a whole number of waves.
+    p.cut = n_items % grid != 0 && (size_t)n_rtiles * tb <= l2_bytes() / 2 ? 1 : 0;
+    // Without cuts the last wave is partly filled (see NaboTailSplit): every CTA signals after its last full-wave item
+    // when the caller can use the gap - the fused re-rank path only, at least two waves, at least 16 SMs idle in the last
+    // one.  At 500 k x 2 M cosine (1 303 items) dropping this overlap cost 2.5 % of the kNN stage.
     const bool fused = raw_out && n_split == 1 && kprime <= 64;
     const int rem_items = n_items % grid;
-    const bool tail_applies = tail && fused && n_items > grid && rem_items > 0 && grid - rem_items >= 16;
+    const bool tail_applies = tail && fused && !p.cut && n_items > grid && rem_items > 0 && grid - rem_items >= 16;
     const bool overlap = tail_applies && !tail->dry;
     p.signal_round = overlap ? n_items / grid : 0;
     if (tail) {
@@ -783,11 +947,19 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
 #ifdef NABO_TC_STATS
 extern "C" int nabo_dbg_tc_stats(unsigned long long* out_host, int reset) {
     cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out_host, tc::g_tc_stats, sizeof(unsigned long long) * 12);
-    if (reset) { unsigned long long z[12] = {0}; cudaMemcpyToSymbol(tc::g_tc_stats, z, sizeof(z)); }
+    cudaMemcpyFromSymbol(out_host, tc::g_tc_stats, sizeof(unsigned long long) * tc::TC_NSTATS);
+    if (reset) { static unsigned long long z[tc::TC_NSTATS]; cudaMemcpyToSymbol(tc::g_tc_stats, z, sizeof(z)); }
     return 0;
 }
 #endif
+
+// The unsplit schedule as the kernel computes it (tests/test_tc_schedule_cpu.py): out[2 b], out[2 b + 1] =
+// sched_bound(b) for b = 0 .. grid; the modelled cost F(x) of the first x reference tiles of an item.
+extern "C" int nabo_dbg_tc_sched_bounds(int n_items, int n_rtiles, int grid, int kprime, int* out) {
+    for (int b = 0; b <= grid; ++b) tc::sched_bound(b, n_items, n_rtiles, grid, kprime, out[2 * b], out[2 * b + 1]);
+    return 0;
+}
+extern "C" double nabo_dbg_tc_sweep_cost(int x, int kprime) { return tc::sweep_cost(x, kprime); }
 
 // ------------------------------------------------------------------ public candidate-pass entry points
 extern "C" int nabo_knn_candidates_width(int k, int drop_first) { return nabo_tc_kprime(k, drop_first); }
