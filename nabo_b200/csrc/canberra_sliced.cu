@@ -11,7 +11,7 @@
 //     (outward rounded) end points, P[hi + 1] & ~P[lo] flags every reference whose bin meets the interval -
 //     a superset of the unsaturated ones, for 32 references with two shared-memory loads and one LOP3;
 //   * the g flag words are summed vertically with a carry-save adder tree (Harley-Seal, 2.25 LOP3 per
-//     dimension) into a 6-bit sliced counter and compared with need(tau) = min{c : g - c < tau};
+//     dimension) into a 6-bit sliced counter (8 bits for g > 56) and compared with need(tau) = min{c : g - c < tau};
 //   * the surviving pairs (about 2 % once tau is warm) go through the dense FP32 evaluation
 //     (same arithmetic and error bound nabo_cb_eps as canberra_candidates.cu) and the running top-K'
 //     selection of select.cuh.
@@ -52,32 +52,44 @@ __device__ unsigned long long g_cbs_prof[12];
 using namespace sel;   // make_key, compact_select, compact_sort_inline
 
 constexpr int NBINS = 32;                 // value bins per dimension
-constexpr int RT = 128;                   // references per tile
-constexpr int WPT = RT / 32;              // words per tile
-constexpr int T64 = RT / 64;              // 64-reference blocks of the FP32 copy per tile
 constexpr int NPL = NBINS + 1;            // cumulative planes per (dimension, word)
-static_assert((WPT * NPL) % 4 == 0, "plane rows must be multiples of 16 bytes (bulk copies)");
 constexpr int SLEEP_NS = 400;             // suspend-time hint of the tile waits
-constexpr int NW = 12;                    // warps per CTA
-constexpr int QB = NW * 32;               // queries a CTA handles per round (at most)
-constexpr int NTHREADS = NW * 32;
-constexpr int LC = 512;                   // work-list entries per warp
 constexpr int CAP = sel::CAP;
 constexpr int MAX_STAGES = 4;
 constexpr int EDGE_SAMPLE = 4096;
 constexpr int TRIG_EXTRA = 24;            // keys above kprime that trigger a compaction
 
+// Tile plan, a function of NB = ceil(g / 8) alone (one kernel instance per NB).
+//   narrow, g <= 56: 12 warps, 128-reference tiles, 6-bit sliced counters (count <= 63), and the FP32 reference
+//                    copy of canberra_candidates.cu ([tile64][k][64]);
+//   wide, 57 <= g <= 128: the query bin intervals (4 NB registers) no longer fit 12 warps' register budget (168
+//                    per thread), so 8 warps (up to 255); 8-bit counters (count <= 128); the per-warp FP32 query
+//                    tiles (1 024 g bytes with 8 warps) leave room for two stages of 64-reference tiles up to
+//                    g = 104 (with 448-entry work lists) and of 32-reference tiles up to g = 128.  64-reference tiles
+//                    are faster where they fit (g = 100: 44 vs 56 ms per 100 k x 100 k call; DESIGN 4.3).  The FP32
+//                    reference copy is this file's own [tile32][k][32] layout (pretile32_kernel), so any multiple of
+//                    32 references is one contiguous span.
+constexpr bool wide_of(int nb) { return nb >= 8; }
+constexpr int nw_of(int nb) { return wide_of(nb) ? 8 : 12; }                        // warps per CTA
+constexpr int rt_of(int nb) { return wide_of(nb) ? (nb <= 13 ? 64 : 32) : 128; }    // references per tile
+constexpr int lc_of(int nb) { return wide_of(nb) ? 448 : 512; }                     // work-list entries per warp
+constexpr int yw_of(int nb) { return wide_of(nb) ? 32 : 64; }                       // references per FP32 copy block
+constexpr int cbits_of(int nb) { return wide_of(nb) ? 8 : 6; }                      // bit planes of the sliced counter
+
 static inline int nblocks8(int g) { return (g + 7) / 8; }
-static inline size_t plane_tile_bytes(int g) { return (size_t)g * WPT * NPL * 4; }
-static inline size_t ys_tile_bytes(int g) { return (size_t)g * RT * 4; }
+// plane rows of one tile, padded to 16 bytes (bulk copies); the narrow tiles (4 x 33 words per dimension) need no pad
+static inline size_t plane_tile_bytes(int g, int rt) { return ((size_t)g * (rt / 32) * NPL * 4 + 15) & ~(size_t)15; }
+static inline size_t ys_tile_bytes(int g, int rt) { return (size_t)g * rt * 4; }
 
 struct SmemPlan {
-    int stages;
+    int stages, nw, rt, yw;
     size_t stage_bytes, stage_off, xs_off, hist_off, work_off, tau_off, cnt_off, bar_off, total;
 };
 static SmemPlan plan_smem(int g) {
     SmemPlan p;
-    p.stage_bytes = plane_tile_bytes(g) + ys_tile_bytes(g);
+    const int nb = nblocks8(g), NW = nw_of(nb), LC = lc_of(nb);
+    p.nw = NW; p.rt = rt_of(nb); p.yw = yw_of(nb);
+    p.stage_bytes = plane_tile_bytes(g, p.rt) + ys_tile_bytes(g, p.rt);
     const size_t fixed = (size_t)NW * g * 32 * 4 + (size_t)NW * 256 * 4 + (size_t)NW * LC * 2 + (size_t)NW * 32 * 8 + 128;
     const size_t cap = 227 * 1024;
     p.stages = 0;
@@ -137,22 +149,26 @@ __device__ __forceinline__ int bin_of(float y, const float* e) {
     return b;
 }
 
-// Cumulative planes of one (tile, dimension): planes[((tile * g + k) * WPT + w) * NPL + p], bit i of word w
-// = reference tile * RT + w * 32 + i is live (in range, not masked) and bin(y) < p.  rt is the FP32
-// pre-tiled reference of canberra_candidates.cu ([tile64][k][64]).
+// Cumulative planes of one (tile, dimension): word w of dimension k of a tile is at (k * WPT + w) * NPL words
+// from the (16-byte aligned) tile start, bit i of it = reference tile * RT + w * 32 + i is live (in range, not
+// masked) and bin(y) < p.  rt is the FP32 pre-tiled reference in YW-row blocks ([block][k][YW]).
+template <int RT, int YW>
 __global__ void __launch_bounds__(RT)
 planes_kernel(const float* __restrict__ rt, const float* __restrict__ edges, const uint8_t* __restrict__ mask,
               int n_ref, int g, uint32_t* __restrict__ planes) {
+    constexpr int WPT = RT / 32, YSH = YW == 64 ? 6 : 5;
+    static_assert(YW == (1 << YSH), "copy block");
     __shared__ float e[NBINS - 1];
     const int tile = blockIdx.x, k = blockIdx.y;
     if (threadIdx.x < NBINS - 1) e[threadIdx.x] = edges[k * (NBINS - 1) + threadIdx.x];
     __syncthreads();
     const int ref = tile * RT + threadIdx.x;
     const bool live = ref < n_ref && !(mask && mask[ref]);
-    const float y = live ? rt[((size_t)(ref >> 6) * g + k) * 64 + (ref & 63)] : 0.f;
+    const float y = live ? rt[((size_t)(ref >> YSH) * g + k) * YW + (ref & (YW - 1))] : 0.f;
     const int b = bin_of(y, e);
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    uint32_t* out = planes + (((size_t)tile * g + k) * WPT + w) * NPL;
+    const size_t tile_words = (WPT * NPL) % 4 == 0 ? (size_t)g * WPT * NPL : ((size_t)g * WPT * NPL + 3) & ~(size_t)3;
+    uint32_t* out = planes + (size_t)tile * tile_words + ((size_t)k * WPT + w) * NPL;
 #pragma unroll
     for (int p = 0; p < NPL; ++p) {
         const uint32_t bits = __ballot_sync(0xffffffffu, live && b < p && p <= NBINS);
@@ -200,7 +216,8 @@ ctrl_kernel(const double* __restrict__ q, int ld, int n_query, int g, int nj, do
     ctrl[e] = word;
 }
 
-// FP32 queries, 32 per group, dimension-major: qx[(group32 * g + k) * 32 + lane]
+// FP32 rows, 32 per group, dimension-major: qx[(group32 * g + k) * 32 + lane] (the queries; in the wide plan the
+// reference copy too)
 __global__ void __launch_bounds__(256)
 pretile32_kernel(const double* __restrict__ x, int ld, int n, int g, float* __restrict__ out, long long total) {
     const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -214,14 +231,14 @@ pretile32_kernel(const double* __restrict__ x, int ld, int n, int g, float* __re
 
 // ------------------------------------------------------------------ the sweep
 struct Params {
-    const uint32_t* planes;     // [n_tiles][g][WPT][NPL]
-    const float* rt;            // [n_tiles64][g][64]
+    const uint32_t* planes;     // [n_tiles][g][WPT][NPL], tiles padded to 16 bytes
+    const float* rt;            // [n_yblk][g][YW]
     const float* qx;            // [n_groups][g][32]
     const uint32_t* ctrl;       // [n_groups][nj][32]
-    int n_query, n_ref, g, n_tiles, n_tiles64, n_groups, kprime, stages, nj, n_split;
+    int n_query, n_ref, g, n_tiles, n_yblk, n_groups, kprime, stages, nj, n_split;
     float fm;
     int trig_extra;
-    unsigned long long* cand_buf;   // [gridDim][QB][CAP]
+    unsigned long long* cand_buf;   // [gridDim][NW * 32][CAP]
     int32_t* cand;              // [n_query][kprime]
     float* tau_out;             // [n_query]
     size_t stage_bytes, stage_off, xs_off, hist_off, work_off, tau_off, cnt_off, bar_off;
@@ -246,20 +263,28 @@ __device__ __forceinline__ float rcp_approx(float x) {       // MUFU.RCP, 1 ulp:
         l = u_ ^ c_;                                      \
     }
 
-// smallest count c with (float)g - c < tau, clamped to [0, 63]
+// smallest count c with (float)g - c < tau, clamped to [0, NEVER]; NEVER (all counter bits set) exceeds every
+// count the counter holds (g <= 63 in 6 bits, g <= 128 in 8), so it rejects everything (tau = -inf, padding queries)
+template <int NEVER>
 __device__ __forceinline__ int need_of(float tau, int g) {
-    if (!(tau > -CUDART_INF_F)) return 63;
+    if (!(tau > -CUDART_INF_F)) return NEVER;
     if (tau == CUDART_INF_F) return 0;
     int c = (int)floorf((float)g - tau) + 1;
     if (c < 0) c = 0;
     while (c > 0 && (float)(g - (c - 1)) < tau) --c;
-    while (c < 63 && !((float)(g - c) < tau)) ++c;
-    return c > 63 ? 63 : c;
+    while (c < NEVER && !((float)(g - c) < tau)) ++c;
+    return c > NEVER ? NEVER : c;
 }
 
 template <int NB, bool SPLIT>      // SPLIT: the CTAs of one query block share out the reference range (n_split > 1)
-__global__ void __launch_bounds__(NTHREADS, 1)
+__global__ void __launch_bounds__(nw_of(NB) * 32, 1)
 sliced_kernel(const Params p) {
+    constexpr int NW = nw_of(NB), QB = NW * 32;
+    constexpr int RT = rt_of(NB), WPT = RT / 32;
+    constexpr int YW = yw_of(NB), YSH = YW == 64 ? 6 : 5, TY = RT / YW;    // FP32 copy blocks per tile
+    constexpr int CB = cbits_of(NB), NEVER = (1 << CB) - 1;
+    constexpr int LC = lc_of(NB);
+    static_assert(YW == (1 << YSH) && RT <= 128 && NB * 8 <= NEVER && LC >= 256, "tile plan");
     extern __shared__ __align__(128) unsigned char smem[];
     Barriers* bars = reinterpret_cast<Barriers*>(smem + p.bar_off);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -286,18 +311,19 @@ sliced_kernel(const Params p) {
     // Reference tiles arrive by TMA bulk copies into a ring of p.stages buffers (full[] mbarriers).  There
     // is no producer warp: every warp counts itself out of a stage when it is done with the tile, and the
     // last one out re-arms the stage with the tile p.stages ahead - the earliest moment it can be issued.
-    const uint32_t plane_bytes = (uint32_t)((size_t)g * WPT * NPL * 4);
+    const uint32_t plane_bytes = (WPT * NPL) % 4 == 0 ? (uint32_t)((size_t)g * WPT * NPL * 4)
+                                                      : ((uint32_t)((size_t)g * WPT * NPL * 4) + 15u) & ~15u;
     auto issue_tile = [&](uint32_t tn, uint32_t s) {          // one thread
         const int j = tile0 + (int)(tn % (uint32_t)n_tiles);
-        const int n64 = min(T64, p.n_tiles64 - T64 * j);
-        const uint32_t ys_bytes = (uint32_t)n64 * g * 64 * 4;
+        const int ny = min(TY, p.n_yblk - TY * j);
+        const uint32_t ys_bytes = (uint32_t)ny * g * YW * 4;
         ptx::mbar_arrive_expect_tx(&bars->full[s], plane_bytes + ys_bytes);
         char* dst = reinterpret_cast<char*>(smem + p.stage_off + (size_t)s * p.stage_bytes);
         const char* src = reinterpret_cast<const char*>(p.planes) + (size_t)j * plane_bytes;
         for (uint32_t o = 0; o < plane_bytes; o += 16384)
             ptx::bulk_g2s(dst + o, src + o, min(16384u, plane_bytes - o), &bars->full[s]);
         dst += plane_bytes;
-        src = reinterpret_cast<const char*>(p.rt) + (size_t)j * T64 * g * 64 * 4;
+        src = reinterpret_cast<const char*>(p.rt) + (size_t)j * TY * g * YW * 4;
         for (uint32_t o = 0; o < ys_bytes; o += 16384)
             ptx::bulk_g2s(dst + o, src + o, min(16384u, ys_bytes - o), &bars->full[s]);
     };
@@ -366,14 +392,14 @@ sliced_kernel(const Params p) {
                 const int e0 = work[i0], e1 = act1 ? work[i1] : 0;
                 const int ql0 = e0 >> 8, rl0 = e0 & 127, ql1 = e1 >> 8, rl1 = e1 & 127;
                 const float* xb0 = xs + ql0;
-                const float* yb0 = ys + (rl0 >> 6) * (g * 64) + (rl0 & 63);
+                const float* yb0 = ys + (rl0 >> YSH) * (g * YW) + (rl0 & (YW - 1));
                 const float* xb1 = xs + ql1;
-                const float* yb1 = ys + (rl1 >> 6) * (g * 64) + (rl1 & 63);
+                const float* yb1 = ys + (rl1 >> YSH) * (g * YW) + (rl1 & (YW - 1));
                 float acc0 = 0.f, acc1 = 0.f;
 #pragma unroll 5
                 for (int k = 0; k < g; ++k) {
-                    const float x0 = xb0[k * 32], y0 = yb0[k * 64];
-                    const float x1 = xb1[k * 32], y1 = yb1[k * 64];
+                    const float x0 = xb0[k * 32], y0 = yb0[k * YW];
+                    const float x1 = xb1[k * 32], y1 = yb1[k * YW];
                     const float num0 = fabsf(x0 - y0), xa0 = fabsf(x0);
                     const float num1 = fabsf(x1 - y1), xa1 = fabsf(x1);
                     const float term0 = fmaf(num0, rcp_approx(xa0 + (fabsf(y0) + 0.01f)), -1.0f);
@@ -399,11 +425,11 @@ sliced_kernel(const Params p) {
                 const int e = active ? work[i] : 0;
                 const int ql = e >> 8, rl = e & 127;
                 const float* xb = xs + ql;
-                const float* yb = ys + (rl >> 6) * (g * 64) + (rl & 63);
+                const float* yb = ys + (rl >> YSH) * (g * YW) + (rl & (YW - 1));
                 float acc = 0.f;
 #pragma unroll 5
                 for (int k = 0; k < g; ++k) {
-                    const float x = xb[k * 32], y = yb[k * 64];
+                    const float x = xb[k * 32], y = yb[k * YW];
                     const float num = fabsf(x - y), xa = fabsf(x);
                     const float term = fmaf(num, rcp_approx(xa + (fabsf(y) + 0.01f)), -1.0f);
                     if (num < fm * xa) acc += term;
@@ -454,12 +480,18 @@ sliced_kernel(const Params p) {
             const char* pl = reinterpret_cast<const char*>(stage);
             const float* ys = reinterpret_cast<const float*>(stage + plane_bytes);
 
-            // ---- phase 0: sliced over-estimate of the unsaturated-dimension count, 4 x 32 references per lane
-            uint32_t c[WPT][6];
+            // ---- phase 0: sliced over-estimate of the unsaturated-dimension count, WPT x 32 references per lane
+            if constexpr (wide_of(NB)) {
+                // the plane offsets derived from ctrl are loop-invariant; hoisted out of the tile loop they would
+                // take 2 g registers instead of g / 2 and spill
+#pragma unroll
+                for (int jj = 0; jj < NB * 4; ++jj) asm volatile("" : "+r"(ctrl[jj]));
+            }
+            uint32_t c[WPT][CB];
 #pragma unroll
             for (int w = 0; w < WPT; ++w)
 #pragma unroll
-                for (int b = 0; b < 6; ++b) c[w][b] = 0u;
+                for (int b = 0; b < CB; ++b) c[w][b] = 0u;
 #pragma unroll
             for (int blk = 0; blk < NB; ++blk) {
                 uint32_t v[8][WPT];
@@ -493,19 +525,26 @@ sliced_kernel(const Params p) {
                     NABO_CSA(f4b, c[w][1], c[w][1], t2a, t2b);
                     NABO_CSA(e8, c[w][2], c[w][2], f4a, f4b);
                     const uint32_t k1 = c[w][3] & e8;
-                    c[w][5] ^= c[w][4] & k1;
+                    if constexpr (CB == 8) {      // ripple the carry of weight 16 up to weight 128
+                        const uint32_t k2 = c[w][4] & k1, k3 = c[w][5] & k2;
+                        c[w][7] ^= c[w][6] & k3;
+                        c[w][6] ^= k3;
+                        c[w][5] ^= k2;
+                    } else {
+                        c[w][5] ^= c[w][4] & k1;
+                    }
                     c[w][4] ^= k1;
                     c[w][3] ^= e8;
                 }
             }
             // count >= need(tau), per lane
-            const int need_c = need_of(s_tau[lane], g);
+            const int need_c = need_of<NEVER>(s_tau[lane], g);
             uint32_t m[WPT];
 #pragma unroll
             for (int w = 0; w < WPT; ++w) {
                 uint32_t gt = 0u, eq = 0xffffffffu;
 #pragma unroll
-                for (int b = 5; b >= 0; --b) {
+                for (int b = CB - 1; b >= 0; --b) {
                     const uint32_t nb = 0u - (uint32_t)((need_c >> b) & 1);
                     gt |= eq & c[w][b] & ~nb;
                     eq &= ~(c[w][b] ^ nb);
@@ -616,7 +655,7 @@ extern "C" int nabo_dbg_cbs_prof(unsigned long long* out_host, int reset) {
 
 // ------------------------------------------------------------------ host side
 bool nabo_cbs_supported(int g, int k, int drop_first) {
-    if (g < 1 || g > 64) return false;
+    if (g < 1 || g > 128) return false;
     const int ksel = k + (drop_first ? 1 : 0);
     return cbs::plan_smem(g).stages >= 2 && ksel + 8 <= cbs::CAP - 64;
 }
@@ -629,28 +668,31 @@ static int cbs_grid(int n_groups) {
 }
 
 size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g) {
-    const size_t n_tiles = (n_ref + cbs::RT - 1) / cbs::RT;
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
+    const size_t n_tiles = (n_ref + pl.rt - 1) / pl.rt;
     const size_t n_groups = (size_t)(n_query + 31) / 32;
     const int nj = cbs::nblocks8(g) * 4;
     size_t b = 0;
-    b += nabo_align_up(n_tiles * cbs::plane_tile_bytes(g), 256);
+    b += nabo_align_up(n_tiles * cbs::plane_tile_bytes(g, pl.rt), 256);
     b += nabo_align_up((size_t)g * (cbs::NBINS - 1) * 4, 256);
     b += nabo_align_up(n_groups * nj * 32 * 4, 256);
     b += nabo_align_up(n_groups * g * 32 * 4, 256);
-    b += nabo_align_up((size_t)148 * cbs::QB * cbs::CAP * 8, 256);
+    b += nabo_align_up((size_t)148 * pl.nw * 32 * cbs::CAP * 8, 256);
     return b + 1024;
 }
 
-// rt: FP32 pre-tiled reference ([tile64][k][64], nabo_cb_pretile_floats(n_ref, g) floats), filled here.
-// Pieces the reference range is cut into (see the kernel): only when a CTA would have at most four busy warps,
-// never below 64 tiles (8 192 references) per piece, and the union of the K' lists must fit the re-rank (128).
-int nabo_cbs_split(int n_query, int n_ref, int k, int drop_first) {
+// rt: FP32 copy of the reference (nabo_cb_pretile_floats(n_ref, g) floats: [tile64][k][64], or [tile32][k][32] in
+// the wide plan), filled here.
+// Pieces the reference range is cut into (see the kernel): only when a CTA would have at most half of its warps
+// busy, never below 8 192 references per piece, and the union of the K' lists must fit the re-rank (128).
+int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first) {
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
     const int n_groups = (n_query + 31) / 32;
-    const int n_tiles = (n_ref + cbs::RT - 1) / cbs::RT;
+    const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
     const int per_cta = (n_groups + cbs_grid(1 << 30) - 1) / cbs_grid(1 << 30);
-    int s = per_cta > 0 ? cbs::NW / per_cta : 1;
+    int s = per_cta > 0 ? pl.nw / per_cta : 1;
     if (s > NABO_CBS_MAX_SPLIT) s = NABO_CBS_MAX_SPLIT;
-    while (s > 1 && (n_tiles / s < 8192 / cbs::RT || s * nabo_cb_kprime(k, drop_first) > 128)) --s;
+    while (s > 1 && (n_tiles / s < 8192 / pl.rt || s * nabo_cb_kprime(k, drop_first) > 128)) --s;
     return s < 1 ? 1 : s;
 }
 
@@ -661,8 +703,8 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     const int kprime = nabo_cb_kprime(k, drop_first);
     if (n_split < 1 || n_split > NABO_CBS_MAX_SPLIT) n_split = 1;
     const cbs::SmemPlan pl = cbs::plan_smem(g);
-    const int n_tiles = (n_ref + cbs::RT - 1) / cbs::RT;
-    const int n_tiles64 = (n_ref + 63) / 64;
+    const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
+    const int n_yblk = (n_ref + pl.yw - 1) / pl.yw;
     const size_t n_groups = (size_t)(n_query + 31) / 32;
     const int nb = cbs::nblocks8(g), nj = nb * 4;
     int grid = cbs_grid((int)n_groups * n_split);
@@ -670,18 +712,27 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     if (grid < n_split) n_split = 1, grid = cbs_grid((int)n_groups);
 
     NaboArena ar(extra, extra_bytes);
-    uint32_t* planes = (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g));
+    uint32_t* planes = (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g, pl.rt));
     float* edges = ar.take<float>((size_t)g * (cbs::NBINS - 1));
     uint32_t* ctrl = ar.take<uint32_t>(n_groups * nj * 32);
     float* qx = ar.take<float>(n_groups * g * 32);
-    unsigned long long* cbuf = ar.take<unsigned long long>((size_t)grid * cbs::QB * cbs::CAP);
+    unsigned long long* cbuf = ar.take<unsigned long long>((size_t)grid * pl.nw * 32 * cbs::CAP);
     if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the sliced Canberra pass");
 
     {
-        int rc = nabo_cb_pretile_launch(r, ldr, n_ref, g, rt, st);
-        if (rc) return rc;
+        if (pl.yw == 64) {
+            int rc = nabo_cb_pretile_launch(r, ldr, n_ref, g, rt, st);
+            if (rc) return rc;
+        } else {
+            const long long tr = (long long)n_yblk * g * 32;
+            cbs::pretile32_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, rt, tr);
+        }
         cbs::edges_kernel<<<g, 1024, 0, st>>>(r, ldr, n_ref, edges);
-        cbs::planes_kernel<<<dim3(n_tiles, g), cbs::RT, 0, st>>>(rt, edges, mask, n_ref, g, planes);
+        switch (pl.rt) {
+            case 128: cbs::planes_kernel<128, 64><<<dim3(n_tiles, g), 128, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
+            case 64: cbs::planes_kernel<64, 32><<<dim3(n_tiles, g), 64, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
+            default: cbs::planes_kernel<32, 32><<<dim3(n_tiles, g), 32, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
+        }
         const long long tc = (long long)n_groups * nj * 32;
         cbs::ctrl_kernel<<<(unsigned)((tc + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, nj, f, edges, ctrl, tc);
         const long long tq = (long long)n_groups * g * 32;
@@ -691,7 +742,7 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
 
     cbs::Params p;
     p.planes = planes; p.rt = rt; p.qx = qx; p.ctrl = ctrl;
-    p.n_query = n_query; p.n_ref = n_ref; p.g = g; p.n_tiles = n_tiles; p.n_tiles64 = n_tiles64;
+    p.n_query = n_query; p.n_ref = n_ref; p.g = g; p.n_tiles = n_tiles; p.n_yblk = n_yblk;
     p.n_groups = (int)n_groups; p.kprime = kprime; p.stages = pl.stages; p.nj = nj; p.n_split = n_split;
     const double delta = fmax(1e-5, 4e-7 * (2.0 + f) / f);      // same optimistic margin as canberra_candidates.cu
     p.fm = (float)(f * (1.0 + delta));
@@ -699,22 +750,25 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     p.trig_extra = cbs::TRIG_EXTRA;
     p.stage_bytes = pl.stage_bytes; p.stage_off = pl.stage_off; p.xs_off = pl.xs_off; p.hist_off = pl.hist_off;
     p.work_off = pl.work_off; p.tau_off = pl.tau_off; p.cnt_off = pl.cnt_off; p.bar_off = pl.bar_off;
+    const int threads = pl.nw * 32;
 #define NABO_CBS_LAUNCH(NBV)                                                                                       \
     case NBV:                                                                                                      \
         if (n_split > 1) {                                                                                         \
             NABO_CUDA(cudaFuncSetAttribute(cbs::sliced_kernel<NBV, true>,                                          \
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.total));           \
-            cbs::sliced_kernel<NBV, true><<<grid, cbs::NTHREADS, pl.total, st>>>(p);                               \
+            cbs::sliced_kernel<NBV, true><<<grid, threads, pl.total, st>>>(p);                                     \
         } else {                                                                                                   \
             NABO_CUDA(cudaFuncSetAttribute(cbs::sliced_kernel<NBV, false>,                                         \
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.total));           \
-            cbs::sliced_kernel<NBV, false><<<grid, cbs::NTHREADS, pl.total, st>>>(p);                              \
+            cbs::sliced_kernel<NBV, false><<<grid, threads, pl.total, st>>>(p);                                    \
         }                                                                                                          \
         break;
     switch (nb) {
         NABO_CBS_LAUNCH(1) NABO_CBS_LAUNCH(2) NABO_CBS_LAUNCH(3) NABO_CBS_LAUNCH(4)
         NABO_CBS_LAUNCH(5) NABO_CBS_LAUNCH(6) NABO_CBS_LAUNCH(7) NABO_CBS_LAUNCH(8)
-        default: return nabo_set_error(NABO_EINVAL, "knn: sliced Canberra pass supports at most 64 dimensions");
+        NABO_CBS_LAUNCH(9) NABO_CBS_LAUNCH(10) NABO_CBS_LAUNCH(11) NABO_CBS_LAUNCH(12)
+        NABO_CBS_LAUNCH(13) NABO_CBS_LAUNCH(14) NABO_CBS_LAUNCH(15) NABO_CBS_LAUNCH(16)
+        default: return nabo_set_error(NABO_EINVAL, "knn: sliced Canberra pass supports at most 128 dimensions");
     }
 #undef NABO_CBS_LAUNCH
     NABO_LAUNCH_CHECK("cbs::sliced_kernel");

@@ -2,7 +2,8 @@
 // for the rows the certificate could not clear.  Results are identical to the exact engine
 // (and hence to the reference) by construction; only the amount of FP64 work changes.
 //   Euclidean / cosine : tensor-core candidate pass (tc_candidates.cu)
-//   modified Canberra  : two-phase FP32 CUDA-core candidate pass (canberra_candidates.cu)
+//   modified Canberra  : bit-sliced count bound + FP32 evaluation (canberra_sliced.cu, g <= 128), or the two-phase
+//                        FP16 / FP32 CUDA-core pass (canberra_candidates.cu, g <= 77) for a vanishing dist_factor
 #include "knn_internal.cuh"
 
 // Accumulation-error constant of the tensor-core score relative to (4|q||r| + |r|^2 + |q|^2);
@@ -32,15 +33,17 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
     tm.begin();
     const bool use_tc = (metric == NABO_EUCLIDEAN || metric == NABO_COSINE) && nabo_tc_supported(g, k, drop_first) &&
                         n_ref > nabo_tc_kprime(k, drop_first);
-    const bool use_cb = metric == NABO_MOD_CANBERRA && nabo_cb_supported(g, k, drop_first) &&
+    // the interval ends of the sliced pass carry a 1e-6 relative margin over f|x|; it must dominate the FP64
+    // rounding of x -+ f|x| (~1e-16 |x|), so a vanishing dist_factor goes to the FP16 two-phase pass instead
+    const bool sliced_ok = metric == NABO_MOD_CANBERRA && nabo_cbs_supported(g, k, drop_first) && f >= 1e-6;
+    const bool use_cb = metric == NABO_MOD_CANBERRA && (sliced_ok || nabo_cb_supported(g, k, drop_first)) &&
                         n_ref > nabo_cb_kprime(k, drop_first);
     if (use_cb) {
         if (workspace_bytes < nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric))
             return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small");
         NaboArena ar(workspace, workspace_bytes);
         const int kprime = nabo_cb_kprime(k, drop_first);
-        const bool sliced_ok = nabo_cbs_supported(g, k, drop_first) && f >= 1e-6;
-        const int n_split = sliced_ok ? nabo_cbs_split(n_query, n_ref, k, drop_first) : 1;
+        const int n_split = sliced_ok ? nabo_cbs_split(n_query, n_ref, g, k, drop_first) : 1;
         int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_split);
         float* tau = ar.take<float>((size_t)n_query * n_split);
         int* fail_rows = ar.take<int>(n_query);
@@ -51,10 +54,7 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
         char* extra = ar.take<char>(cb_extra_bytes(n_query, n_ref, g));
         if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small");
         NABO_CUDA(cudaMemsetAsync(fail_count, 0, sizeof(int), st));
-        // the interval ends of the sliced pass carry a 1e-6 relative margin over f|x|; it must dominate the FP64
-        // rounding of x -+ f|x| (~1e-16 |x|), so a vanishing dist_factor goes to the FP16 two-phase pass instead
-        const bool sliced = sliced_ok;
-        int rc = sliced
+        int rc = sliced_ok
                      ? nabo_cbs_candidates(q, ldq, r, ldr, n_query, n_ref, g, k, f, mask, drop_first, n_split, rt, extra,
                                            cb_extra_bytes(n_query, n_ref, g), cand, tau, st)
                      : nabo_cb_candidates(q, ldq, r, ldr, n_query, n_ref, g, k, f, mask, drop_first, qt, rt, extra, cand,
@@ -80,7 +80,7 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
             NABO_CUDA(cudaMemcpyAsync(&nfail, fail_count, sizeof(int), cudaMemcpyDeviceToHost, st));
             NABO_CUDA(cudaStreamSynchronize(st));
             stats_host[0] = n_query; stats_host[1] = nfail; stats_host[2] = kprime;
-            stats_host[3] = sliced ? 10 : 11;      // preparation + candidate pass + re-rank + 3 fallback kernels
+            stats_host[3] = sliced_ok ? 10 : 11;      // preparation + candidate pass + re-rank + 3 fallback kernels
             stats_host[4] = tm.ns(0); stats_host[5] = tm.ns(1); stats_host[6] = tm.ns(2);
         }
         return 0;

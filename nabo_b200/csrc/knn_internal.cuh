@@ -128,7 +128,7 @@ int nabo_cb_pretile_launch(const double* x, int ld, int n, int g, float* out, cu
 bool nabo_cbs_supported(int g, int k, int drop_first);
 size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g);
 #define NABO_CBS_MAX_SPLIT 3
-int nabo_cbs_split(int n_query, int n_ref, int k, int drop_first);
+int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first);
 int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                         double f, const uint8_t* mask, int drop_first, int n_split, float* rt, void* extra,
                         size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st);
