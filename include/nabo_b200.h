@@ -133,6 +133,56 @@ int nabo_knn_routed(const double* q, int ldq, const double* r, int ldr, int n_qu
                     int32_t* const* part_idx_host, double* const* part_dist_host, void* workspace,
                     size_t workspace_bytes, int64_t* stats_host, void* stream);
 
+/* ---- (3b) prepared reference: pack a reference once, map any number of query batches ------
+ * The reference-side operands of the fast engine - the packed FP16 tensor-core tiles and their scale
+ * (Euclidean / cosine), or the FP32 copy, bin edges and bit planes of the sliced pass (modified Canberra) -
+ * depend on (reference rows, g, metric, ref_mask) alone.  nabo_ref_prepare builds them once into a caller-owned
+ * device buffer and fills a host descriptor; nabo_knn_prepared then maps query batches against it.  Every result
+ * is bit-identical to nabo_knn / nabo_knn_routed on the same inputs (the exact re-rank, the certificate and the
+ * exact fallback decide every row).  The descriptor keeps the caller's FP64 rows and mask by address (the re-rank
+ * and the fallback read them): both, and the buffer, must stay allocated and unchanged while it is in use.
+ *
+ * The tensor-core scale of a prepared reference comes from the reference's largest norm alone (cosine: 32), not
+ * from the queries: a query whose scaled coordinates would overflow FP16 (about 500x the largest reference norm)
+ * is sent to the exact fallback and counted in stats_host[1].
+ * Calls the prepared operands do not serve run the existing path on the stored rows: mode = NABO_MODE_EXACT, k
+ * beyond the fast plans (the exact engine), and modified Canberra with dist_factor < 1e-6 (the FP16 two-phase pass);
+ * nabo_knn_prepared_workspace_bytes then returns the one-shot size.
+ * Status: a descriptor that was not filled by nabo_ref_prepare or does not match its buffer -> NABO_EINVAL; another
+ * ABI version, a metric / g without a fast plan (1 <= g <= 128) or k + drop_first > 128 -> NABO_EUNSUPPORTED. */
+#define NABO_PREPARED_MAGIC 0x5250424eu   /* "NBPR" */
+#define NABO_PLAN_TC 1                     /* tensor-core operands (Euclidean, cosine)   */
+#define NABO_PLAN_SLICED 2                 /* bit-sliced operands (modified Canberra)    */
+typedef struct nabo_prepared_ref {
+    uint32_t magic;            /* NABO_PREPARED_MAGIC                                        */
+    int abi_version;           /* NABO_ABI_VERSION of the library that prepared it           */
+    int n_ref, g, metric, plan;
+    const double* r;           /* the caller's FP64 rows (n_ref x g, row stride ldr)         */
+    int ldr;
+    const uint8_t* ref_mask;   /* the caller's mask or NULL                                  */
+    void* buffer;              /* the caller's buffer (nabo_ref_prepared_bytes)              */
+    size_t buffer_bytes;
+    const void* ops[3];        /* operand addresses inside buffer (tiles, scale / FP32 copy, planes, edges) */
+} nabo_prepared_ref;
+
+/* device bytes of the prepared operands; 0 when metric / g have no fast plan.  Tensor-core plan: 128-row tiles of
+ * 2 * ceil16(3g + 3) bytes per row (320 B per row at g = 50) + 8 B per row. */
+size_t nabo_ref_prepared_bytes(int n_ref, int g, int metric);
+int nabo_ref_prepare(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* ref_mask, void* buffer,
+                     size_t buffer_bytes, nabo_prepared_ref* prepared_host, void* stream);
+/* per-call (query-side) workspace; smaller than nabo_knn_workspace_bytes by the reference's share.  0 for an
+ * invalid descriptor. */
+size_t nabo_knn_prepared_workspace_bytes(int n_query, const nabo_prepared_ref* prepared_host, int k,
+                                         double dist_factor, int mode);
+int nabo_knn_prepared(const double* q, int ldq, int n_query, const nabo_prepared_ref* prepared_host, int k,
+                      double dist_factor, int drop_first, int idx_offset, int mode, int32_t* out_idx,
+                      double* out_dist, void* workspace, size_t workspace_bytes, int64_t* stats_host, void* stream);
+int nabo_knn_prepared_routed(const double* q, int ldq, int n_query, const nabo_prepared_ref* prepared_host, int k,
+                             double dist_factor, int drop_first, int idx_offset, int mode, int n_parts,
+                             const int* part_bounds_host, int32_t* const* part_idx_host,
+                             double* const* part_dist_host, void* workspace, size_t workspace_bytes,
+                             int64_t* stats_host, void* stream);
+
 /* ---- (4) SNN neighbour weights: replaces _calc_snn ------------------------------
  * nabo/_mapping.py:151-200.  counts[t][j] = |set(tgt_knn[t]) & set(ref_knn[tgt_knn[t][j]])|
  * weights[t][j] = lut[counts] with lut[s] = round(s / (2(k-1) - s), 2) built on

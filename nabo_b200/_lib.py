@@ -25,6 +25,15 @@ _i = C.c_int
 _d = C.c_double
 _z = C.c_size_t
 
+
+class PreparedDesc(C.Structure):
+    """``nabo_prepared_ref``: host descriptor of a prepared reference (filled by ``nabo_ref_prepare``)."""
+    _fields_ = [("magic", C.c_uint32), ("abi_version", _i), ("n_ref", _i), ("g", _i), ("metric", _i), ("plan", _i),
+                ("r", _p), ("ldr", _i), ("ref_mask", _p), ("buffer", _p), ("buffer_bytes", _z), ("ops", _p * 3)]
+
+
+_PD = C.POINTER(PreparedDesc)
+
 # name -> (restype, argtypes); mirrors include/nabo_b200.h one to one
 SIGNATURES: Dict[str, tuple] = {
     "nabo_abi_version": (_i, []),
@@ -44,6 +53,12 @@ SIGNATURES: Dict[str, tuple] = {
     "nabo_merge_topk_parts": (_i, [_i, _p, _p, _i, _i, _i, _p, _p, _p]),
     "nabo_knn_routed": (_i, [_p, _i, _p, _i, _i, _i, _i, _i, _i, _d, _p, _i, _i, _i, _i, _p, _p, _p, _p, _z,
                              C.POINTER(C.c_int64), _p]),
+    "nabo_ref_prepared_bytes": (_z, [_i, _i, _i]),
+    "nabo_ref_prepare": (_i, [_p, _i, _i, _i, _i, _p, _p, _z, _PD, _p]),
+    "nabo_knn_prepared_workspace_bytes": (_z, [_i, _PD, _i, _d, _i]),
+    "nabo_knn_prepared": (_i, [_p, _i, _i, _PD, _i, _d, _i, _i, _i, _p, _p, _p, _z, C.POINTER(C.c_int64), _p]),
+    "nabo_knn_prepared_routed": (_i, [_p, _i, _i, _PD, _i, _d, _i, _i, _i, _i, _p, _p, _p, _p, _z,
+                                      C.POINTER(C.c_int64), _p]),
     "nabo_score_accumulate": (_i, [_p, _p, _p, _i, _i, _i, _p, _p, _p]),
     "nabo_scores_finalize": (_i, [_p, _i, _d, _d, C.c_longlong, _d, _p, _p]),
     "nabo_snn_weights": (_i, [_p, _i, _i, _p, _i, _i, _p, _p, _p, _p]),

@@ -14,9 +14,9 @@ from typing import Dict, Optional
 import numpy as np
 import torch
 
-from ._lib import METRICS, MODE_EXACT, MODE_FAST, check, lib, require_device
+from ._lib import METRICS, MODE_EXACT, MODE_FAST, PreparedDesc, check, lib, require_device
 
-__all__ = ["euclidean_dist", "mod_canberra_dist", "cosine_dist", "knn", "knn_candidates", "rerank_exact", "merge_topk",
+__all__ = ["euclidean_dist", "mod_canberra_dist", "cosine_dist", "knn", "prepare_reference", "PreparedReference", "knn_candidates", "rerank_exact", "merge_topk",
            "merge_topk_parts", "snn_int_weights", "score_accumulate", "scores_finalize", "snn_weight_lut", "fix_weight", "snn_weights", "mapping_scores", "classify_targets", "mapping_specificity", "sparse_row_stats", "connected_components",
            "project", "project_csr", "scale_counts", "map_cells", "map_cells_host", "resolve_metric"]
 
@@ -125,27 +125,111 @@ def cosine_dist(x, y, d=None):
 
 
 # ----------------------------------------------------------------------------- (2) kNN
-def knn(q, r, k: int, metric: str = "euclidean", dist_factor: float = 0.25, ref_mask=None,
+PREPARED_MAX_G = 128      # widest PCA space with a prepared form (the fast plans' limit, nabo_ref_prepared_bytes)
+
+
+class PreparedReference:
+    """A reference packed once for any number of ``knn`` calls (``nabo_ref_prepare``): the reference-side operands
+    of the fast engine for one (rows, g, metric, mask) in a device buffer this object owns, plus the FP64 rows and
+    the mask it keeps on the device (the exact re-rank and fallback read them).  Results are bit-identical to
+    ``knn`` with the raw rows.  Device memory: the packed tensor-core tiles take 2 * ceil16(3g + 3) bytes per
+    reference (about 31 MB per 100 k references at g = 50); see ``nbytes``.
+
+    The rows must not change while the object is in use: a CUDA tensor passed in (or the float64 copy made of
+    it) that is modified in place afterwards makes every later call raise ``ValueError``.  NumPy input is copied
+    at preparation, so later changes to the array are not seen at all."""
+
+    def __init__(self, r, metric: str, ref_mask=None):
+        require_device()
+        if metric not in METRICS:
+            raise ValueError("ERROR: unknown metric %r" % (metric,))
+        rd = _dev(r, torch.float64)
+        if rd.dim() != 2 or rd.shape[0] < 1:
+            raise ValueError("ERROR: the reference must be a non-empty 2-D array")
+        md = _mask_dev(ref_mask)
+        if md is not None and md.numel() != rd.shape[0]:
+            raise ValueError("ERROR: ref_mask must have one entry per reference cell")
+        self.metric = metric
+        self.n_ref, self.g = int(rd.shape[0]), int(rd.shape[1])
+        self.r, self.mask, self._mask_src = rd, md, ref_mask
+        self._sources = [(t, t._version) for t in {id(x): x for x in (r, rd, ref_mask, md)
+                                                   if isinstance(x, torch.Tensor)}.values()]
+        L = lib()
+        nbytes = int(L.nabo_ref_prepared_bytes(self.n_ref, self.g, METRICS[metric]))
+        if nbytes == 0:
+            raise ValueError("ERROR: metric %r with g=%d has no prepared form (1 <= g <= 128)" % (metric, self.g))
+        self.buffer = torch.empty(nbytes, dtype=torch.uint8, device=rd.device)
+        self.desc = PreparedDesc()
+        check(L.nabo_ref_prepare(_ptr(rd), self.g, self.n_ref, self.g, METRICS[metric], _ptr(md), _ptr(self.buffer),
+                                 nbytes, C.byref(self.desc), C.c_void_p(_stream())), "ref_prepare")
+
+    @property
+    def shape(self):
+        return (self.n_ref, self.g)
+
+    @property
+    def device(self):
+        return self.r.device
+
+    @property
+    def nbytes(self) -> int:
+        """Device bytes of the packed operands (the FP64 rows and the mask not included)."""
+        return self.buffer.numel()
+
+    def check_unchanged(self) -> None:
+        for t, v in self._sources:
+            if t._version != v:
+                raise ValueError("ERROR: the reference rows or mask were modified in place after prepare_reference; "
+                                 "prepare the reference again")
+
+
+def prepare_reference(r, metric: str, ref_mask=None) -> PreparedReference:
+    """Pack the reference ``r`` (M,g) once for ``metric`` (and ``ref_mask``); pass the result to ``knn`` /
+    ``map_cells`` / the sharded mappers in place of ``r``."""
+    return PreparedReference(r, metric, ref_mask)
+
+
+def _check_prepared_args(pr: PreparedReference, metric, ref_mask, g: int) -> str:
+    """Metric, mask and g of a call on a prepared reference come from the object; conflicting arguments raise."""
+    if metric is not None and metric != pr.metric:
+        raise ValueError("ERROR: metric %r conflicts with the prepared reference's %r" % (metric, pr.metric))
+    if ref_mask is not None and ref_mask is not pr._mask_src and ref_mask is not pr.mask:
+        raise ValueError("ERROR: ref_mask comes from the prepared reference; do not pass another one")
+    if g != pr.g:
+        raise ValueError("ERROR: queries have %d columns, the prepared reference %d" % (g, pr.g))
+    pr.check_unchanged()
+    return pr.metric
+
+
+def knn(q, r, k: int, metric: Optional[str] = None, dist_factor: float = 0.25, ref_mask=None,
         drop_first: bool = False, idx_offset: int = 0, mode: str = "fast", return_stats: bool = False, out=None,
         out_parts=None):
     """Fused distance + per-query top-k: what ``_calc_dist`` (nabo/_mapping.py:48-148) leaves
     for ``_calc_snn`` to read (``[:k]`` of each sorted row), without the N x M matrix.
 
     q (N,g), r (M,g) float64.  ``ref_mask`` (M,) bool marks ``ignore_ref_cells`` (sorted last,
-    :135-140); ``drop_first`` is the reference<->reference ``[1:]`` (:141-142).
+    :135-140); ``drop_first`` is the reference<->reference ``[1:]`` (:141-142).  ``metric`` defaults to
+    Euclidean.  ``r`` may be a ``PreparedReference``: metric, mask and g then come from it (a conflicting
+    ``metric`` / ``ref_mask`` / query width raises ``ValueError``) and the reference is not packed again.
     Returns (idx int32 (N,k), dist float64 (N,k)) [+ stats dict].
 
     ``out_parts=(bounds, idx_ptrs, dist_ptrs)`` routes the result rows instead (``nabo_knn_routed``): row t
     with bounds[p] <= t < bounds[p+1] is written to row t - bounds[p] of the (rows_p, k) int32 / float64
     blocks at the device ADDRESSES idx_ptrs[p] / dist_ptrs[p] (local buffers or NVLink-mapped peer memory);
     the call then returns (None, None)."""
+    pr = r if isinstance(r, PreparedReference) else None
+    if pr is not None:
+        metric = _check_prepared_args(pr, metric, ref_mask, _ncols(q))
+    elif metric is None:
+        metric = "euclidean"
     require_device()
     if metric not in METRICS:
         raise ValueError("ERROR: unknown metric %r" % (metric,))
     if mode not in ("fast", "exact"):
         raise ValueError("ERROR: mode must be 'fast' or 'exact'")
-    host = _is_host(q, r)
-    qd, rd = _dev(q, torch.float64), _dev(r, torch.float64)
+    host = _is_host(q) if pr is not None else _is_host(q, r)
+    qd = _dev(q, torch.float64)
+    rd = pr.r if pr is not None else _dev(r, torch.float64)
     if qd.dim() != 2 or rd.dim() != 2 or qd.shape[1] != rd.shape[1]:
         raise ValueError("ERROR: q and r must be 2-D with the same number of columns")
     n, g = qd.shape
@@ -153,12 +237,12 @@ def knn(q, r, k: int, metric: str = "euclidean", dist_factor: float = 0.25, ref_
     k = int(k)
     if k < 1 or k + (1 if drop_first else 0) > m:
         raise ValueError("ERROR: k=%d is not in 1..%d" % (k, m - (1 if drop_first else 0)))
-    md = _mask_dev(ref_mask)
+    md = pr.mask if pr is not None else _mask_dev(ref_mask)
     if md is not None and md.numel() != m:
         raise ValueError("ERROR: ref_mask must have one entry per reference cell")
     if out_parts is not None:
         return _knn_routed(qd, rd, n, m, g, k, metric, dist_factor, md, drop_first, idx_offset, mode, out_parts,
-                           return_stats)
+                           return_stats, pr)
     if out is not None:                                    # caller-owned (n, k) int32 / float64 device buffers
         idx, dst = out
         if tuple(idx.shape) != (n, k) or tuple(dst.shape) != (n, k) or idx.dtype != torch.int32 or \
@@ -169,12 +253,19 @@ def knn(q, r, k: int, metric: str = "euclidean", dist_factor: float = 0.25, ref_
         dst = torch.empty((n, k), dtype=torch.float64, device=qd.device)
     mode_i = MODE_FAST if mode == "fast" else MODE_EXACT
     L = lib()
-    ws_bytes = int(L.nabo_knn_workspace_bytes(n, m, g, k, METRICS[metric], mode_i))
-    ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=qd.device)
     stats = (C.c_int64 * 8)() if return_stats else None
-    check(L.nabo_knn(_ptr(qd), g, _ptr(rd), g, n, m, g, k, METRICS[metric], float(dist_factor), _ptr(md),
-                     1 if drop_first else 0, int(idx_offset), mode_i, _ptr(idx), _ptr(dst), _ptr(ws),
-                     ws.numel(), stats, C.c_void_p(_stream())), "knn")
+    if pr is not None:
+        ws_bytes = int(L.nabo_knn_prepared_workspace_bytes(n, C.byref(pr.desc), k, float(dist_factor), mode_i))
+        ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=qd.device)
+        check(L.nabo_knn_prepared(_ptr(qd), g, n, C.byref(pr.desc), k, float(dist_factor), 1 if drop_first else 0,
+                                  int(idx_offset), mode_i, _ptr(idx), _ptr(dst), _ptr(ws), ws.numel(), stats,
+                                  C.c_void_p(_stream())), "knn_prepared")
+    else:
+        ws_bytes = int(L.nabo_knn_workspace_bytes(n, m, g, k, METRICS[metric], mode_i))
+        ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=qd.device)
+        check(L.nabo_knn(_ptr(qd), g, _ptr(rd), g, n, m, g, k, METRICS[metric], float(dist_factor), _ptr(md),
+                         1 if drop_first else 0, int(idx_offset), mode_i, _ptr(idx), _ptr(dst), _ptr(ws),
+                         ws.numel(), stats, C.c_void_p(_stream())), "knn")
     res = (_out(idx, host), _out(dst, host))
     if return_stats:
         res = res + (_stats_dict(stats),)
@@ -188,22 +279,34 @@ def _stats_dict(stats):
             "fallback_ms": stats[6] / 1e6, "prep_ms": stats[7] / 1e6}
 
 
-def _knn_routed(qd, rd, n, m, g, k, metric, dist_factor, md, drop_first, idx_offset, mode, out_parts, return_stats):
+def _ncols(x) -> int:
+    return int(x.shape[1]) if getattr(x, "ndim", 0) == 2 else -1
+
+
+def _knn_routed(qd, rd, n, m, g, k, metric, dist_factor, md, drop_first, idx_offset, mode, out_parts, return_stats,
+                pr=None):
     bounds, idx_ptrs, dist_ptrs = out_parts
     n_parts = len(idx_ptrs)
     if len(bounds) != n_parts + 1 or len(dist_ptrs) != n_parts:
         raise ValueError("ERROR: out_parts needs n_parts + 1 bounds and n_parts idx / dist addresses")
     mode_i = MODE_FAST if mode == "fast" else MODE_EXACT
     L = lib()
-    ws_bytes = int(L.nabo_knn_workspace_bytes(n, m, g, k, METRICS[metric], mode_i))
-    ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=qd.device)
     stats = (C.c_int64 * 8)() if return_stats else None
     b = (C.c_int * (n_parts + 1))(*[int(x) for x in bounds])
     pi = (C.c_void_p * n_parts)(*[int(x) if x else None for x in idx_ptrs])
     pd = (C.c_void_p * n_parts)(*[int(x) if x else None for x in dist_ptrs])
-    check(L.nabo_knn_routed(_ptr(qd), g, _ptr(rd), g, n, m, g, k, METRICS[metric], float(dist_factor), _ptr(md),
-                            1 if drop_first else 0, int(idx_offset), mode_i, n_parts, b, pi, pd, _ptr(ws), ws.numel(),
-                            stats, C.c_void_p(_stream())), "knn_routed")
+    if pr is not None:
+        ws_bytes = int(L.nabo_knn_prepared_workspace_bytes(n, C.byref(pr.desc), k, float(dist_factor), mode_i))
+        ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=qd.device)
+        check(L.nabo_knn_prepared_routed(_ptr(qd), g, n, C.byref(pr.desc), k, float(dist_factor), 1 if drop_first else 0,
+                                         int(idx_offset), mode_i, n_parts, b, pi, pd, _ptr(ws), ws.numel(), stats,
+                                         C.c_void_p(_stream())), "knn_prepared_routed")
+    else:
+        ws_bytes = int(L.nabo_knn_workspace_bytes(n, m, g, k, METRICS[metric], mode_i))
+        ws = torch.empty(max(ws_bytes, 256), dtype=torch.uint8, device=qd.device)
+        check(L.nabo_knn_routed(_ptr(qd), g, _ptr(rd), g, n, m, g, k, METRICS[metric], float(dist_factor), _ptr(md),
+                                1 if drop_first else 0, int(idx_offset), mode_i, n_parts, b, pi, pd, _ptr(ws),
+                                ws.numel(), stats, C.c_void_p(_stream())), "knn_routed")
     return (None, None, _stats_dict(stats)) if return_stats else (None, None)
 
 
@@ -595,6 +698,16 @@ def project_csr(indptr, col, val, gene_pos, sf, mu, sigma, components, mean):
 
 
 # ----------------------------------------------------------------------------- whole path
+def _call_metric(pr: Optional[PreparedReference], metric: Optional[str]) -> str:
+    """The mapping metric of a call: the prepared reference's when one is given (``knn`` rejects a conflicting
+    ``metric``), else the reference's dispatch (modified Canberra for targets)."""
+    if pr is not None:
+        if metric is not None and metric != pr.metric:
+            raise ValueError("ERROR: metric %r conflicts with the prepared reference's %r" % (metric, pr.metric))
+        return pr.metric
+    return resolve_metric(metric, False)
+
+
 def map_cells(target, ref, ref_knn, k: int, metric: Optional[str] = None, dist_factor: float = 0.25,
               ref_mask=None, mode: str = "fast", pca_model: Optional[Dict] = None,
               scores: bool = True) -> Dict[str, object]:
@@ -606,21 +719,23 @@ def map_cells(target, ref, ref_knn, k: int, metric: Optional[str] = None, dist_f
       ref      (M,g) float64 reference PCA coordinates
       ref_knn  (M,k) int32 reference self-kNN (``make_ref_graph``'s sorted rows)
 
+    ``ref`` may be a ``PreparedReference`` (``prepare_reference``): the metric and mask then come from it.
     Returns dict(idx, dist, counts, weights, scores[, pca]) - NumPy if the inputs were."""
-    host = _is_host(target, ref, ref_knn)
+    pr = ref if isinstance(ref, PreparedReference) else None
+    m = _call_metric(pr, metric)
+    host = _is_host(target, ref_knn) if pr is not None else _is_host(target, ref, ref_knn)
     res: Dict[str, object] = {}
+    rd = pr.r if pr is not None else _dev(ref, torch.float64)
     if pca_model is not None:
         tq = project(_dev(target, torch.float32), pca_model["gene_idx"], pca_model["sf"], pca_model["mu"],
                      pca_model["sigma"], pca_model["components"], pca_model["mean"])
-        g = _dev(ref, torch.float64).shape[1]
+        g = rd.shape[1]
         res["pca"] = tq
         tq = tq[:, :g].contiguous()
     else:
         tq = _dev(target, torch.float64)
-    rd = _dev(ref, torch.float64)
     rk = _dev(ref_knn, torch.int32)
-    m = resolve_metric(metric, False)
-    idx, dst = knn(tq, rd, k, m, dist_factor, ref_mask, False, 0, mode)
+    idx, dst = knn(tq, pr if pr is not None else rd, k, m, dist_factor, ref_mask, False, 0, mode)
     cnt, w = snn_weights(idx, rk, k)
     res.update(idx=idx, dist=dst, counts=cnt, weights=w)
     if scores:
@@ -659,9 +774,10 @@ def map_cells_host(target_host: torch.Tensor, ref, ref_knn, k: int, metric: Opti
     land in pinned host tensors (idx, dist, weights, scores).  The targets are processed in ``chunks``
     pieces so that the host->device copy of piece i+1 and the device->host copy of piece i-1 overlap the
     kernels of piece i (three CUDA streams); the per-reference scores are integer weight sums accumulated piece by
-    piece (``score_accumulate``), finalised once."""
+    piece (``score_accumulate``), finalised once.  ``ref`` may be a ``PreparedReference``."""
     require_device()
-    rd = _dev(ref, torch.float64)
+    pr = ref if isinstance(ref, PreparedReference) else None
+    rd = pr.r if pr is not None else _dev(ref, torch.float64)
     rk = _dev(ref_knn, torch.int32)
     n, g = target_host.shape
     m = rd.shape[0]
@@ -670,7 +786,7 @@ def map_cells_host(target_host: torch.Tensor, ref, ref_knn, k: int, metric: Opti
     if pipe is None:
         _PIPE.clear()
         pipe = _PIPE[key] = _HostPipeline(n, g, int(k), m, rd.device)
-    met = resolve_metric(metric, False)
+    met = _call_metric(pr, metric)
     comp = torch.cuda.current_stream()
     chunks = max(1, min(int(chunks), n // int(min_piece) if n >= 2 * int(min_piece) else 1))
     bounds = [n * i // chunks for i in range(chunks + 1)]
@@ -692,7 +808,7 @@ def map_cells_host(target_host: torch.Tensor, ref, ref_knn, k: int, metric: Opti
         ready.append(ev)
     for (lo, hi), ev in zip(zip(bounds, bounds[1:]), ready):
         comp.wait_event(ev)
-        knn(pipe.dev_in[lo:hi], rd, k, met, dist_factor, ref_mask, False, 0, mode, out=(pipe.idx[lo:hi], pipe.dist[lo:hi]))
+        knn(pipe.dev_in[lo:hi], pr if pr is not None else rd, k, met, dist_factor, ref_mask, False, 0, mode, out=(pipe.idx[lo:hi], pipe.dist[lo:hi]))
         found = torch.cuda.Event()
         found.record(comp)
         with torch.cuda.stream(pipe.s_out):                 # neighbours go home while the weights are still being made

@@ -667,14 +667,20 @@ static int cbs_grid(int n_groups) {
     return n_groups < sms ? n_groups : sms;
 }
 
-size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g) {
+// planes + bin edges: the reference half of the extra workspace (and of a prepared reference's buffer)
+static size_t cbs_ref_extra_bytes(int n_ref, int g) {
     const cbs::SmemPlan pl = cbs::plan_smem(g);
     const size_t n_tiles = (n_ref + pl.rt - 1) / pl.rt;
+    return nabo_align_up(n_tiles * cbs::plane_tile_bytes(g, pl.rt), 256) +
+           nabo_align_up((size_t)g * (cbs::NBINS - 1) * 4, 256);
+}
+
+size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g, bool with_ref) {
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
     const size_t n_groups = (size_t)(n_query + 31) / 32;
     const int nj = cbs::nblocks8(g) * 4;
     size_t b = 0;
-    b += nabo_align_up(n_tiles * cbs::plane_tile_bytes(g, pl.rt), 256);
-    b += nabo_align_up((size_t)g * (cbs::NBINS - 1) * 4, 256);
+    if (with_ref) b += cbs_ref_extra_bytes(n_ref, g);
     b += nabo_align_up(n_groups * nj * 32 * 4, 256);
     b += nabo_align_up(n_groups * g * 32 * 4, 256);
     b += nabo_align_up((size_t)148 * pl.nw * 32 * cbs::CAP * 8, 256);
@@ -696,10 +702,57 @@ int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first) {
     return s < 1 ? 1 : s;
 }
 
-// cand: [n_query][n_split][K'], tau: [n_split][n_query]
+// The reference half of the sliced pass: the FP32 copy rt (nabo_cb_pretile_floats(n_ref, g) floats), the bin edges
+// and the cumulative planes.  None of it depends on the queries or on dist_factor.
+static int cbs_ref_launch(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, float* rt, float* edges,
+                          uint32_t* planes, cudaStream_t st) {
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
+    const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
+    const int n_yblk = (n_ref + pl.yw - 1) / pl.yw;
+    if (pl.yw == 64) {
+        int rc = nabo_cb_pretile_launch(r, ldr, n_ref, g, rt, st);
+        if (rc) return rc;
+    } else {
+        const long long tr = (long long)n_yblk * g * 32;
+        cbs::pretile32_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, rt, tr);
+    }
+    cbs::edges_kernel<<<g, 1024, 0, st>>>(r, ldr, n_ref, edges);
+    switch (pl.rt) {
+        case 128: cbs::planes_kernel<128, 64><<<dim3(n_tiles, g), 128, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
+        case 64: cbs::planes_kernel<64, 32><<<dim3(n_tiles, g), 64, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
+        default: cbs::planes_kernel<32, 32><<<dim3(n_tiles, g), 32, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
+    }
+    return 0;
+}
+
+size_t nabo_cbs_prepared_bytes(int n_ref, int g) {
+    return nabo_align_up(nabo_cb_pretile_floats(n_ref, g) * 4, 256) + cbs_ref_extra_bytes(n_ref, g);
+}
+
+// A prepared reference's sliced operands, in the layout nabo_cbs_candidates builds per call.
+int nabo_cbs_prepare_ref(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, void* buffer, NaboCbsRef* out,
+                         cudaStream_t st) {
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
+    const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
+    NaboArena ar(buffer, nabo_cbs_prepared_bytes(n_ref, g));
+    float* rt = ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
+    uint32_t* planes = (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g, pl.rt));
+    float* edges = ar.take<float>((size_t)g * (cbs::NBINS - 1));
+    if (!ar.ok) return nabo_set_error(NABO_EINVAL, "ref_prepare: buffer layout");
+    int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
+    if (rc) return rc;
+    NABO_LAUNCH_CHECK("cbs reference preparation");
+    out->rt = rt;
+    out->planes = planes;
+    out->edges = edges;
+    return 0;
+}
+
+// cand: [n_query][n_split][K'], tau: [n_split][n_query].  pre != NULL: rt, planes and edges come from a prepared
+// reference (rt, r and mask are not read); extra then needs only the query half (nabo_cbs_extra_bytes(.., false)).
 int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                         double f, const uint8_t* mask, int drop_first, int n_split, float* rt, void* extra,
-                        size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st) {
+                        size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st, const NaboCbsRef* pre) {
     const int kprime = nabo_cb_kprime(k, drop_first);
     if (n_split < 1 || n_split > NABO_CBS_MAX_SPLIT) n_split = 1;
     const cbs::SmemPlan pl = cbs::plan_smem(g);
@@ -712,26 +765,18 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     if (grid < n_split) n_split = 1, grid = cbs_grid((int)n_groups);
 
     NaboArena ar(extra, extra_bytes);
-    uint32_t* planes = (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g, pl.rt));
-    float* edges = ar.take<float>((size_t)g * (cbs::NBINS - 1));
+    uint32_t* planes = pre ? (uint32_t*)pre->planes : (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g, pl.rt));
+    float* edges = pre ? (float*)pre->edges : ar.take<float>((size_t)g * (cbs::NBINS - 1));
     uint32_t* ctrl = ar.take<uint32_t>(n_groups * nj * 32);
     float* qx = ar.take<float>(n_groups * g * 32);
     unsigned long long* cbuf = ar.take<unsigned long long>((size_t)grid * pl.nw * 32 * cbs::CAP);
     if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the sliced Canberra pass");
+    if (pre) rt = (float*)pre->rt;
 
     {
-        if (pl.yw == 64) {
-            int rc = nabo_cb_pretile_launch(r, ldr, n_ref, g, rt, st);
+        if (!pre) {
+            int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
             if (rc) return rc;
-        } else {
-            const long long tr = (long long)n_yblk * g * 32;
-            cbs::pretile32_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, rt, tr);
-        }
-        cbs::edges_kernel<<<g, 1024, 0, st>>>(r, ldr, n_ref, edges);
-        switch (pl.rt) {
-            case 128: cbs::planes_kernel<128, 64><<<dim3(n_tiles, g), 128, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
-            case 64: cbs::planes_kernel<64, 32><<<dim3(n_tiles, g), 64, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
-            default: cbs::planes_kernel<32, 32><<<dim3(n_tiles, g), 32, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
         }
         const long long tc = (long long)n_groups * nj * 32;
         cbs::ctrl_kernel<<<(unsigned)((tc + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, nj, f, edges, ctrl, tc);

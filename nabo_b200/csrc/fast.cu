@@ -25,10 +25,27 @@ size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metri
            nabo_align_up(nabo_exact_split_workspace(k + 1), 256) + 1024;
 }
 
+// The prepared operands serve a call when its engine is the one they were built for; the size below covers every
+// drop_first, so it is the query half only where both take that engine (else the full one-shot size).
+static bool cbs_prepared_used(int g, int k, int drop_first, double f) { return f >= 1e-6 && nabo_cbs_supported(g, k, drop_first); }
+
+size_t nabo_fast_prepared_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, double f) {
+    if (metric == NABO_MOD_CANBERRA) {
+        if (!cbs_prepared_used(g, k, 1, f)) return nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
+        return nabo_align_up((size_t)n_query * nabo_cb_kprime(k, 1) * 4 * NABO_CBS_MAX_SPLIT, 256) +
+               (2 + NABO_CBS_MAX_SPLIT) * nabo_align_up((size_t)n_query * 4, 256) +
+               nabo_align_up(nabo_exact_split_workspace(k + 1), 256) +
+               nabo_align_up(nabo_cbs_extra_bytes(n_query, n_ref, g, false), 256) + 4096;
+    }
+    if (!nabo_tc_supported(g, k, 1)) return nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
+    return nabo_tc_workspace_bytes(n_query, n_ref, g, k, 1, false) + nabo_align_up((size_t)n_query * 4, 256) +
+           nabo_align_up(nabo_exact_split_workspace(k + 1), 256) + 1024;
+}
+
 int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                   int metric, double f, const uint8_t* mask, int drop_first, int idx_offset, int32_t* out_idx,
                   double* out_dist, const NaboRoute& route, void* workspace, size_t workspace_bytes,
-                  int64_t* stats_host, cudaStream_t st) {
+                  int64_t* stats_host, cudaStream_t st, const NaboFastRef* pre) {
     NaboStageTimer tm(stats_host != nullptr, st);
     tm.begin();
     const bool use_tc = (metric == NABO_EUCLIDEAN || metric == NABO_COSINE) && nabo_tc_supported(g, k, drop_first) &&
@@ -39,8 +56,11 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
     const bool use_cb = metric == NABO_MOD_CANBERRA && (sliced_ok || nabo_cb_supported(g, k, drop_first)) &&
                         n_ref > nabo_cb_kprime(k, drop_first);
     if (use_cb) {
-        if (workspace_bytes < nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric))
-            return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small");
+        // a prepared reference's sliced operands replace the FP32 copy, planes and edges of this call
+        const NaboCbsRef* pre_cb = sliced_ok && pre && pre->cbs.planes ? &pre->cbs : nullptr;
+        const size_t need = pre ? nabo_fast_prepared_workspace_bytes(n_query, n_ref, g, k, metric, f)
+                                : nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
+        if (workspace_bytes < need) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small");
         NaboArena ar(workspace, workspace_bytes);
         const int kprime = nabo_cb_kprime(k, drop_first);
         const int n_split = sliced_ok ? nabo_cbs_split(n_query, n_ref, g, k, drop_first) : 1;
@@ -48,15 +68,16 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
         float* tau = ar.take<float>((size_t)n_query * n_split);
         int* fail_rows = ar.take<int>(n_query);
         int* fail_count = ar.take<int>(1);
-        float* qt = ar.take<float>(nabo_cb_pretile_floats(n_query, g));
-        float* rt = ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
+        float* qt = pre_cb ? nullptr : ar.take<float>(nabo_cb_pretile_floats(n_query, g));
+        float* rt = pre_cb ? nullptr : ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
         char* split_ws = ar.take<char>(nabo_exact_split_workspace(k + (drop_first ? 1 : 0)));
-        char* extra = ar.take<char>(cb_extra_bytes(n_query, n_ref, g));
+        const size_t extra_bytes = pre_cb ? nabo_cbs_extra_bytes(n_query, n_ref, g, false) : cb_extra_bytes(n_query, n_ref, g);
+        char* extra = ar.take<char>(extra_bytes);
         if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small");
         NABO_CUDA(cudaMemsetAsync(fail_count, 0, sizeof(int), st));
         int rc = sliced_ok
                      ? nabo_cbs_candidates(q, ldq, r, ldr, n_query, n_ref, g, k, f, mask, drop_first, n_split, rt, extra,
-                                           cb_extra_bytes(n_query, n_ref, g), cand, tau, st)
+                                           extra_bytes, cand, tau, st, pre_cb)
                      : nabo_cb_candidates(q, ldq, r, ldr, n_query, n_ref, g, k, f, mask, drop_first, qt, rt, extra, cand,
                                           tau, st);
         if (rc) return rc;
@@ -98,9 +119,11 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
         }
         return 0;
     }
-    if (workspace_bytes < nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric))
-        return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small (%zu < %zu)", workspace_bytes,
-                              nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric));
+    const NaboTcRef* pre_tc = pre && pre->tc.rb ? &pre->tc : nullptr;
+    const size_t need = pre ? nabo_fast_prepared_workspace_bytes(n_query, n_ref, g, k, metric, f)
+                            : nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
+    if (workspace_bytes < need)
+        return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small (%zu < %zu)", workspace_bytes, need);
     NaboArena ar(workspace, workspace_bytes);
     int32_t* cand = nullptr;
     float* tau = nullptr;
@@ -120,7 +143,7 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
     tail.rows_full = 0; tail.applies = 0;
     tail.dry = stats_host != nullptr;      // stage timing asked for: the candidate kernel is timed on its own
     int rc = nabo_tc_candidates(q, ldq, r, ldr, n_query, n_ref, g, k, metric, mask, drop_first, &n_split, ar, &cand,
-                                &kprime, &tau, &qn2, &scal, &launches, tm, st, &raw, &tail);  // n_split out: K' lists per query
+                                &kprime, &tau, &qn2, &scal, &launches, tm, st, &raw, &tail, pre_tc);  // n_split out: K' lists per query
     if (rc) return rc;
     if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small");
     NaboCert cert;

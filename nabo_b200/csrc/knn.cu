@@ -3,6 +3,8 @@
 #include "common.cuh"
 #include "knn_internal.cuh"
 
+#include <string.h>
+
 extern "C" size_t nabo_knn_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, int mode) {
     if (mode == NABO_MODE_EXACT) return 256;
     return nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
@@ -11,7 +13,25 @@ extern "C" size_t nabo_knn_workspace_bytes(int n_query, int n_ref, int g, int k,
 static int knn_impl(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                     int metric, double dist_factor, const uint8_t* ref_mask, int drop_first, int idx_offset,
                     int mode, int32_t* out_idx, double* out_dist, const NaboRoute& route, void* workspace,
-                    size_t workspace_bytes, int64_t* stats_host, void* stream);
+                    size_t workspace_bytes, int64_t* stats_host, void* stream, const NaboFastRef* pre = nullptr);
+
+static int parse_route(int n_query, int n_parts, const int* part_bounds_host, int32_t* const* part_idx_host,
+                       double* const* part_dist_host, NaboRoute& route) {
+    NABO_ARG(n_parts >= 1 && n_parts <= NABO_MAX_PARTS, "knn_routed: n_parts=%d outside 1..%d", n_parts, NABO_MAX_PARTS);
+    NABO_ARG(part_bounds_host && part_idx_host && part_dist_host, "knn_routed: null table");
+    NABO_ARG(part_bounds_host[0] == 0 && part_bounds_host[n_parts] == n_query,
+             "knn_routed: part bounds must run from 0 to n_query");
+    route.n_parts = n_parts;
+    for (int p = 0; p <= n_parts; ++p) route.bounds[p] = part_bounds_host[p];
+    for (int p = 0; p < n_parts; ++p) {
+        NABO_ARG(route.bounds[p] <= route.bounds[p + 1], "knn_routed: part bounds must not decrease");
+        NABO_ARG(route.bounds[p] == route.bounds[p + 1] || (part_idx_host[p] && part_dist_host[p]),
+                 "knn_routed: part %d has rows but no buffers", p);
+        route.idx[p] = part_idx_host[p];
+        route.dist[p] = part_dist_host[p];
+    }
+    return 0;
+}
 
 extern "C" int nabo_knn(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                         int metric, double dist_factor, const uint8_t* ref_mask, int drop_first, int idx_offset,
@@ -28,20 +48,9 @@ extern "C" int nabo_knn_routed(const double* q, int ldq, const double* r, int ld
                                int idx_offset, int mode, int n_parts, const int* part_bounds_host,
                                int32_t* const* part_idx_host, double* const* part_dist_host, void* workspace,
                                size_t workspace_bytes, int64_t* stats_host, void* stream) {
-    NABO_ARG(n_parts >= 1 && n_parts <= NABO_MAX_PARTS, "knn_routed: n_parts=%d outside 1..%d", n_parts, NABO_MAX_PARTS);
-    NABO_ARG(part_bounds_host && part_idx_host && part_dist_host, "knn_routed: null table");
-    NABO_ARG(part_bounds_host[0] == 0 && part_bounds_host[n_parts] == n_query,
-             "knn_routed: part bounds must run from 0 to n_query");
     NaboRoute route;
-    route.n_parts = n_parts;
-    for (int p = 0; p <= n_parts; ++p) route.bounds[p] = part_bounds_host[p];
-    for (int p = 0; p < n_parts; ++p) {
-        NABO_ARG(route.bounds[p] <= route.bounds[p + 1], "knn_routed: part bounds must not decrease");
-        NABO_ARG(route.bounds[p] == route.bounds[p + 1] || (part_idx_host[p] && part_dist_host[p]),
-                 "knn_routed: part %d has rows but no buffers", p);
-        route.idx[p] = part_idx_host[p];
-        route.dist[p] = part_dist_host[p];
-    }
+    int rc = parse_route(n_query, n_parts, part_bounds_host, part_idx_host, part_dist_host, route);
+    if (rc) return rc;
     return knn_impl(q, ldq, r, ldr, n_query, n_ref, g, k, metric, dist_factor, ref_mask, drop_first, idx_offset, mode,
                     nullptr, nullptr, route, workspace, workspace_bytes, stats_host, stream);
 }
@@ -49,7 +58,7 @@ extern "C" int nabo_knn_routed(const double* q, int ldq, const double* r, int ld
 static int knn_impl(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                     int metric, double dist_factor, const uint8_t* ref_mask, int drop_first, int idx_offset,
                     int mode, int32_t* out_idx, double* out_dist, const NaboRoute& route, void* workspace,
-                    size_t workspace_bytes, int64_t* stats_host, void* stream) {
+                    size_t workspace_bytes, int64_t* stats_host, void* stream, const NaboFastRef* pre) {
     cudaStream_t st = (cudaStream_t)stream;
     NABO_ARG(n_query >= 0 && n_ref >= 1 && g >= 1 && k >= 1, "knn: bad sizes n_query=%d n_ref=%d g=%d k=%d",
              n_query, n_ref, g, k);
@@ -77,5 +86,139 @@ static int knn_impl(const double* q, int ldq, const double* r, int ldr, int n_qu
     }
     NABO_ARG(mode == NABO_MODE_FAST, "knn: unknown mode %d", mode);
     return nabo_knn_fast(q, ldq, r, ldr, n_query, n_ref, g, k, metric, dist_factor, ref_mask, drop_first,
-                         idx_offset, out_idx, out_dist, route, workspace, workspace_bytes, stats_host, st);
+                         idx_offset, out_idx, out_dist, route, workspace, workspace_bytes, stats_host, st, pre);
+}
+
+// ------------------------------------------------------------------ prepared reference
+// Buffer layout: the reference half of the fast engine's operands for the metric (tc_candidates.cu /
+// canberra_sliced.cu own the layout inside), at offset 0.  The descriptor keeps the device addresses.
+static bool prepared_plan(int g, int metric, int* plan) {
+    if (g < 1 || g > 128) return false;
+    if (metric == NABO_EUCLIDEAN || metric == NABO_COSINE) {
+        *plan = NABO_PLAN_TC;
+        return nabo_tc_supported(g, 1, 0);
+    }
+    if (metric == NABO_MOD_CANBERRA) {
+        *plan = NABO_PLAN_SLICED;
+        return nabo_cbs_supported(g, 1, 0);
+    }
+    return false;
+}
+
+extern "C" size_t nabo_ref_prepared_bytes(int n_ref, int g, int metric) {
+    int plan = 0;
+    if (n_ref < 1 || !prepared_plan(g, metric, &plan)) return 0;
+    return plan == NABO_PLAN_TC ? nabo_tc_prepared_bytes(n_ref, g) : nabo_cbs_prepared_bytes(n_ref, g);
+}
+
+extern "C" int nabo_ref_prepare(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* ref_mask,
+                                void* buffer, size_t buffer_bytes, nabo_prepared_ref* prepared_host, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    NABO_ARG(prepared_host, "ref_prepare: null descriptor");
+    memset(prepared_host, 0, sizeof(*prepared_host));
+    int plan = 0;
+    if (!prepared_plan(g, metric, &plan))
+        return nabo_set_error(NABO_EUNSUPPORTED, "ref_prepare: metric %d with g=%d has no fast plan (1 <= g <= 128)",
+                              metric, g);
+    NABO_ARG(n_ref >= 1 && ldr >= g, "ref_prepare: bad sizes n_ref=%d ldr=%d g=%d", n_ref, ldr, g);
+    NABO_ARG(r && buffer, "ref_prepare: null pointer");
+    const size_t need = nabo_ref_prepared_bytes(n_ref, g, metric);
+    NABO_ARG(buffer_bytes >= need, "ref_prepare: buffer too small (%zu < %zu)", buffer_bytes, need);
+    nabo_prepared_ref d;
+    memset(&d, 0, sizeof(d));
+    d.magic = NABO_PREPARED_MAGIC;
+    d.abi_version = NABO_ABI_VERSION;
+    d.n_ref = n_ref; d.g = g; d.metric = metric; d.plan = plan;
+    d.r = r; d.ldr = ldr; d.ref_mask = ref_mask;
+    d.buffer = buffer; d.buffer_bytes = buffer_bytes;
+    if (plan == NABO_PLAN_TC) {
+        NaboTcRef t;
+        int rc = nabo_tc_prepare_ref(r, ldr, n_ref, g, metric, ref_mask, buffer, &t, st);
+        if (rc) return rc;
+        d.ops[0] = t.rb; d.ops[1] = t.scal;
+    } else {
+        NaboCbsRef c;
+        int rc = nabo_cbs_prepare_ref(r, ldr, n_ref, g, ref_mask, buffer, &c, st);
+        if (rc) return rc;
+        d.ops[0] = c.rt; d.ops[1] = c.planes; d.ops[2] = c.edges;
+    }
+    *prepared_host = d;
+    return 0;
+}
+
+// A descriptor this library prepared, unchanged: NABO_EINVAL otherwise (NABO_EUNSUPPORTED for another ABI version).
+static int check_prepared(const nabo_prepared_ref* pr, NaboFastRef* ops) {
+    NABO_ARG(pr, "knn_prepared: null descriptor");
+    NABO_ARG(pr->magic == NABO_PREPARED_MAGIC, "knn_prepared: not a prepared reference (bad magic)");
+    if (pr->abi_version != NABO_ABI_VERSION)
+        return nabo_set_error(NABO_EUNSUPPORTED, "knn_prepared: prepared by ABI version %d, this library is %d",
+                              pr->abi_version, NABO_ABI_VERSION);
+    int plan = 0;
+    if (!prepared_plan(pr->g, pr->metric, &plan))
+        return nabo_set_error(NABO_EUNSUPPORTED, "knn_prepared: metric %d with g=%d has no fast plan", pr->metric, pr->g);
+    NABO_ARG(pr->plan == plan, "knn_prepared: plan %d does not match metric %d", pr->plan, pr->metric);
+    NABO_ARG(pr->n_ref >= 1 && pr->ldr >= pr->g, "knn_prepared: bad descriptor sizes");
+    NABO_ARG(pr->r && pr->buffer, "knn_prepared: descriptor without rows or buffer");
+    NABO_ARG(pr->buffer_bytes >= nabo_ref_prepared_bytes(pr->n_ref, pr->g, pr->metric),
+             "knn_prepared: descriptor buffer smaller than its shape needs");
+    memset(ops, 0, sizeof(*ops));
+    for (int i = 0; i < (plan == NABO_PLAN_TC ? 2 : 3); ++i) {
+        const char* a = (const char*)pr->ops[i];
+        NABO_ARG(a >= (const char*)pr->buffer && a < (const char*)pr->buffer + pr->buffer_bytes,
+                 "knn_prepared: operand %d outside the buffer", i);
+    }
+    if (plan == NABO_PLAN_TC) {
+        ops->tc.rb = pr->ops[0];
+        ops->tc.scal = (const double*)pr->ops[1];
+    } else {
+        ops->cbs.rt = (const float*)pr->ops[0];
+        ops->cbs.planes = (const uint32_t*)pr->ops[1];
+        ops->cbs.edges = (const float*)pr->ops[2];
+    }
+    return 0;
+}
+
+extern "C" size_t nabo_knn_prepared_workspace_bytes(int n_query, const nabo_prepared_ref* prepared_host, int k,
+                                                    double dist_factor, int mode) {
+    NaboFastRef ops;
+    if (check_prepared(prepared_host, &ops) != 0) return 0;
+    if (mode == NABO_MODE_EXACT) return 256;
+    return nabo_fast_prepared_workspace_bytes(n_query, prepared_host->n_ref, prepared_host->g, k, prepared_host->metric,
+                                              dist_factor);
+}
+
+static int knn_prepared_impl(const double* q, int ldq, int n_query, const nabo_prepared_ref* pr, int k,
+                             double dist_factor, int drop_first, int idx_offset, int mode, int32_t* out_idx,
+                             double* out_dist, const NaboRoute& route, void* workspace, size_t workspace_bytes,
+                             int64_t* stats_host, void* stream) {
+    NaboFastRef ops;
+    int rc = check_prepared(pr, &ops);
+    if (rc) return rc;
+    if (k < 1 || k + (drop_first ? 1 : 0) > 128)
+        return nabo_set_error(NABO_EUNSUPPORTED, "knn_prepared: k=%d outside the kNN plans (k + drop_first <= 128)", k);
+    return knn_impl(q, ldq, pr->r, pr->ldr, n_query, pr->n_ref, pr->g, k, pr->metric, dist_factor, pr->ref_mask,
+                    drop_first, idx_offset, mode, out_idx, out_dist, route, workspace, workspace_bytes, stats_host,
+                    stream, &ops);
+}
+
+extern "C" int nabo_knn_prepared(const double* q, int ldq, int n_query, const nabo_prepared_ref* prepared_host, int k,
+                                 double dist_factor, int drop_first, int idx_offset, int mode, int32_t* out_idx,
+                                 double* out_dist, void* workspace, size_t workspace_bytes, int64_t* stats_host,
+                                 void* stream) {
+    NaboRoute plain;
+    plain.n_parts = 0;
+    return knn_prepared_impl(q, ldq, n_query, prepared_host, k, dist_factor, drop_first, idx_offset, mode, out_idx,
+                             out_dist, plain, workspace, workspace_bytes, stats_host, stream);
+}
+
+extern "C" int nabo_knn_prepared_routed(const double* q, int ldq, int n_query, const nabo_prepared_ref* prepared_host,
+                                        int k, double dist_factor, int drop_first, int idx_offset, int mode, int n_parts,
+                                        const int* part_bounds_host, int32_t* const* part_idx_host,
+                                        double* const* part_dist_host, void* workspace, size_t workspace_bytes,
+                                        int64_t* stats_host, void* stream) {
+    NaboRoute route;
+    int rc = parse_route(n_query, n_parts, part_bounds_host, part_idx_host, part_dist_host, route);
+    if (rc) return rc;
+    return knn_prepared_impl(q, ldq, n_query, prepared_host, k, dist_factor, drop_first, idx_offset, mode, nullptr,
+                             nullptr, route, workspace, workspace_bytes, stats_host, stream);
 }

@@ -103,16 +103,28 @@ struct NaboTailSplit {
     int applies;               // out: 1 when the shape qualifies (with or without dry)
 };
 
+// Reference half of the tensor-core operands, built once by nabo_tc_prepare_ref (prepared reference, prepared.cu):
+// the packed tiles in the layout the one-shot path writes, and the scale {sc, 1/sc, max scaled reference norm, cosine}.
+struct NaboTcRef {
+    const void* rb;
+    const double* scal;
+};
+
 struct NaboStageTimer;
 bool nabo_tc_supported(int g, int k, int drop_first);
 int nabo_tc_kprime(int k, int drop_first);
-size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first);
+size_t nabo_tc_ref_bytes(int n_ref, int g);
+size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first, bool with_ref = true);
+size_t nabo_tc_prepared_bytes(int n_ref, int g);
+int nabo_tc_prepare_ref(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* mask, void* buffer,
+                        NaboTcRef* out, cudaStream_t st);
 #define NABO_TC_MAX_SPLIT 3
 int nabo_tc_split(int n_query, int n_ref, int g);
 int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                        int metric, const uint8_t* mask, int drop_first, int* n_split_io, NaboArena& ar, int32_t** cand_idx_out,
                        int* kprime_out, float** cert_tau_out, double** qn2_out, double** scal_out, int* launches,
-                       NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out = nullptr, NaboTailSplit* tail = nullptr);
+                       NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out = nullptr, NaboTailSplit* tail = nullptr,
+                       const NaboTcRef* pre = nullptr);
 
 bool nabo_cb_supported(int g, int k, int drop_first);
 int nabo_cb_kprime(int k, int drop_first);
@@ -125,20 +137,38 @@ int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n
 
 int nabo_cb_pretile_launch(const double* x, int ld, int n, int g, float* out, cudaStream_t st);
 // bit-sliced Canberra pass (canberra_sliced.cu); same outputs as nabo_cb_candidates
+// Reference half of the sliced pass, built once by nabo_cbs_prepare_ref: FP32 copy, cumulative planes, bin edges.
+struct NaboCbsRef {
+    const float* rt;
+    const uint32_t* planes;
+    const float* edges;
+};
 bool nabo_cbs_supported(int g, int k, int drop_first);
-size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g);
+size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g, bool with_ref = true);
+size_t nabo_cbs_prepared_bytes(int n_ref, int g);
+int nabo_cbs_prepare_ref(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, void* buffer, NaboCbsRef* out,
+                         cudaStream_t st);
 #define NABO_CBS_MAX_SPLIT 3
 int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first);
 int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                         double f, const uint8_t* mask, int drop_first, int n_split, float* rt, void* extra,
-                        size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st);
+                        size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st, const NaboCbsRef* pre = nullptr);
 int nabo_tau_min_launch(float* tau, int n_query, int n_split, cudaStream_t st);
 
+// Reference-side operands of a prepared reference (prepared.cu): the tensor-core tiles (Euclidean / cosine) or the
+// sliced-pass state (modified Canberra); the pointers of the other engine are NULL.
+struct NaboFastRef {
+    NaboTcRef tc;
+    NaboCbsRef cbs;
+};
 size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric);
+// per-call workspace of nabo_knn_fast with a prepared reference (smaller by the reference's share wherever the
+// prepared operands are used for every drop_first; the full size otherwise)
+size_t nabo_fast_prepared_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, double f);
 int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                   int metric, double f, const uint8_t* mask, int drop_first, int idx_offset, int32_t* out_idx,
                   double* out_dist, const NaboRoute& route, void* workspace, size_t workspace_bytes,
-                  int64_t* stats_host, cudaStream_t st);
+                  int64_t* stats_host, cudaStream_t st, const NaboFastRef* pre = nullptr);
 
 // CUDA-event stage timer, active only when the caller asked for stats (stats_host != NULL).
 // Usage: begin(); <launch stage 0>; end(0); <launch stage 1>; end(1); ... sync; ns(i).

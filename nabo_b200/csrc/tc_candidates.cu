@@ -238,6 +238,13 @@ pack_kernel(const double* __restrict__ x, int ld, int n, int g, int kp, const do
                 if (IS_QUERY) {
                     const __half src = seg == 2 ? lo : hi;
                     v = __float2half(-2.0f * __half2float(src));      // exact: power-of-two scaling
+                    if (__hisinf(v)) {
+                        // a query far outside the scale of a prepared reference (|x~| >= 32 760): its operand would
+                        // overflow FP16.  The row is fed zeros and its |q~|^2 becomes NaN, which fails the certificate
+                        // and sends it to the exact fallback.  (With the joint scale of the one-shot path |x~| < 64.)
+                        v = __float2half(0.f);
+                        n2 = CUDART_NAN;
+                    }
                 } else {
                     v = seg == 1 ? lo : hi;
                 }
@@ -805,18 +812,16 @@ int nabo_tau_min_launch(float* tau, int n_query, int n_split, cudaStream_t st) {
     return 0;
 }
 
-size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first) {
+size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first, bool with_ref) {
     const int kp = tc::kp_for(g);
     const size_t tb = tc::tile_bytes(kp);
     const int nq = tc::plan_smem(g).nq;
     const int n_items = (n_query + nq * tc::TILE - 1) / (nq * tc::TILE);
-    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
     const int kprime = nabo_tc_kprime(k, drop_first);
     size_t b = 0;
     b += nabo_align_up((size_t)n_items * nq * tb, 256);          // packed queries
-    b += nabo_align_up((size_t)n_rtiles * tb, 256);                   // packed references
+    if (with_ref) b += nabo_tc_ref_bytes(n_ref, g);                   // packed references, r norms, scale
     b += nabo_align_up((size_t)n_query * 8, 256) * 2;                 // q norms, qn2
-    b += nabo_align_up((size_t)n_ref * 8, 256);                       // r norms
     b += nabo_align_up((size_t)n_items * NABO_TC_MAX_SPLIT * nq * tc::TILE * (tc::CAP * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
     b += nabo_align_up((size_t)n_query * kprime * 4 * NABO_TC_MAX_SPLIT, 256);   // candidate indices (per reference range)
     b += nabo_align_up((size_t)n_query * 4 * NABO_TC_MAX_SPLIT, 256) + nabo_align_up((size_t)n_query * 4, 256);   // cert tau, fail rows
@@ -825,12 +830,57 @@ size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_fi
     return b;
 }
 
+// ------------------------------------------------------------------ reference half of the operands
+// Packed reference tiles and their norms: what the workspace holds for one call, and the first part of a prepared
+// reference's buffer (which adds the scale and the norm maximum, kTcRefTail bytes).
+size_t nabo_tc_ref_bytes(int n_ref, int g) {
+    const size_t tb = tc::tile_bytes(tc::kp_for(g));
+    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
+    return nabo_align_up((size_t)n_rtiles * tb, 256) + nabo_align_up((size_t)n_ref * 8, 256);
+}
+static const size_t kTcRefTail = 512;      // scal[4] and the reference's norm maximum, 256-aligned pieces each
+
+static void tc_ref_norms(const double* r, int ldr, int n_ref, int g, double* rnorm, unsigned int* maxr_bits, cudaStream_t st) {
+    tc::norms_kernel<<<(n_ref + 255) / 256, 256, 0, st>>>(r, ldr, n_ref, g, rnorm, maxr_bits);
+}
+
+static void tc_ref_pack(const double* r, int ldr, int n_ref, int g, const double* rnorm, const double* scal,
+                        const uint8_t* mask, __half* rb, cudaStream_t st) {
+    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
+    tc::pack_kernel<false><<<n_rtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(r, ldr, n_ref, g, tc::kp_for(g), rnorm, scal, mask,
+                                                                          rb, nullptr);
+}
+
+size_t nabo_tc_prepared_bytes(int n_ref, int g) { return nabo_tc_ref_bytes(n_ref, g) + kTcRefTail; }
+
+// A prepared reference's operands: the same norms and packing as a one-shot call, but the scale comes from the
+// reference's largest norm alone (cosine: 32), so that any later query batch can use the tiles.
+int nabo_tc_prepare_ref(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* mask, void* buffer,
+                        NaboTcRef* out, cudaStream_t st) {
+    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
+    NaboArena ar(buffer, nabo_tc_prepared_bytes(n_ref, g));
+    __half* rb = (__half*)ar.take<char>((size_t)n_rtiles * tc::tile_bytes(tc::kp_for(g)));
+    double* rnorm = ar.take<double>(n_ref);
+    double* scal = ar.take<double>(4);
+    unsigned int* maxr = ar.take<unsigned int>(1);
+    if (!ar.ok) return nabo_set_error(NABO_EINVAL, "ref_prepare: buffer layout");
+    NABO_CUDA(cudaMemsetAsync(maxr, 0, sizeof(unsigned int), st));
+    tc_ref_norms(r, ldr, n_ref, g, rnorm, maxr, st);
+    tc::scale_kernel<<<1, 1, 0, st>>>(maxr, maxr, metric == NABO_COSINE ? 1 : 0, scal);
+    tc_ref_pack(r, ldr, n_ref, g, rnorm, scal, mask, rb, st);
+    NABO_LAUNCH_CHECK("tc reference preparation");
+    out->rb = rb;
+    out->scal = scal;
+    return 0;
+}
+
 // Runs norms -> scale -> pack -> candidate kernel.  Outputs (device, inside the arena):
-// cand_idx [n_query][kprime], cert_tau [n_query], qn2 [n_query], scal[4].
+// cand_idx [n_query][kprime], cert_tau [n_query], qn2 [n_query], scal[4].  pre != NULL: the reference half comes
+// from a prepared reference (nabo_tc_prepare_ref) and only the queries are packed, with its scale.
 int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                        int metric, const uint8_t* mask, int drop_first, int* n_split_io, NaboArena& ar, int32_t** cand_idx_out,
                        int* kprime_out, float** cert_tau_out, double** qn2_out, double** scal_out, int* launches,
-                       NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out, NaboTailSplit* tail) {
+                       NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out, NaboTailSplit* tail, const NaboTcRef* pre) {
     // raw_out != NULL: when every query has ONE buffer (no reference split, K' <= 64) the final selection is left to
     // the re-rank kernel: raw_out is filled and no emit kernel runs.
     // *n_split_io in: reference pieces per item when there are few items (nabo_tc_split), or 0 = one piece (the
@@ -847,26 +897,28 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     const int grid = tc_grid(n_items * n_split);
 
     __half* qa = (__half*)ar.take<char>((size_t)n_qtiles * tb);
-    __half* rb = (__half*)ar.take<char>((size_t)n_rtiles * tb);
+    __half* rb = pre ? (__half*)pre->rb : (__half*)ar.take<char>((size_t)n_rtiles * tb);
     double* qnorm = ar.take<double>(n_query);
     double* qn2 = ar.take<double>(n_query);
-    double* rnorm = ar.take<double>(n_ref);
+    double* rnorm = pre ? nullptr : ar.take<double>(n_ref);
     const size_t n_slots = (size_t)n_items * n_split * pl.nq * tc::TILE;
     unsigned long long* cbuf = ar.take<unsigned long long>(n_slots * tc::CAP);
     int* ccnt = ar.take<int>(n_slots);
     float* ctau = ar.take<float>(n_slots);
     int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_split);
     float* tau = ar.take<float>((size_t)n_query * n_split);
-    double* scal = ar.take<double>(4);
+    double* scal = pre ? (double*)pre->scal : ar.take<double>(4);
     unsigned int* maxbits = ar.take<unsigned int>(3 + (size_t)n_items);    // 2 norm maxima, CTA ticket, head flags
     if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the tensor-core pass");
 
     NABO_CUDA(cudaMemsetAsync(maxbits, 0, (3 + (size_t)n_items) * sizeof(unsigned int), st));
     tc::norms_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(q, ldq, n_query, g, qnorm, maxbits);
-    tc::norms_kernel<<<(n_ref + 255) / 256, 256, 0, st>>>(r, ldr, n_ref, g, rnorm, maxbits + 1);
-    tc::scale_kernel<<<1, 1, 0, st>>>(maxbits, maxbits + 1, metric == NABO_COSINE ? 1 : 0, scal);
+    if (!pre) {
+        tc_ref_norms(r, ldr, n_ref, g, rnorm, maxbits + 1, st);
+        tc::scale_kernel<<<1, 1, 0, st>>>(maxbits, maxbits + 1, metric == NABO_COSINE ? 1 : 0, scal);
+    }
     tc::pack_kernel<true><<<n_qtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(q, ldq, n_query, g, kp, qnorm, scal, nullptr, qa, qn2);
-    tc::pack_kernel<false><<<n_rtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(r, ldr, n_ref, g, kp, rnorm, scal, mask, rb, nullptr);
+    if (!pre) tc_ref_pack(r, ldr, n_ref, g, rnorm, scal, mask, rb, st);
     NABO_LAUNCH_CHECK("tc pack kernels");
     tm.end(3);
 
@@ -924,7 +976,7 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     if (fused) {
         raw_out->buf = cbuf; raw_out->cnt = ccnt; raw_out->tau = ctau; raw_out->kprime = kprime;
         *cand_idx_out = cand; *kprime_out = kprime; *cert_tau_out = tau; *qn2_out = qn2; *scal_out = scal;
-        *launches += 6;
+        *launches += pre ? 3 : 6;
         *n_split_io = 1;
         return 0;
     }
@@ -940,7 +992,7 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     }
     *n_split_io = n_split;
     *cand_idx_out = cand; *kprime_out = kprime; *cert_tau_out = tau; *qn2_out = qn2; *scal_out = scal;
-    *launches += 6;
+    *launches += pre ? 3 : 6;
     return 0;
 }
 

@@ -89,6 +89,7 @@ class Mapping:
         self._distFactor = None
         self._chunkSize = None
         self._refMatCache = None
+        self._refPrepCache = None       # (key, core.PreparedReference) of the last calc_dist, see _prepared_ref
 
     # ------------------------------------------------------------------ files
     @staticmethod
@@ -173,6 +174,7 @@ class Mapping:
         self._distFactor = dist_factor
         self._chunkSize = chunk_size
         self._refMatCache = None
+        self._refPrepCache = None
         return None
 
     def _ref_matrix(self) -> np.ndarray:
@@ -186,6 +188,22 @@ class Mapping:
                 mat = np.ascontiguousarray(mat[[pos[c] for c in self.refCells]])
             self._refMatCache = mat
         return self._refMatCache
+
+    def _prepared_ref(self, metric: str, ignore_ref_cells: List[str], mask) -> Optional["core.PreparedReference"]:
+        """The reference packed for (use_comps, metric, ignore_ref_cells), kept between calc_dist calls so that
+        mapping several targets uploads and packs the reference once.  One is kept at a time (its device memory:
+        the FP64 rows plus about 31 MB per 100 k references at use_comps = 50).  None where no prepared form
+        exists (use_comps > core.PREPARED_MAX_G): the call then takes the host matrix."""
+        key = (self._useComps, metric, frozenset(ignore_ref_cells))
+        if self._refPrepCache is not None and self._refPrepCache[0] == key:
+            return self._refPrepCache[1]
+        ref = self._ref_matrix()
+        if ref.shape[1] > core.PREPARED_MAX_G:
+            return None
+        self._refPrepCache = None                           # release the previous one before packing
+        pr = core.prepare_reference(ref, metric, mask)
+        self._refPrepCache = (key, pr)
+        return pr
 
     # ------------------------------------------------------------------ distances + top-k
     def calc_dist(self, target_fn: str, target_grp: str, dist_grp: str, sorted_dist_grp: str,
@@ -216,8 +234,12 @@ class Mapping:
         keep = min(self._k, m - (1 if drop else 0))
         if keep < 1:
             raise ValueError("ERROR: k=%s needs at least %d reference cells" % (self._k, 2 if drop else 1))
-        idx, dst = core.knn(tmat, ref, keep, metric, float(self._distFactor), ref_mask=mask, drop_first=drop,
-                            mode=mode)
+        pr = self._prepared_ref(metric, ignore_ref_cells, mask)
+        if pr is not None:
+            idx, dst = core.knn(tmat, pr, keep, metric, float(self._distFactor), drop_first=drop, mode=mode)
+        else:
+            idx, dst = core.knn(tmat, ref, keep, metric, float(self._distFactor), ref_mask=mask, drop_first=drop,
+                                mode=mode)
         out = open_file(self._h5Fn, mode="a")
         for g in (dist_grp, sorted_dist_grp):
             if g in out:

@@ -19,6 +19,10 @@ the path shards because every target cell is an independent query (nabo/_mapping
   (transport ``"a2a"``; also what the CPU/gloo tests run).  ``nabo_merge_topk_parts`` then merges
   the per-source blocks in place by (distance, index) - bit-identical to the unsharded result.
 
+Wherever a function takes ``ref`` / ``ref_shard`` it also takes a ``core.PreparedReference`` of it: a rank that
+maps many target batches against the same reference (or shard) prepares it once, and every step reuses the packed
+operands.  The metric and mask then come from the prepared object (pass ``ref_mask`` / ``ref_mask_shard`` = None).
+
 The compute engine is a parameter so that the host-side logic (bounds, offsets, block layout,
 merge slices) is testable on CPU with ``gloo``; the default engine is the CUDA library and
 raises without a GPU.
@@ -46,6 +50,14 @@ def _world() -> Tuple[int, int]:
     if dist.is_available() and dist.is_initialized():
         return dist.get_rank(), dist.get_world_size()
     return 0, 1
+
+
+def _metric_for(ref, metric: Optional[str]) -> str:
+    """The call's metric: an explicit one, else the prepared reference's, else modified Canberra (targets)."""
+    if metric:
+        return metric
+    from .core import PreparedReference
+    return ref.metric if isinstance(ref, PreparedReference) else "mod_canberra"
 
 
 # ----------------------------------------------------------------------------- engines
@@ -211,7 +223,7 @@ def map_targets_sharded(target_shard, ref, ref_knn, k: int, n_targets_total: int
     mapping scores (identical on every rank, and for every world size, after the integer all-reduce)."""
     engine = engine or CudaEngine()
     rank, world = _world()
-    metric = metric or "mod_canberra"
+    metric = _metric_for(ref, metric)
     idx, dst = engine.knn(target_shard, ref, k, metric, dist_factor, ref_mask, False, 0, mode)
     cnt, w = engine.snn_weights(idx, ref_knn, k)
     out = {"idx": idx, "dist": dst, "counts": cnt, "weights": w}
@@ -305,7 +317,7 @@ def map_reference_sharded(targets, ref_shard, ref_offset: int, n_ref_total: int,
     target block [lo, hi)."""
     engine = engine or CudaEngine()
     rank, world = _world()
-    metric = metric or "mod_canberra"
+    metric = _metric_for(ref_shard, metric)
     lo, hi, idx, dst = knn_reference_sharded(targets, ref_shard, ref_offset, k, metric, dist_factor, ref_mask_shard,
                                              False, mode, engine, merge_slice=True, transport=transport,
                                              timings=timings)
