@@ -79,6 +79,12 @@ int nabo_cosine_dist(const double* x, int ldx, const double* y, int ldy, double*
  *              [4] ns spent in the dominant distance/top-k kernel (CUDA events on
  *              `stream`), [5] ns in the exact re-rank, [6] ns in the exact fallback,
  *              [7] ns in operand preparation.
+ *   mode = NABO_MODE_FAST runs the candidate pass + re-rank where a fast plan exists, and
+ *   the exact engine (same results) elsewhere; ksel = k + drop_first:
+ *     Euclidean / cosine  1 <= g <= 128, ksel <= 128 (tensor-core pass: 128-key buffers for
+ *                         ksel + 8 <= 96, 256-key buffers for 89 <= ksel <= 128)
+ *     modified Canberra   ksel + 8 <= 64; g <= 128 with dist_factor >= 1e-6 (bit-sliced
+ *                         pass), g <= 77 otherwise (FP16 two-phase pass)
  */
 size_t nabo_knn_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, int mode);
 int nabo_knn(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,

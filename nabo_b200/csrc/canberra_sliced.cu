@@ -374,7 +374,7 @@ sliced_kernel(const Params p) {
             need &= need - 1;
             int nc;
             float nt;
-            compact_select(gbuf + (size_t)src * CAP, s_cnt[src], lane, kprime, trig - 4 > kprime ? trig - 4 : kprime, hist, nc, nt);
+            compact_select<CAP / 32>(gbuf + (size_t)src * CAP, s_cnt[src], lane, kprime, trig - 4 > kprime ? trig - 4 : kprime, hist, nc, nt);
             if (lane == src) { s_cnt[lane] = nc; s_tau[lane] = nt; }
             __syncwarp();
             CBS_PROF_COUNT(9, 1)

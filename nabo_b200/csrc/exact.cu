@@ -687,7 +687,9 @@ extern "C" int nabo_dbg_rr_stats(unsigned long long* out_host, int reset) {
     return 0;
 }
 #endif
-template <int METRIC, bool FROM_BUF>
+// NS: candidate slots per lane - 4 for capp <= 128; 8 for capp = 256 (Euclidean / cosine without FROM_BUF: the
+// 256-key tensor-core plan, K' up to 160)
+template <int METRIC, bool FROM_BUF, int NS = 4>
 __global__ void __launch_bounds__(128)
 rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ r, int ldr, int n_query,
               int n_ref, int g, int k, double f, const uint8_t* __restrict__ mask, int drop_first,
@@ -695,6 +697,7 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
               int* __restrict__ fail_rows, int* __restrict__ fail_count,
               int32_t* __restrict__ out_idx, double* __restrict__ out_dist, const NaboRoute route,
               const NaboCandBuf cb, int xs_dims, bool vec2, int row0) {
+    static_assert(NS == 4 || (NS == 8 && !FROM_BUF), "8 slots per lane: candidate lists only (capp = 256)");
     extern __shared__ double smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int qi = row0 + blockIdx.x * 4 + warp;
@@ -800,11 +803,11 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
         __syncwarp();
     }
     const double* xq = xw ? xw : x;
-    int jj[4];
+    int jj[NS];
     int n_slots = 0;
     const bool scramble = (long long)n_ref * ldr * 8 > (96ll << 20);
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < NS; ++u) {
         const int c = u * 32 + lane;
         int j = -1;
         if (u * 32 < capp) {
@@ -822,19 +825,22 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
         jj[u] = j;
         if (__any_sync(0xffffffffu, j >= 0)) n_slots = u + 1;
     }
-    double accs[4] = {0.0, 0.0, 0.0, 0.0};
+    double accs[NS];
+#pragma unroll
+    for (int u = 0; u < NS; ++u) accs[u] = 0.0;
     if (METRIC == NABO_MOD_CANBERRA) {
         // the FP64 division sits under a divergent branch: slot by slot, so that a slot with few lanes costs few divisions
 #pragma unroll
-        for (int u = 0; u < 4; ++u)
+        for (int u = 0; u < NS; ++u)
             if (u < n_slots) pair_rows<METRIC, 1>(xq, r, ldr, jj + u, g, f, vec2, accs + u);
     } else if (n_slots == 1) pair_rows<METRIC, 1>(xq, r, ldr, jj, g, f, vec2, accs);
     else if (n_slots == 2) pair_rows<METRIC, 2>(xq, r, ldr, jj, g, f, vec2, accs);
+    else if (NS > 4 && n_slots > 4) pair_rows<METRIC, NS>(xq, r, ldr, jj, g, f, vec2, accs);
     else if (n_slots > 2) pair_rows<METRIC, 4>(xq, r, ldr, jj, g, f, vec2, accs);
     int n_valid = 0, n_finite = 0;
-    int ids[4];
+    int ids[NS];
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {
+    for (int u = 0; u < NS; ++u) {
         const int j = jj[u];
         double key = CUDART_INF;
         int id = 0x7fffffff;
@@ -863,9 +869,12 @@ rerank_kernel(const double* __restrict__ q, int ldq, const double* __restrict__ 
 #pragma unroll
         for (int u = 0; u < 2; ++u) { d[u * 32 + lane] = d2[u]; ix[u * 32 + lane] = i2[u]; }
     } else {
-        warp_bitonic_sort_regs<4>(accs, ids, lane);
+        // every slot of every lane holds a candidate position: capp == 32 * NS (128 for NS = 4, 256 for NS = 8; the
+        // launcher picks NS = 8 only for capp > 128)
+        NABO_DEV_ASSERT(capp == 32 * NS);
+        warp_bitonic_sort_regs<NS>(accs, ids, lane);
 #pragma unroll
-        for (int u = 0; u < 4; ++u) { d[u * 32 + lane] = accs[u]; ix[u * 32 + lane] = ids[u]; }
+        for (int u = 0; u < NS; ++u) { d[u * 32 + lane] = accs[u]; ix[u * 32 + lane] = ids[u]; }
     }
     __syncwarp();
     for (int o = 16; o > 0; o >>= 1) {
@@ -903,7 +912,9 @@ int nabo_rerank_launch(const double* q, int ldq, const double* r, int ldr, int n
                        const int32_t* cand, int n_cand, const NaboCert& cert, int* fail_rows, int* fail_count,
                        int32_t* out_idx, double* out_dist, const NaboRoute& route, cudaStream_t st,
                        const NaboCandBuf* from_buf, int row0, bool dependent) {
-    NABO_ARG(n_cand >= 1 && n_cand <= 128, "rerank: n_cand=%d unsupported (1..128)", n_cand);
+    // up to 128 candidates per query; 256 for Euclidean / cosine (the 256-key tensor-core plan, K' <= 160)
+    const int max_cand = metric == NABO_MOD_CANBERRA ? 128 : 256;
+    NABO_ARG(n_cand >= 1 && n_cand <= max_cand, "rerank: n_cand=%d unsupported (1..%d)", n_cand, max_cand);
     NABO_ARG(k >= 1 && k + (drop_first ? 1 : 0) <= n_cand, "rerank: k=%d does not fit n_cand=%d", k, n_cand);
     NABO_ARG(row0 >= 0 && row0 <= n_query, "rerank: row0=%d outside [0, %d]", row0, n_query);
     if (n_query - row0 == 0) return 0;
@@ -942,10 +953,17 @@ int nabo_rerank_launch(const double* q, int ldq, const double* r, int ldr, int n
         NABO_CUDA(cudaLaunchKernelEx(&cfg, rerank_kernel<M, false>, q, ldq, r, ldr, n_query, n_ref, g, k, f, mask, \
                                      drop_first, idx_offset, cand, n_cand, capp, cert, fail_rows, fail_count,  \
                                      out_idx, out_dist, route, cb, xs_dims, vec2, row0));
-    if (metric == NABO_EUCLIDEAN) { LAUNCH(NABO_EUCLIDEAN) }
+#define LAUNCH_WIDE(M)                                                                                         \
+    if (capp > 128)                                                                                            \
+        NABO_CUDA(cudaLaunchKernelEx(&cfg, rerank_kernel<M, false, 8>, q, ldq, r, ldr, n_query, n_ref, g, k, f,   \
+                                     mask, drop_first, idx_offset, cand, n_cand, capp, cert, fail_rows,        \
+                                     fail_count, out_idx, out_dist, route, cb, xs_dims, vec2, row0));          \
+    else LAUNCH(M)
+    if (metric == NABO_EUCLIDEAN) { LAUNCH_WIDE(NABO_EUCLIDEAN) }
     else if (metric == NABO_MOD_CANBERRA) { LAUNCH(NABO_MOD_CANBERRA) }
-    else if (metric == NABO_COSINE) { LAUNCH(NABO_COSINE) }
+    else if (metric == NABO_COSINE) { LAUNCH_WIDE(NABO_COSINE) }
     else return nabo_set_error(NABO_EINVAL, "rerank: unknown metric %d", metric);
+#undef LAUNCH_WIDE
 #undef LAUNCH
     NABO_LAUNCH_CHECK("rerank_kernel");
     return 0;
@@ -957,6 +975,7 @@ extern "C" int nabo_rerank_exact(const double* q, int ldq, const double* r, int 
                                  int32_t* out_idx, double* out_dist, void* stream) {
     NABO_ARG(q && r && cand && out_idx && out_dist, "rerank: null pointer");
     NABO_ARG(ldq >= g && ldr >= g, "rerank: leading dimension smaller than g");
+    NABO_ARG(n_cand >= 1 && n_cand <= 128, "rerank: n_cand=%d unsupported (1..128)", n_cand);
     NaboCert none;
     none.kind = NABO_CERT_NONE; none.tau = nullptr; none.qn2 = nullptr; none.scal = nullptr; none.c_acc = 0.0; none.abs_slack = 0.0;
     NaboRoute plain;

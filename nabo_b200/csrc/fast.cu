@@ -15,13 +15,21 @@ static size_t cb_extra_bytes(int n_query, int n_ref, int g) {
     return a > b ? a : b;
 }
 
+// Tensor-core share of the workspace for every drop_first: with drop_first the buffer plan may be the 256-key one
+// (k + 1 >= 89) while k alone still takes the 128-key plan with its reference splits, so the larger of the two.
+static size_t tc_workspace_any_drop(int n_query, int n_ref, int g, int k, bool with_ref) {
+    const size_t a = nabo_tc_workspace_bytes(n_query, n_ref, g, k, 1, with_ref);
+    const size_t b = nabo_tc_workspace_bytes(n_query, n_ref, g, k, 0, with_ref);
+    return a > b ? a : b;
+}
+
 size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric) {
     if (metric == NABO_MOD_CANBERRA)
         return nabo_align_up((size_t)n_query * nabo_cb_kprime(k, 1) * 4 * NABO_CBS_MAX_SPLIT, 256) +
                (2 + NABO_CBS_MAX_SPLIT) * nabo_align_up((size_t)n_query * 4, 256) +
                nabo_align_up(nabo_cb_pretile_floats(n_query, g) * 4, 256) + nabo_align_up(nabo_cb_pretile_floats(n_ref, g) * 4, 256) +
                nabo_align_up(nabo_exact_split_workspace(k + 1), 256) + nabo_align_up(cb_extra_bytes(n_query, n_ref, g), 256) + 4096;
-    return nabo_tc_workspace_bytes(n_query, n_ref, g, k, 1) + nabo_align_up((size_t)n_query * 4, 256) +
+    return tc_workspace_any_drop(n_query, n_ref, g, k, true) + nabo_align_up((size_t)n_query * 4, 256) +
            nabo_align_up(nabo_exact_split_workspace(k + 1), 256) + 1024;
 }
 
@@ -38,7 +46,7 @@ size_t nabo_fast_prepared_workspace_bytes(int n_query, int n_ref, int g, int k, 
                nabo_align_up(nabo_cbs_extra_bytes(n_query, n_ref, g, false), 256) + 4096;
     }
     if (!nabo_tc_supported(g, k, 1)) return nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
-    return nabo_tc_workspace_bytes(n_query, n_ref, g, k, 1, false) + nabo_align_up((size_t)n_query * 4, 256) +
+    return tc_workspace_any_drop(n_query, n_ref, g, k, false) + nabo_align_up((size_t)n_query * 4, 256) +
            nabo_align_up(nabo_exact_split_workspace(k + 1), 256) + 1024;
 }
 
@@ -132,7 +140,8 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
     NaboCandBuf raw;
     raw.buf = nullptr;
     int n_split = nabo_tc_split(n_query, n_ref, g);              // > 1 only when there are fewer query items than SMs
-    while (n_split > 1 && n_split * nabo_tc_kprime(k, drop_first) > 128) --n_split;     // the re-rank takes <= 128 candidates
+    // split lists stay within 128 candidates per query: every K' > 64 (and the whole 256-key plan) runs unsplit
+    while (n_split > 1 && n_split * nabo_tc_kprime(k, drop_first) > 128) --n_split;
     // the failure list first: the re-rank of the full waves may start while the candidate pass is still running
     int* fail_rows = ar.take<int>(n_query);
     int* fail_count = ar.take<int>(1);

@@ -6,8 +6,10 @@
 
 namespace sel {
 
-constexpr int CAP = 128;        // keys per query buffer
-constexpr int KPL = CAP / 32;   // keys per lane: element i = u * 32 + lane sits in slot u of its lane
+// A buffer holds 32 * KPL keys (KPL keys per lane: element i = u * 32 + lane sits in slot u of its lane); KPL is a
+// template parameter of every routine below.  CAP: the 128-key buffers of the Canberra pass, the fused re-rank
+// (exact.cu) and the tensor-core pass up to K' = 96; the tensor-core pass for K' > 96 uses 256 keys (tc_candidates.cu).
+constexpr int CAP = 128;
 
 // buffer key = raw float bits of the score (high word) | local reference index (low word);
 // the compaction routines convert to an order-preserving integer when they load a key
@@ -16,7 +18,7 @@ __device__ __forceinline__ unsigned long long make_key(float score, uint32_t col
 }
 
 // ---- warp-cooperative compaction entirely in registers -----------------------------------
-// The CAP keys of one query are spread KPL per lane (element i = u*32 + lane) and sorted by
+// The 32 * KPL keys of one query are spread KPL per lane (element i = u*32 + lane) and sorted by
 // score with a bitonic network: strides >= 32 are register-to-register, smaller strides are
 // shuffles.  Only the score is compared (ties keep an arbitrary member; everything dropped
 // still has score >= the new threshold, which is all the certificate needs).
@@ -26,6 +28,7 @@ __device__ __forceinline__ void cex(uint32_t& s0, uint32_t& p0, uint32_t& s1, ui
     if (sw) { uint32_t t = s0; s0 = s1; s1 = t; t = p0; p0 = p1; p1 = t; }
 }
 
+template <int KPL>
 __device__ __forceinline__ void sortn(uint32_t (&s)[KPL], uint32_t (&pl)[KPL], int lane) {
 #pragma unroll
     for (int size = 2; size <= 32 * KPL; size <<= 1) {
@@ -61,6 +64,7 @@ __device__ __forceinline__ void sortn(uint32_t (&s)[KPL], uint32_t (&pl)[KPL], i
 // buffer.  New count / threshold come back through nc / nt (valid on every lane); s / pl hold the sorted
 // keys.  Force-inlined where the caller consumes s / pl (the per-item final emit) so that the arrays
 // stay in registers; compact_select uses the out-of-line wrapper below as its rare fallback.
+template <int KPL>
 __device__ __forceinline__ void compact_sort_inline(unsigned long long* gbuf, int n, int lane, int kprime,
                                                     uint32_t (&s)[KPL], uint32_t (&pl)[KPL], int& nc, float& nt) {
     __syncwarp();            // the owner's appends (plain global stores) are ordered before our loads
@@ -89,6 +93,7 @@ __device__ __forceinline__ void compact_sort_inline(unsigned long long* gbuf, in
     __syncwarp();
 }
 
+template <int KPL>
 static __device__ __noinline__ void compact_sort(unsigned long long* gbuf, int n, int lane, int kprime, int& nc, float& nt) {
     uint32_t s[KPL], pl[KPL];
     compact_sort_inline(gbuf, n, lane, kprime, s, pl, nc, nt);
@@ -101,6 +106,7 @@ static __device__ __noinline__ void compact_sort(unsigned long long* gbuf, int n
 // ("everything rejected or dropped has score >= tau") holds without an exact selection.
 // If the cut keeps more than max_keep keys (ties, duplicates) the exact sort takes over.
 // hist: 256 counters of this warp in shared memory.
+template <int KPL>
 static __device__ __noinline__ void compact_select(unsigned long long* gbuf, int n, int lane, int kprime, int max_keep,
                                             uint32_t* hist, int& nc, float& nt) {
     __syncwarp();
@@ -163,7 +169,7 @@ static __device__ __noinline__ void compact_select(unsigned long long* gbuf, int
         kept = __shfl_sync(0xffffffffu, k_at, owner);
     }
     if ((int)kept > max_keep) {
-        compact_sort(gbuf, n, lane, kprime, nc, nt);
+        compact_sort<KPL>(gbuf, n, lane, kprime, nc, nt);
         return;
     }
     // stream-compact the kept keys to the front (all keys are in registers: in-place is safe)
@@ -189,6 +195,7 @@ static __device__ __noinline__ void compact_select(unsigned long long* gbuf, int
 // The histogram cut of compact_select on keys already in registers: bin[u] of every live key and the cut bin with
 // at least kprime keys at or below it (kept = how many).  reach = false when n < kprime (keep everything).
 // fv[u] of element i = u * 32 + lane, live iff i < n.  hist: 256 counters of this warp in shared memory.
+template <int KPL>
 __device__ __forceinline__ void histogram_cut(const float (&fv)[KPL], int n, int lane, int kprime, uint32_t* hist,
                                               int (&bin)[KPL], int& cut_bin, int& kept, bool& reach_out) {
     float flo = CUDART_INF_F, fhi = -CUDART_INF_F;

@@ -43,14 +43,17 @@ constexpr int MAX_G = 128;           // widest PCA space of the tensor-core pass
 constexpr int PRODUCER_WARP = 12;    // highest warp ids on their schedulers: the arbiter favours them,
 constexpr int MMA_WARP = 13;         // so the single-thread producer / issuer are never starved
 constexpr int TMEM_WARP = 12;
-constexpr int KPL = 4;               // keys per lane.  Measured with 8 (256-key buffers, a quarter of the compactions):
-                                     // candidate kernel 3.78 -> 4.51 ms at 100 k x 100 k (staler thresholds, 2 KB per
-                                     // query in L2) and the final selection 0.17 -> 1.8 ms; it only pays for K' > 56
-                                     // (k = 60: 55 -> 7.4 ms)
-constexpr int CAP = 32 * KPL;        // candidate buffer entries per query
-static_assert(CAP == sel::CAP, "the fused re-rank (exact.cu) reads the candidate buffers with sel::CAP keys per query");
+// Candidate buffer entries per query: CAP_SMALL up to K' = MAX_KPRIME, CAP_LARGE above (see plan_k).  256-key buffers
+// compact a quarter as often, but measured at 100 k x 100 k, k = 30 the candidate kernel went 3.78 -> 4.51 ms
+// (staler thresholds, 2 KB per query in L2) and the final selection 0.17 -> 1.8 ms: they only pay for large K'
+// (k = 60: 55 -> 7.4 ms), so they serve only the k the 128-key plan cannot take.
+constexpr int CAP_SMALL = 128;
+constexpr int CAP_LARGE = 256;
+static_assert(CAP_SMALL == sel::CAP, "the fused re-rank (exact.cu) reads the candidate buffers with sel::CAP keys per query");
 constexpr int CHUNK = 32;           // columns per tcgen05.ld
-constexpr int MAX_KPRIME = 96;      // K' lists go to the re-rank, which takes at most 128 candidates per query
+constexpr int MAX_KPRIME = 96;      // K' of the 128-key plan (K' lists go to the re-rank, up to 128 per query with splits)
+constexpr int MAX_KPRIME_LARGE = 160;   // K' of the 256-key plan (unsplit: the re-rank takes up to 256 per query)
+constexpr int MAX_KSEL = 128;       // k + drop_first of the 256-key plan (the exact engine's limit)
 constexpr int SLEEP_NS = 2000;      // suspend-time hint of the producer's mbarrier waits
 // accumulators in TMEM (128 columns each): the NQ query tiles share four buffers in a fixed rotation
 // (job n = tile * NQ + q uses buffer n % 4), so the MMAs of a warpgroup's next tile run while it is still
@@ -147,6 +150,27 @@ inline SmemPlan plan_smem(int g) {
     p.bar_off = p.sort_off + (size_t)4 * p.nq * 256 * 4;     // per-warp histogram
     p.total = p.bar_off + bars;
     return p;
+}
+
+// The candidate-buffer plan of ksel = k + drop_first - the one place that decides it.  K' = ksel + max(ksel / 4, 8)
+// (the extra ranks are the certificate margin, see nabo_tc_kprime), capped by the plan:
+//   ksel + 8 <= MAX_KPRIME   128-key buffers, K' <= 96 (every k the pass took before the 256-key plan existed)
+//   89 <= ksel <= 128        256-key buffers, K' = 111 .. 160
+// ksel > 128 has no plan; workspace sizing still gets the 256-key one (supported() decides what runs).
+struct KPlan {
+    int cap;
+    int kprime;
+};
+inline int kprime_for(int ksel, int cap_kprime) {
+    const int kprime = ksel + (ksel / 4 > 8 ? ksel / 4 : 8);
+    return kprime < cap_kprime ? kprime : cap_kprime;
+}
+inline KPlan plan_k(int ksel) {
+    KPlan kp;
+    const bool small = ksel + 8 <= MAX_KPRIME;
+    kp.cap = small ? CAP_SMALL : CAP_LARGE;
+    kp.kprime = kprime_for(ksel, small ? MAX_KPRIME : MAX_KPRIME_LARGE);
+    return kp;
 }
 
 // ------------------------------------------------------------------ operand packing
@@ -312,7 +336,7 @@ struct Params {
                             // only without cuts and with n_split = 1)
     unsigned int* ticket;   // n_split = 1: CTA ticket counter, then one flag per item: its head is in global memory
                             // (zeroed before every launch)
-    unsigned long long* cand_buf;   // [work item][NQ*TILE][CAP]: every (query, reference range) owns CAP keys
+    unsigned long long* cand_buf;   // [work item][NQ*TILE][CAP]: every (query, reference range) owns CAP keys (plan_k)
     int* cand_cnt;          // [work item][NQ*TILE] live keys of each buffer when its sweep ended
     float* cand_tau;        // [work item][NQ*TILE] running threshold when its sweep ended
     int32_t* cand_idx;      // [n_query][n_split][kc_out]      (written by emit_kernel)
@@ -363,6 +387,7 @@ __device__ __forceinline__ unsigned long long globaltimer() {
 #endif
 
 // 32 freshly loaded scores of one query: reduce with FMNMX3 and append the ones below tau
+template <int CAP>
 __device__ __forceinline__ void filter_chunk(const uint32_t (&vr)[32], uint32_t col0, float tau,
                                              unsigned long long* mybuf, int& cnt TC_ARG) {
     float v[32];
@@ -447,9 +472,11 @@ __device__ __forceinline__ bool work_piece(const Params& p, const int (&sched)[4
 
 // KSTEPS: K steps of 16 known at compile time (0 = runtime loop); SPLIT: see work_piece; NQ: query tiles per work item;
 // SLAB: K steps per reference slab (0 = whole reference tiles).  The tile plan (plan_smem) picks NQ and SLAB.
-template <int KSTEPS, bool SPLIT, int NQ = 3, int SLAB = 0>
+// CAP: keys per candidate buffer (plan_k); the 256-key plan only runs unsplit.
+template <int KSTEPS, bool SPLIT, int NQ = 3, int SLAB = 0, int CAP = CAP_SMALL>
 __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p) {
     static_assert(NQ * 4 <= PRODUCER_WARP && (SLAB == 0 || KSTEPS == 0), "tile plan");
+    static_assert(CAP == CAP_SMALL || (CAP == CAP_LARGE && !SPLIT), "buffer plan");
     constexpr int N_EPI_WARPS = 4 * NQ;
     extern __shared__ __align__(1024) uint8_t smem[];
     Barriers* bars = reinterpret_cast<Barriers*>(smem + p.bar_off);
@@ -654,7 +681,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                         const int n = __shfl_sync(0xffffffffu, cnt, src);
                         int nc;
                         float nt;
-                        compact_select(gb, n, lane, p.kprime, p.soft - 8, hist, nc, nt);
+                        compact_select<CAP / 32>(gb, n, lane, p.kprime, p.soft - 8, hist, nc, nt);
                         if (lane == src) { cnt = nc; tau = nt; }
                         if (lane == 0) TC_STAT(4, 1);
                     }
@@ -673,7 +700,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
                         if (lane == 0) ptx::mbar_arrive(&bars->acc_empty[buf]);
                     }
                     TC_CLK(t_f);
-                    filter_chunk(vr, (uint32_t)(j * TILE + c * CHUNK), tau, mybuf, cnt TC_PASS);
+                    filter_chunk<CAP>(vr, (uint32_t)(j * TILE + c * CHUNK), tau, mybuf, cnt TC_PASS);
                     TC_CLK_ADD(6, t_f);
                     compact_over(c == TILE / CHUNK - 1 ? p.soft : CAP - CHUNK);
                 }
@@ -721,9 +748,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) candidates_kernel(const Params p)
 
 // Final selection: one warp per (query, reference range).  Sorts the buffer the sweep left behind, emits the K'
 // best reference rows and the threshold every other reference of the range is at or above.
-template <int NQ>
+template <int NQ, int CAP = CAP_SMALL>
 __global__ void __launch_bounds__(256)
 emit_kernel(const Params p) {
+    constexpr int KPL = CAP / 32;
     const int lane = threadIdx.x & 31;
     const long long wq = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);          // (buffer slot, query of the item)
     if (wq >= (long long)p.n_items * p.n_split * NQ * TILE) return;
@@ -739,7 +767,7 @@ emit_kernel(const Params p) {
     float nt;
     compact_sort_inline(p.cand_buf + (size_t)wq * CAP, n, lane, p.kprime, ks, kpl, nc, nt);
 #pragma unroll
-    for (int u = 0; u < 4; ++u) {                 // kc_out <= 128
+    for (int u = 0; u < KPL; ++u) {               // kc_out <= K' <= CAP
         const int i = u * 32 + lane;
         if (i < p.kc_out) {
             int32_t id = -1;
@@ -753,21 +781,18 @@ emit_kernel(const Params p) {
 }  // namespace tc
 
 // ------------------------------------------------------------------ host side
+static bool tc_plan_fits(int g) { return g >= 1 && g <= tc::MAX_G && tc::plan_smem(g).stages >= 2; }
+
 bool nabo_tc_supported(int g, int k, int drop_first) {
-    if (g < 1 || g > tc::MAX_G) return false;
-    const tc::SmemPlan pl = tc::plan_smem(g);
     const int ksel = k + (drop_first ? 1 : 0);
-    return pl.stages >= 2 && ksel + 8 <= tc::MAX_KPRIME;
+    return tc_plan_fits(g) && ksel <= tc::MAX_KSEL;
 }
 
 int nabo_tc_kprime(int k, int drop_first) {
-    const int ksel = k + (drop_first ? 1 : 0);
     // Extra ranks = certificate margin.  A row fails when ranks ksel..K' lie closer together than the
     // (provable, 2^-16) score error bound; measured at 100k x 100k / 200k x 1.25M, k = 30: +4 ranks ->
     // 76 / 944 uncertified rows, +6 -> 0 / 12, +8 -> 0 / 0, while the kernel time barely moves.
-    int kprime = ksel + (ksel / 4 > 8 ? ksel / 4 : 8);
-    if (kprime > tc::MAX_KPRIME) kprime = tc::MAX_KPRIME;
-    return kprime;
+    return tc::plan_k(k + (drop_first ? 1 : 0)).kprime;
 }
 
 static int tc_grid(int n_items) {
@@ -817,12 +842,14 @@ size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_fi
     const size_t tb = tc::tile_bytes(kp);
     const int nq = tc::plan_smem(g).nq;
     const int n_items = (n_query + nq * tc::TILE - 1) / (nq * tc::TILE);
-    const int kprime = nabo_tc_kprime(k, drop_first);
+    const tc::KPlan kpl = tc::plan_k(k + (drop_first ? 1 : 0));
+    const int kprime = kpl.kprime;
+    const int max_split = kpl.cap == tc::CAP_SMALL ? NABO_TC_MAX_SPLIT : 1;
     size_t b = 0;
     b += nabo_align_up((size_t)n_items * nq * tb, 256);          // packed queries
     if (with_ref) b += nabo_tc_ref_bytes(n_ref, g);                   // packed references, r norms, scale
     b += nabo_align_up((size_t)n_query * 8, 256) * 2;                 // q norms, qn2
-    b += nabo_align_up((size_t)n_items * NABO_TC_MAX_SPLIT * nq * tc::TILE * (tc::CAP * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
+    b += nabo_align_up((size_t)n_items * max_split * nq * tc::TILE * ((size_t)kpl.cap * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
     b += nabo_align_up((size_t)n_query * kprime * 4 * NABO_TC_MAX_SPLIT, 256);   // candidate indices (per reference range)
     b += nabo_align_up((size_t)n_query * 4 * NABO_TC_MAX_SPLIT, 256) + nabo_align_up((size_t)n_query * 4, 256);   // cert tau, fail rows
     b += nabo_align_up((size_t)(3 + n_items) * 4, 256);              // norm maxima, CTA ticket, head flags
@@ -892,8 +919,9 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     const int n_items = (n_query + pl.nq * tc::TILE - 1) / (pl.nq * tc::TILE);
     const int n_qtiles = n_items * pl.nq;
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
-    const int kprime = nabo_tc_kprime(k, drop_first);
-    if (n_split < 1 || n_split > NABO_TC_MAX_SPLIT) n_split = 1;
+    const tc::KPlan kpl = tc::plan_k(k + (drop_first ? 1 : 0));
+    const int kprime = kpl.kprime;
+    if (n_split < 1 || n_split > NABO_TC_MAX_SPLIT || kpl.cap != tc::CAP_SMALL) n_split = 1;   // 256 keys: unsplit only
     const int grid = tc_grid(n_items * n_split);
 
     __half* qa = (__half*)ar.take<char>((size_t)n_qtiles * tb);
@@ -902,7 +930,7 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     double* qn2 = ar.take<double>(n_query);
     double* rnorm = pre ? nullptr : ar.take<double>(n_ref);
     const size_t n_slots = (size_t)n_items * n_split * pl.nq * tc::TILE;
-    unsigned long long* cbuf = ar.take<unsigned long long>(n_slots * tc::CAP);
+    unsigned long long* cbuf = ar.take<unsigned long long>(n_slots * kpl.cap);
     int* ccnt = ar.take<int>(n_slots);
     float* ctau = ar.take<float>(n_slots);
     int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_split);
@@ -928,9 +956,12 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     p.stages = pl.stages; p.kprime = kprime; p.kc_out = kprime; p.n_split = n_split;
     p.cand_buf = cbuf; p.cand_cnt = ccnt; p.cand_tau = ctau; p.cand_idx = cand; p.cert_tau = tau; p.ticket = maxbits + 2;
     p.a_off = pl.a_off; p.b_off = pl.b_off; p.sort_off = pl.sort_off; p.bar_off = pl.bar_off;
-    p.soft = tc::CAP - tc::CHUNK - 16 > kprime ? tc::CAP - tc::CHUNK - 16 : kprime;
+    p.soft = kpl.cap - tc::CHUNK - 16 > kprime ? kpl.cap - tc::CHUNK - 16 : kprime;
     // Cut items at CTA boundaries only when the last wave would be partly filled and the packed reference fits in half of
-    // L2 (the other half holds the candidate buffers of the running items, 57 MB at g <= 52).  The cuts put the CTAs'
+    // L2 (the running items' candidate buffers take 57 MB at g <= 52 with 128 keys; with 256 keys they take 116 MB, 78 MB
+    // in the wide plan, and reference + buffers exceed L2 - yet the cuts still pay there: 100 k queries at k = 100,
+    // g = 50, candidate kernel 5.36 -> 4.80 ms against 100 k references (31 MB packed) and 7.68 -> 6.81 ms against 190 k
+    // (61 MB), B200 at a 1 000 W power limit, so both plans keep this rule).  The cuts put the CTAs'
     // sweeps out of step by up to an item.  Measured on a B200 (1 000 W power limit) at the two ends only: at 100 k x 100 k,
     // g = 50 (31 MB packed) the cuts take the candidate kernel from 3.62 to 3.25 ms; at 500 k x 2 M cosine, g = 50 (625 MB
     // packed) they took the kNN from 3.9e12 to 3.3e12 pairs/s (-18 %; the SM clock under the power cap fell from 1.52 to
@@ -950,16 +981,17 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
         tail->applies = tail_applies ? 1 : 0;
         tail->rows_full = overlap ? (n_items - rem_items) * pl.nq * tc::TILE : 0;
     }
-#define NABO_TC_LAUNCH1(KS, SPLIT, NQ, SLAB)                                                                       \
+#define NABO_TC_LAUNCH1(KS, SPLIT, NQ, SLAB, CAP)                                                                  \
     do {                                                                                                           \
-        NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, SPLIT, NQ, SLAB>,                                 \
+        NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, SPLIT, NQ, SLAB, CAP>,                            \
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.total));               \
-        tc::candidates_kernel<KS, SPLIT, NQ, SLAB><<<grid, tc::NTHREADS, pl.total, st>>>(p);                       \
+        tc::candidates_kernel<KS, SPLIT, NQ, SLAB, CAP><<<grid, tc::NTHREADS, pl.total, st>>>(p);                  \
     } while (0)
 #define NABO_TC_LAUNCH(KS, NQ, SLAB)                                                                               \
     do {                                                                                                           \
-        if (n_split > 1) NABO_TC_LAUNCH1(KS, true, NQ, SLAB);                                                      \
-        else NABO_TC_LAUNCH1(KS, false, NQ, SLAB);                                                                 \
+        if (kpl.cap == tc::CAP_LARGE) NABO_TC_LAUNCH1(KS, false, NQ, SLAB, tc::CAP_LARGE);                         \
+        else if (n_split > 1) NABO_TC_LAUNCH1(KS, true, NQ, SLAB, tc::CAP_SMALL);                                  \
+        else NABO_TC_LAUNCH1(KS, false, NQ, SLAB, tc::CAP_SMALL);                                                  \
     } while (0)
     if (pl.stages < 2) return nabo_set_error(NABO_EUNSUPPORTED, "knn: g=%d outside the tensor-core tile plans", g);
     if (pl.nq == 2) {                             // 53 <= g <= 128 (wide plan): slabs of 4 or 2 K steps
@@ -981,8 +1013,12 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
         return 0;
     }
     if (raw_out) raw_out->buf = nullptr;
-    if (pl.nq == 2) tc::emit_kernel<2><<<(unsigned)((n_slots + 7) / 8), 256, 0, st>>>(p);
-    else tc::emit_kernel<3><<<(unsigned)((n_slots + 7) / 8), 256, 0, st>>>(p);
+    const unsigned emit_blocks = (unsigned)((n_slots + 7) / 8);
+    if (kpl.cap == tc::CAP_LARGE) {
+        if (pl.nq == 2) tc::emit_kernel<2, tc::CAP_LARGE><<<emit_blocks, 256, 0, st>>>(p);
+        else tc::emit_kernel<3, tc::CAP_LARGE><<<emit_blocks, 256, 0, st>>>(p);
+    } else if (pl.nq == 2) tc::emit_kernel<2><<<emit_blocks, 256, 0, st>>>(p);
+    else tc::emit_kernel<3><<<emit_blocks, 256, 0, st>>>(p);
     NABO_LAUNCH_CHECK("emit_kernel");
     *launches += 1;
     if (n_split > 1) {
@@ -1014,7 +1050,14 @@ extern "C" int nabo_dbg_tc_sched_bounds(int n_items, int n_rtiles, int grid, int
 extern "C" double nabo_dbg_tc_sweep_cost(int x, int kprime) { return tc::sweep_cost(x, kprime); }
 
 // ------------------------------------------------------------------ public candidate-pass entry points
-extern "C" int nabo_knn_candidates_width(int k, int drop_first) { return nabo_tc_kprime(k, drop_first); }
+// The public candidate pass keeps the 128-key plan only (k + drop_first + 8 <= 96): its K' never exceeds 96.
+static bool candidates_supported(int g, int k, int drop_first) {
+    return tc_plan_fits(g) && k + (drop_first ? 1 : 0) + 8 <= tc::MAX_KPRIME;
+}
+
+extern "C" int nabo_knn_candidates_width(int k, int drop_first) {
+    return tc::kprime_for(k + (drop_first ? 1 : 0), tc::MAX_KPRIME);
+}
 
 extern "C" size_t nabo_knn_candidates_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first) {
     return nabo_tc_workspace_bytes(n_query, n_ref, g, k, drop_first);
@@ -1028,7 +1071,7 @@ extern "C" int nabo_knn_candidates(const double* q, int ldq, const double* r, in
     NABO_ARG(metric == NABO_EUCLIDEAN || metric == NABO_COSINE, "candidates: metric %d has no tensor-core pass", metric);
     NABO_ARG(n_query >= 1 && n_ref >= 1 && ldq >= g && ldr >= g, "candidates: bad sizes");
     NABO_ARG(q && r && out_cand && out_tau, "candidates: null pointer");
-    if (!nabo_tc_supported(g, k, drop_first))
+    if (!candidates_supported(g, k, drop_first))
         return nabo_set_error(NABO_EUNSUPPORTED, "candidates: g=%d k=%d outside the tensor-core tile plan", g, k);
     NaboArena ar(workspace, workspace_bytes);
     NaboStageTimer tm(false, st);
