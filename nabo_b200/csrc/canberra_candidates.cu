@@ -293,29 +293,39 @@ int nabo_cb_pretile_launch(const double* x, int ld, int n, int g, float* out, cu
     NABO_LAUNCH_CHECK("cb::pretile_kernel");
     return 0;
 }
-// extra workspace of the FP16 phase: half tiles of the reference + per-dimension max / scale
-size_t nabo_cb_extra_bytes(int n_ref, int g) {
-    return nabo_align_up(nabo_cb_pretile_floats(n_ref, g) * 2, 256) + 2 * nabo_align_up((size_t)g * 4, 256) + 512;
+
+void nabo_cb_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboCbWork* w) {
+    w->cand = ar.take<int32_t>((size_t)n_query * p.kprime);
+    w->tau = ar.take<float>(n_query);
+    w->qt = ar.take<float>(nabo_cb_pretile_floats(n_query, g));
+    w->rt = ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
+    w->rh = ar.take<char>(nabo_cb_pretile_floats(n_ref, g) * 2);      // FP16 tiles of the reference
+    w->maxbits = ar.take<unsigned>(g);                                // per-dimension maximum and scale
+    w->scale = ar.take<float>(g);
 }
 
-int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
-                       double f, const uint8_t* mask, int drop_first, float* qt, float* rt, void* extra, int32_t* cand,
-                       float* tau, cudaStream_t st) {
-    const int kprime = nabo_cb_kprime(k, drop_first);
-    NaboArena ar(extra, nabo_cb_extra_bytes(n_ref, g));
-    __half* rh = (__half*)ar.take<char>(nabo_cb_pretile_floats(n_ref, g) * 2);
-    unsigned* maxbits = ar.take<unsigned>(g);
-    float* scale = ar.take<float>(g);
-    if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the Canberra pass");
+// What either modified-Canberra pass hands to the re-rank: its score is a lower bound of the distance up to
+// nabo_cb_eps(g).
+void nabo_cb_result(const int32_t* cand, const float* tau, int n_cand, int g, int launches, NaboCandidates* out) {
+    out->cand = cand; out->n_cand = n_cand; out->raw.buf = nullptr; out->rows_full = 0; out->launches = launches;
+    out->cert.kind = NABO_CERT_LINEAR; out->cert.tau = tau; out->cert.qn2 = nullptr; out->cert.scal = nullptr;
+    out->cert.c_acc = nabo_cb_eps(g); out->cert.abs_slack = 0.0;
+}
+
+int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, double f,
+                       const uint8_t* mask, const NaboFastPlan& p, const NaboCbWork& w, cudaStream_t st,
+                       NaboCandidates* out) {
+    const int kprime = p.kprime;
+    __half* rh = (__half*)w.rh;
     {
         const size_t tq = nabo_cb_pretile_floats(n_query, g), tr = nabo_cb_pretile_floats(n_ref, g);
-        NABO_CUDA(cudaMemsetAsync(maxbits, 0, sizeof(unsigned) * g, st));
-        cb::dimmax_kernel<<<(unsigned)(((size_t)n_query * g + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, maxbits);
-        cb::dimmax_kernel<<<(unsigned)(((size_t)n_ref * g + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, maxbits);
-        cb::dimscale_kernel<<<(g + 63) / 64, 64, 0, st>>>(maxbits, g, scale);
-        cb::pretile_kernel<<<(unsigned)((tq + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, qt);
-        cb::pretile_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, rt);
-        cb::pretile_half_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, scale, rh);
+        NABO_CUDA(cudaMemsetAsync(w.maxbits, 0, sizeof(unsigned) * g, st));
+        cb::dimmax_kernel<<<(unsigned)(((size_t)n_query * g + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, w.maxbits);
+        cb::dimmax_kernel<<<(unsigned)(((size_t)n_ref * g + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, w.maxbits);
+        cb::dimscale_kernel<<<(g + 63) / 64, 64, 0, st>>>(w.maxbits, g, w.scale);
+        cb::pretile_kernel<<<(unsigned)((tq + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, w.qt);
+        cb::pretile_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, w.rt);
+        cb::pretile_half_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, w.scale, rh);
         NABO_LAUNCH_CHECK("cb::pretile kernels");
     }
     const size_t smem = cb::smem_bytes(g);
@@ -335,9 +345,10 @@ int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n
     const double fm0 = (1.0 + u) * (f + u * (2.0 + f)) / (1.0 - u);
     const float fm16 = (float)(fm0 * (1.0 + 1e-4));
     const float a16 = (float)((fm0 + 4.0) * eta);
-    cb::candidates_kernel<<<(n_query + cb::TQ - 1) / cb::TQ, cb::NT, smem, st>>>(qt, rt, rh, scale, n_query, n_ref, g, fm,
-                                                                              fm16, a16, mask, kprime, cand, tau);
+    cb::candidates_kernel<<<(n_query + cb::TQ - 1) / cb::TQ, cb::NT, smem, st>>>(w.qt, w.rt, rh, w.scale, n_query, n_ref, g,
+                                                                              fm, fm16, a16, mask, kprime, w.cand, w.tau);
     NABO_LAUNCH_CHECK("cb::candidates_kernel");
+    nabo_cb_result(w.cand, w.tau, kprime, g, 7, out);
     return 0;
 }
 

@@ -660,50 +660,51 @@ bool nabo_cbs_supported(int g, int k, int drop_first) {
     return cbs::plan_smem(g).stages >= 2 && ksel + 8 <= cbs::CAP - 64;
 }
 
-static int cbs_grid(int n_groups) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return n_groups < sms ? n_groups : sms;
+// CTAs of the sweep: whole query blocks, each cut into the plan's reference pieces (nabo_fast_plan keeps n_split at
+// most the SM count)
+static int cbs_grid(int n_query, int n_split) {
+    const int n_groups = (n_query + 31) / 32, sms = nabo_sm_count();
+    const int grid = n_groups * n_split < sms ? n_groups * n_split : sms;
+    return grid / n_split * n_split;
 }
 
-// planes + bin edges: the reference half of the extra workspace (and of a prepared reference's buffer)
-static size_t cbs_ref_extra_bytes(int n_ref, int g) {
-    const cbs::SmemPlan pl = cbs::plan_smem(g);
-    const size_t n_tiles = (n_ref + pl.rt - 1) / pl.rt;
-    return nabo_align_up(n_tiles * cbs::plane_tile_bytes(g, pl.rt), 256) +
-           nabo_align_up((size_t)g * (cbs::NBINS - 1) * 4, 256);
-}
-
-size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g, bool with_ref) {
-    const cbs::SmemPlan pl = cbs::plan_smem(g);
-    const size_t n_groups = (size_t)(n_query + 31) / 32;
-    const int nj = cbs::nblocks8(g) * 4;
-    size_t b = 0;
-    if (with_ref) b += cbs_ref_extra_bytes(n_ref, g);
-    b += nabo_align_up(n_groups * nj * 32 * 4, 256);
-    b += nabo_align_up(n_groups * g * 32 * 4, 256);
-    b += nabo_align_up((size_t)148 * pl.nw * 32 * cbs::CAP * 8, 256);
-    return b + 1024;
-}
-
-// rt: FP32 copy of the reference (nabo_cb_pretile_floats(n_ref, g) floats: [tile64][k][64], or [tile32][k][32] in
-// the wide plan), filled here.
 // Pieces the reference range is cut into (see the kernel): only when a CTA would have at most half of its warps
 // busy, never below 8 192 references per piece, and the union of the K' lists must fit the re-rank (128).
 int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first) {
     const cbs::SmemPlan pl = cbs::plan_smem(g);
     const int n_groups = (n_query + 31) / 32;
     const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
-    const int per_cta = (n_groups + cbs_grid(1 << 30) - 1) / cbs_grid(1 << 30);
+    const int sms = nabo_sm_count();
+    const int per_cta = (n_groups + sms - 1) / sms;
     int s = per_cta > 0 ? pl.nw / per_cta : 1;
     if (s > NABO_CBS_MAX_SPLIT) s = NABO_CBS_MAX_SPLIT;
     while (s > 1 && (n_tiles / s < 8192 / pl.rt || s * nabo_cb_kprime(k, drop_first) > 128)) --s;
     return s < 1 ? 1 : s;
 }
 
-// The reference half of the sliced pass: the FP32 copy rt (nabo_cb_pretile_floats(n_ref, g) floats), the bin edges
-// and the cumulative planes.  None of it depends on the queries or on dist_factor.
+// The reference half: FP32 copy (nabo_cb_pretile_floats(n_ref, g) floats: [tile64][k][64], or [tile32][k][32] in the
+// wide plan), cumulative planes, bin edges.  The regions of a prepared reference's buffer, and of a call without one.
+static void cbs_ref_carve(NaboArena& ar, int n_ref, int g, NaboCbsWork* w) {
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
+    const size_t n_tiles = (n_ref + pl.rt - 1) / pl.rt;
+    w->rt = ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
+    w->planes = (uint32_t*)ar.take<char>(n_tiles * cbs::plane_tile_bytes(g, pl.rt));
+    w->edges = ar.take<float>((size_t)g * (cbs::NBINS - 1));
+}
+
+void nabo_cbs_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboCbsWork* w) {
+    const cbs::SmemPlan pl = cbs::plan_smem(g);
+    const size_t n_groups = (size_t)(n_query + 31) / 32;
+    w->cand = ar.take<int32_t>((size_t)n_query * p.kprime * p.n_split);
+    w->tau = ar.take<float>((size_t)n_query * p.n_split);
+    w->rt = nullptr; w->planes = nullptr; w->edges = nullptr;
+    if (!p.prepared) cbs_ref_carve(ar, n_ref, g, w);
+    w->ctrl = ar.take<uint32_t>(n_groups * cbs::nblocks8(g) * 4 * 32);
+    w->qx = ar.take<float>(n_groups * g * 32);
+    w->cbuf = ar.take<unsigned long long>((size_t)cbs_grid(n_query, p.n_split) * pl.nw * 32 * cbs::CAP);
+}
+
+// The reference half of the sliced pass.  None of it depends on the queries or on dist_factor.
 static int cbs_ref_launch(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, float* rt, float* edges,
                           uint32_t* planes, cudaStream_t st) {
     const cbs::SmemPlan pl = cbs::plan_smem(g);
@@ -726,72 +727,61 @@ static int cbs_ref_launch(const double* r, int ldr, int n_ref, int g, const uint
 }
 
 size_t nabo_cbs_prepared_bytes(int n_ref, int g) {
-    return nabo_align_up(nabo_cb_pretile_floats(n_ref, g) * 4, 256) + cbs_ref_extra_bytes(n_ref, g);
+    NaboArena m = NaboArena::measure();
+    NaboCbsWork w;
+    cbs_ref_carve(m, n_ref, g, &w);
+    return m.off;
 }
 
 // A prepared reference's sliced operands, in the layout nabo_cbs_candidates builds per call.
 int nabo_cbs_prepare_ref(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, void* buffer, NaboCbsRef* out,
                          cudaStream_t st) {
-    const cbs::SmemPlan pl = cbs::plan_smem(g);
-    const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
     NaboArena ar(buffer, nabo_cbs_prepared_bytes(n_ref, g));
-    float* rt = ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
-    uint32_t* planes = (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g, pl.rt));
-    float* edges = ar.take<float>((size_t)g * (cbs::NBINS - 1));
+    NaboCbsWork w;
+    cbs_ref_carve(ar, n_ref, g, &w);
     if (!ar.ok) return nabo_set_error(NABO_EINVAL, "ref_prepare: buffer layout");
-    int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
+    int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, w.rt, w.edges, w.planes, st);
     if (rc) return rc;
     NABO_LAUNCH_CHECK("cbs reference preparation");
-    out->rt = rt;
-    out->planes = planes;
-    out->edges = edges;
+    out->rt = w.rt;
+    out->planes = w.planes;
+    out->edges = w.edges;
     return 0;
 }
 
-// cand: [n_query][n_split][K'], tau: [n_split][n_query].  pre != NULL: rt, planes and edges come from a prepared
-// reference (rt, r and mask are not read); extra then needs only the query half (nabo_cbs_extra_bytes(.., false)).
-int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
-                        double f, const uint8_t* mask, int drop_first, int n_split, float* rt, void* extra,
-                        size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st, const NaboCbsRef* pre) {
-    const int kprime = nabo_cb_kprime(k, drop_first);
-    if (n_split < 1 || n_split > NABO_CBS_MAX_SPLIT) n_split = 1;
+// cand: [n_query][n_split][K'], tau: [n_split][n_query], in the regions of nabo_cbs_carve.  pre != NULL: rt, planes
+// and edges come from a prepared reference (r and mask are not read).
+int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, double f,
+                        const uint8_t* mask, const NaboFastPlan& plan, const NaboCbsWork& w, cudaStream_t st,
+                        const NaboCbsRef* pre, NaboCandidates* out) {
+    const int kprime = plan.kprime, n_split = plan.n_split;
     const cbs::SmemPlan pl = cbs::plan_smem(g);
     const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
     const int n_yblk = (n_ref + pl.yw - 1) / pl.yw;
     const size_t n_groups = (size_t)(n_query + 31) / 32;
     const int nb = cbs::nblocks8(g), nj = nb * 4;
-    int grid = cbs_grid((int)n_groups * n_split);
-    if (n_split > 1) grid = grid / n_split * n_split;      // whole query blocks
-    if (grid < n_split) n_split = 1, grid = cbs_grid((int)n_groups);
+    const int grid = cbs_grid(n_query, n_split);
+    float* rt = pre ? (float*)pre->rt : w.rt;
+    uint32_t* planes = pre ? (uint32_t*)pre->planes : w.planes;
+    float* edges = pre ? (float*)pre->edges : w.edges;
 
-    NaboArena ar(extra, extra_bytes);
-    uint32_t* planes = pre ? (uint32_t*)pre->planes : (uint32_t*)ar.take<char>((size_t)n_tiles * cbs::plane_tile_bytes(g, pl.rt));
-    float* edges = pre ? (float*)pre->edges : ar.take<float>((size_t)g * (cbs::NBINS - 1));
-    uint32_t* ctrl = ar.take<uint32_t>(n_groups * nj * 32);
-    float* qx = ar.take<float>(n_groups * g * 32);
-    unsigned long long* cbuf = ar.take<unsigned long long>((size_t)grid * pl.nw * 32 * cbs::CAP);
-    if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the sliced Canberra pass");
-    if (pre) rt = (float*)pre->rt;
-
-    {
-        if (!pre) {
-            int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
-            if (rc) return rc;
-        }
-        const long long tc = (long long)n_groups * nj * 32;
-        cbs::ctrl_kernel<<<(unsigned)((tc + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, nj, f, edges, ctrl, tc);
-        const long long tq = (long long)n_groups * g * 32;
-        cbs::pretile32_kernel<<<(unsigned)((tq + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, qx, tq);
-        NABO_LAUNCH_CHECK("cbs preparation kernels");
+    if (!pre) {
+        int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
+        if (rc) return rc;
     }
+    const long long tc = (long long)n_groups * nj * 32;
+    cbs::ctrl_kernel<<<(unsigned)((tc + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, nj, f, edges, w.ctrl, tc);
+    const long long tq = (long long)n_groups * g * 32;
+    cbs::pretile32_kernel<<<(unsigned)((tq + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, w.qx, tq);
+    NABO_LAUNCH_CHECK("cbs preparation kernels");
 
     cbs::Params p;
-    p.planes = planes; p.rt = rt; p.qx = qx; p.ctrl = ctrl;
+    p.planes = planes; p.rt = rt; p.qx = w.qx; p.ctrl = w.ctrl;
     p.n_query = n_query; p.n_ref = n_ref; p.g = g; p.n_tiles = n_tiles; p.n_yblk = n_yblk;
     p.n_groups = (int)n_groups; p.kprime = kprime; p.stages = pl.stages; p.nj = nj; p.n_split = n_split;
     const double delta = fmax(1e-5, 4e-7 * (2.0 + f) / f);      // same optimistic margin as canberra_candidates.cu
     p.fm = (float)(f * (1.0 + delta));
-    p.cand_buf = cbuf; p.cand = cand; p.tau_out = tau;
+    p.cand_buf = w.cbuf; p.cand = w.cand; p.tau_out = w.tau;
     p.trig_extra = cbs::TRIG_EXTRA;
     p.stage_bytes = pl.stage_bytes; p.stage_off = pl.stage_off; p.xs_off = pl.xs_off; p.hist_off = pl.hist_off;
     p.work_off = pl.work_off; p.tau_off = pl.tau_off; p.cnt_off = pl.cnt_off; p.bar_off = pl.bar_off;
@@ -817,5 +807,6 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     }
 #undef NABO_CBS_LAUNCH
     NABO_LAUNCH_CHECK("cbs::sliced_kernel");
+    nabo_cb_result(w.cand, w.tau, kprime * n_split, g, 6, out);    // 6 launches reported, prepared or not
     return 0;
 }

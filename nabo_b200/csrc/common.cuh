@@ -40,12 +40,14 @@ int nabo_set_error(int code, const char* fmt, ...);
 
 static inline size_t nabo_align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-// Bump allocator over a caller-owned workspace.
+// Bump allocator over a caller-owned workspace.  A measuring arena (no memory) only counts: running a carve on it
+// and reading `off` gives the bytes the same carve takes from a real workspace.
 struct NaboArena {
     char* base;
     size_t off, cap;
     bool ok;
     NaboArena(void* p, size_t bytes) : base((char*)p), off(0), cap(bytes), ok(true) {}
+    static NaboArena measure() { return NaboArena(nullptr, 0); }
     template <typename T>
     T* take(size_t n) {
         off = nabo_align_up(off, 256);
@@ -145,6 +147,14 @@ __device__ __forceinline__ uint32_t float_to_sortable(float f) {
 __device__ __forceinline__ float sortable_to_float(uint32_t u) {
     uint32_t b = u ^ ((u >> 31) ? 0x80000000u : 0xFFFFFFFFu);
     return __uint_as_float(b);
+}
+
+// SMs of the current device; 148 (B200) when no device answers, so that the workspace-size functions run without one.
+static inline int nabo_sm_count() {
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
 }
 
 static inline int nabo_next_pow2(int x) {

@@ -513,71 +513,65 @@ fallback_merge_few_kernel(const NaboExactSplit sp, const int* __restrict__ row_i
     }
 }
 
-int nabo_exact_split_count(int ksel) {
-    int s = 2048 / ksel;
-    return s > 48 ? 48 : (s < 1 ? 1 : s);
+static void split_carve(NaboArena& ar, int nsplit, int f_max, int ksel, NaboExactSplit* sp) {
+    sp->mode = 1;
+    sp->nsplit = nsplit;
+    sp->f_max = f_max;
+    sp->f_min = 0;
+    sp->part_dist = ar.take<double>((size_t)nsplit * f_max * ksel);
+    sp->part_idx = ar.take<int32_t>((size_t)nsplit * f_max * ksel);
 }
-size_t nabo_exact_split_workspace(int ksel) {
-    (void)ksel;   // nsplit * ksel <= 2048 for every ksel: one bound, monotone in nothing; + the few-rows region
-    return (size_t)2048 * NABO_FALLBACK_SPLIT_ROWS * (sizeof(int32_t) + sizeof(double)) + 512 +
-           (size_t)NABO_FALLBACK_FEW_ENTRIES * NABO_FALLBACK_FEW_ROWS * (sizeof(int32_t) + sizeof(double)) + 512;
+
+void nabo_exact_split_carve(NaboArena& ar, int n_ref, int ksel, NaboExactSplit* split, NaboExactSplit* few) {
+    // (b) up to NABO_FALLBACK_SPLIT_ROWS rows: up to 48 pieces, one warp merges a row
+    const int s = 2048 / ksel;
+    split_carve(ar, s > 48 ? 48 : (s < 1 ? 1 : s), NABO_FALLBACK_SPLIT_ROWS, ksel, split);
+    few->nsplit = 0;
+    if (n_ref < NABO_FALLBACK_FEW_MIN_REF) return;
+    // (a) a handful of rows against a large reference: two pieces per SM, block-wide merge
+    const int sms2 = 2 * nabo_sm_count();
+    split_carve(ar, NABO_FALLBACK_FEW_ENTRIES / ksel < sms2 ? NABO_FALLBACK_FEW_ENTRIES / ksel : sms2,
+                NABO_FALLBACK_FEW_ROWS, ksel, few);
+    split->f_min = NABO_FALLBACK_FEW_ROWS;
 }
 
 // Exact engine on the rows listed in row_ids[0 .. *n_rows_dev): split over the reference when the rows
-// are few (one block would otherwise scan the whole reference alone), row-parallel otherwise.  Both
+// are few (one block would otherwise scan the whole reference alone), row-parallel otherwise.  All
 // variants are launched; each checks the device-side row count and exits at once if it is not its turn,
 // so no host synchronisation is needed.
 int nabo_knn_exact_fallback(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                             int metric, double f, const uint8_t* mask, int drop_first, int idx_offset,
-                            const int* row_ids, const int* n_rows_dev, void* split_ws, int32_t* out_idx,
-                            double* out_dist, const NaboRoute& route, cudaStream_t st) {
+                            const int* row_ids, const int* n_rows_dev, const NaboExactSplit& split,
+                            const NaboExactSplit& few, int32_t* out_idx, double* out_dist, const NaboRoute& route,
+                            cudaStream_t st) {
     const int ksel = k + (drop_first ? 1 : 0);
-    // (a) a handful of rows against a large reference: two pieces per SM, block-wide merge
-    const bool few = n_ref >= NABO_FALLBACK_FEW_MIN_REF;
-    if (few) {
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        NaboExactSplit sf;
-        sf.mode = 1;
-        sf.nsplit = NABO_FALLBACK_FEW_ENTRIES / ksel < 2 * sms ? NABO_FALLBACK_FEW_ENTRIES / ksel : 2 * sms;
-        sf.f_max = NABO_FALLBACK_FEW_ROWS;
-        sf.f_min = 0;
-        char* base = (char*)split_ws + (size_t)2048 * NABO_FALLBACK_SPLIT_ROWS * (sizeof(int32_t) + sizeof(double)) + 512;
-        sf.part_dist = (double*)base;
-        sf.part_idx = (int32_t*)(sf.part_dist + (size_t)sf.nsplit * sf.f_max * ksel);
+    if (few.nsplit > 0) {
         int rc0 = nabo_knn_exact_launch_ex(q, ldq, r, ldr, NABO_FALLBACK_FEW_ROWS, n_ref, g, ksel, metric, f, mask, 0, 0,
-                                           row_ids, n_rows_dev, sf, out_idx, out_dist, route, st);
+                                           row_ids, n_rows_dev, few, out_idx, out_dist, route, st);
         if (rc0) return rc0;
-        const int cappf = nabo_next_pow2(sf.nsplit * ksel);
+        const int cappf = nabo_next_pow2(few.nsplit * ksel);
         const size_t smf = (size_t)cappf * (sizeof(double) + sizeof(int));
         NABO_CUDA(cudaFuncSetAttribute(fallback_merge_few_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smf));
-        fallback_merge_few_kernel<<<NABO_FALLBACK_FEW_ROWS, 256, smf, st>>>(sf, row_ids, n_rows_dev, k, drop_first, idx_offset,
-                                                                         mask, cappf, out_idx, out_dist, route);
+        fallback_merge_few_kernel<<<NABO_FALLBACK_FEW_ROWS, 256, smf, st>>>(few, row_ids, n_rows_dev, k, drop_first,
+                                                                         idx_offset, mask, cappf, out_idx, out_dist,
+                                                                         route);
         NABO_LAUNCH_CHECK("fallback_merge_few_kernel");
     }
-    // (b) up to NABO_FALLBACK_SPLIT_ROWS rows: up to 48 pieces, one warp merges a row
-    NaboExactSplit sp;
-    sp.mode = 1;
-    sp.nsplit = nabo_exact_split_count(ksel);
-    sp.f_max = NABO_FALLBACK_SPLIT_ROWS;
-    sp.f_min = few ? NABO_FALLBACK_FEW_ROWS : 0;
-    sp.part_dist = (double*)split_ws;
-    sp.part_idx = (int32_t*)(sp.part_dist + (size_t)sp.nsplit * sp.f_max * ksel);
     int rc = nabo_knn_exact_launch_ex(q, ldq, r, ldr, NABO_FALLBACK_SPLIT_ROWS, n_ref, g, ksel, metric, f, mask, 0, 0,
-                                      row_ids, n_rows_dev, sp, out_idx, out_dist, route, st);
+                                      row_ids, n_rows_dev, split, out_idx, out_dist, route, st);
     if (rc) return rc;
-    int capp = nabo_next_pow2(sp.nsplit * ksel);
+    int capp = nabo_next_pow2(split.nsplit * ksel);
     if (capp < 32) capp = 32;
     const size_t smem = (size_t)4 * capp * (sizeof(double) + sizeof(int));
     NABO_CUDA(cudaFuncSetAttribute(fallback_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fallback_merge_kernel<<<(NABO_FALLBACK_SPLIT_ROWS + 3) / 4, 128, smem, st>>>(sp, row_ids, n_rows_dev, k, drop_first,
+    fallback_merge_kernel<<<(NABO_FALLBACK_SPLIT_ROWS + 3) / 4, 128, smem, st>>>(split, row_ids, n_rows_dev, k, drop_first,
                                                                                idx_offset, mask, capp, out_idx, out_dist,
                                                                                route);
     NABO_LAUNCH_CHECK("fallback_merge_kernel");
-    sp.mode = 2;
+    NaboExactSplit rest = split;
+    rest.mode = 2;
     return nabo_knn_exact_launch_ex(q, ldq, r, ldr, n_query, n_ref, g, k, metric, f, mask, drop_first, idx_offset,
-                                    row_ids, n_rows_dev, sp, out_idx, out_dist, route, st);
+                                    row_ids, n_rows_dev, rest, out_idx, out_dist, route, st);
 }
 
 int nabo_knn_exact_launch(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,
@@ -588,6 +582,24 @@ int nabo_knn_exact_launch(const double* q, int ldq, const double* r, int ldr, in
     sp.mode = 0; sp.nsplit = 1; sp.f_max = 0; sp.f_min = 0; sp.part_idx = nullptr; sp.part_dist = nullptr;
     return nabo_knn_exact_launch_ex(q, ldq, r, ldr, n_query, n_ref, g, k, metric, f, mask, drop_first, idx_offset,
                                     row_ids, n_rows_dev, sp, out_idx, out_dist, route, st);
+}
+
+int nabo_knn_exact_call(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
+                        int metric, double f, const uint8_t* mask, int drop_first, int idx_offset, int32_t* out_idx,
+                        double* out_dist, const NaboRoute& route, int64_t* stats_host, cudaStream_t st) {
+    NaboStageTimer tm(stats_host != nullptr, st);
+    tm.begin();
+    int rc = nabo_knn_exact_launch(q, ldq, r, ldr, n_query, n_ref, g, k, metric, f, mask, drop_first, idx_offset,
+                                   nullptr, nullptr, out_idx, out_dist, route, st);
+    tm.end(0);
+    if (rc) return rc;
+    if (stats_host) {
+        NABO_CUDA(cudaStreamSynchronize(st));
+        stats_host[1] = n_query;
+        stats_host[3] = 1;
+        stats_host[4] = tm.ns(0);
+    }
+    return 0;
 }
 
 int nabo_knn_exact_launch_ex(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,

@@ -7,7 +7,7 @@
 
 extern "C" size_t nabo_knn_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, int mode) {
     if (mode == NABO_MODE_EXACT) return 256;
-    return nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric);
+    return nabo_fast_workspace_bytes(n_query, n_ref, g, k, metric, false, 0.0);
 }
 
 static int knn_impl(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
@@ -69,21 +69,9 @@ static int knn_impl(const double* q, int ldq, const double* r, int ldr, int n_qu
     if (n_query == 0) return 0;
     NABO_ARG(q && r && (route.n_parts > 0 || (out_idx && out_dist)), "knn: null pointer");
     if (stats_host) for (int i = 0; i < 8; ++i) stats_host[i] = 0;
-    if (mode == NABO_MODE_EXACT) {
-        NaboStageTimer tm(stats_host != nullptr, st);
-        tm.begin();
-        int rc = nabo_knn_exact_launch(q, ldq, r, ldr, n_query, n_ref, g, k, metric, dist_factor, ref_mask,
-                                       drop_first, idx_offset, nullptr, nullptr, out_idx, out_dist, route, st);
-        tm.end(0);
-        if (rc) return rc;
-        if (stats_host) {
-            NABO_CUDA(cudaStreamSynchronize(st));
-            stats_host[1] = n_query;
-            stats_host[3] = 1;
-            stats_host[4] = tm.ns(0);
-        }
-        return 0;
-    }
+    if (mode == NABO_MODE_EXACT)
+        return nabo_knn_exact_call(q, ldq, r, ldr, n_query, n_ref, g, k, metric, dist_factor, ref_mask, drop_first,
+                                   idx_offset, out_idx, out_dist, route, stats_host, st);
     NABO_ARG(mode == NABO_MODE_FAST, "knn: unknown mode %d", mode);
     return nabo_knn_fast(q, ldq, r, ldr, n_query, n_ref, g, k, metric, dist_factor, ref_mask, drop_first,
                          idx_offset, out_idx, out_dist, route, workspace, workspace_bytes, stats_host, st, pre);
@@ -92,17 +80,12 @@ static int knn_impl(const double* q, int ldq, const double* r, int ldr, int n_qu
 // ------------------------------------------------------------------ prepared reference
 // Buffer layout: the reference half of the fast engine's operands for the metric (tc_candidates.cu /
 // canberra_sliced.cu own the layout inside), at offset 0.  The descriptor keeps the device addresses.
+// The plan is the pass the fast engine takes for the metric at k = 1 against a large reference: the tensor-core or the
+// sliced pass, whose operands then serve every call that takes the same pass.
 static bool prepared_plan(int g, int metric, int* plan) {
-    if (g < 1 || g > 128) return false;
-    if (metric == NABO_EUCLIDEAN || metric == NABO_COSINE) {
-        *plan = NABO_PLAN_TC;
-        return nabo_tc_supported(g, 1, 0);
-    }
-    if (metric == NABO_MOD_CANBERRA) {
-        *plan = NABO_PLAN_SLICED;
-        return nabo_cbs_supported(g, 1, 0);
-    }
-    return false;
+    const int path = nabo_fast_plan(1, 1 << 30, g, 1, metric, 1.0, 0, true).path;
+    *plan = path == NABO_PATH_TC ? NABO_PLAN_TC : NABO_PLAN_SLICED;
+    return path == NABO_PATH_TC || path == NABO_PATH_SLICED;
 }
 
 extern "C" size_t nabo_ref_prepared_bytes(int n_ref, int g, int metric) {
@@ -183,8 +166,8 @@ extern "C" size_t nabo_knn_prepared_workspace_bytes(int n_query, const nabo_prep
     NaboFastRef ops;
     if (check_prepared(prepared_host, &ops) != 0) return 0;
     if (mode == NABO_MODE_EXACT) return 256;
-    return nabo_fast_prepared_workspace_bytes(n_query, prepared_host->n_ref, prepared_host->g, k, prepared_host->metric,
-                                              dist_factor);
+    return nabo_fast_workspace_bytes(n_query, prepared_host->n_ref, prepared_host->g, k, prepared_host->metric, true,
+                                     dist_factor);
 }
 
 static int knn_prepared_impl(const double* q, int ldq, int n_query, const nabo_prepared_ref* pr, int k,

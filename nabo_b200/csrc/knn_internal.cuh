@@ -43,21 +43,27 @@ struct NaboExactSplit {
     int32_t* part_idx;   // [nsplit][f_max][ksel]
     double* part_dist;
 };
-int nabo_exact_split_count(int ksel);
-size_t nabo_exact_split_workspace(int ksel);
 int nabo_knn_exact_launch_ex(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,
                              int k, int metric, double f, const uint8_t* mask, int drop_first, int idx_offset,
                              const int* row_ids, const int* n_rows_dev, const NaboExactSplit& sp, int32_t* out_idx,
                              double* out_dist, const NaboRoute& route, cudaStream_t st);
+// Partial-list regions of the split fallback: the split pass and, against n_ref >= NABO_FALLBACK_FEW_MIN_REF, the
+// few-rows pass (few->nsplit = 0 otherwise).
+void nabo_exact_split_carve(NaboArena& ar, int n_ref, int ksel, NaboExactSplit* split, NaboExactSplit* few);
 int nabo_knn_exact_fallback(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                             int metric, double f, const uint8_t* mask, int drop_first, int idx_offset,
-                            const int* row_ids, const int* n_rows_dev, void* split_ws, int32_t* out_idx,
-                            double* out_dist, const NaboRoute& route, cudaStream_t st);
+                            const int* row_ids, const int* n_rows_dev, const NaboExactSplit& split,
+                            const NaboExactSplit& few, int32_t* out_idx, double* out_dist, const NaboRoute& route,
+                            cudaStream_t st);
 
 int nabo_knn_exact_launch(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,
                           int k, int metric, double f, const uint8_t* mask, int drop_first, int idx_offset,
                           const int* row_ids, const int* n_rows_dev, int32_t* out_idx, double* out_dist,
                           const NaboRoute& route, cudaStream_t st);
+// The exact engine on every row with its stats (one launch, all of it timed as the candidate stage).
+int nabo_knn_exact_call(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
+                        int metric, double f, const uint8_t* mask, int drop_first, int idx_offset, int32_t* out_idx,
+                        double* out_dist, const NaboRoute& route, int64_t* stats_host, cudaStream_t st);
 
 // Candidate certificate evaluated by the re-rank (see rerank_kernel).
 #define NABO_CERT_NONE 0
@@ -84,56 +90,91 @@ struct NaboCandBuf {
     int kprime;
 };
 // row0: the launch covers the queries [row0, n_query) (all pointers are those of row 0); dependent: launched with
-// programmatic stream serialisation behind a kernel that signals (NaboTailSplit)
+// programmatic stream serialisation behind a kernel that signals (NaboCandidates::rows_full)
 int nabo_rerank_launch(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                        int metric, double f, const uint8_t* mask, int drop_first, int idx_offset,
                        const int32_t* cand, int n_cand, const NaboCert& cert, int* fail_rows, int* fail_count,
                        int32_t* out_idx, double* out_dist, const NaboRoute& route, cudaStream_t st,
                        const NaboCandBuf* from_buf = nullptr, int row0 = 0, bool dependent = false);
 
-// Partly filled last wave of the persistent candidate kernel (tc_candidates.cu; only where it does not cut items at
-// CTA boundaries, i.e. packed references larger than half of L2): every CTA executes
-// griddepcontrol.launch_dependents once its full-wave items are done, so a kernel launched right behind it on the same
-// stream with programmatic stream serialisation - the re-rank of the first rows_full queries - runs while the last wave is
-// still busy, on the SMs that wave leaves idle.  rows_full = 0: nothing to overlap.  When rows_full > 0 the candidate pass
-// has NOT closed its timing stage: the caller does, after the dependent launch.
-struct NaboTailSplit {
-    int dry;                   // in: 1 = only report (the per-stage timing pass measures the candidate kernel alone)
-    int rows_full;             // out: queries the dependent launch may take (0 with dry)
-    int applies;               // out: 1 when the shape qualifies (with or without dry)
+// Which pass of the fast engine serves a call, and its parameters (nabo_fast_plan, fast.cu).  The passes, the
+// workspace carves and the workspace-size functions all take these values from the plan and change none of them.
+#define NABO_PATH_EXACT 0        // the exact engine on every row
+#define NABO_PATH_TC 1           // tensor-core candidate pass (Euclidean / cosine)
+#define NABO_PATH_SLICED 2       // bit-sliced modified-Canberra pass
+#define NABO_PATH_TWO_PHASE 3    // FP16 / FP32 two-phase modified-Canberra pass
+struct NaboFastPlan {
+    int path;
+    int kprime;       // K': candidates per list
+    int cap;          // tensor core: keys per candidate buffer (128 or 256)
+    int n_split;      // reference pieces, each with its own K' list and threshold per query
+    bool fused;       // tensor core: the re-rank makes the final K' selection from the raw buffers (no emit kernel)
+    bool prepared;    // a prepared reference's operands replace the reference half of the pass
+};
+NaboFastPlan nabo_fast_plan(int n_query, int n_ref, int g, int k, int metric, double f, int drop_first, bool pre);
+
+// What a candidate pass hands to the fast engine's re-rank.
+struct NaboCandidates {
+    const int32_t* cand;       // [n_query][n_cand] candidate lists (K' per reference piece)
+    int n_cand;
+    NaboCert cert;             // cert.tau: [n_split][n_query] thresholds; the engine reduces them to row 0 when split
+    NaboCandBuf raw;           // fused path: raw.buf != NULL, the re-rank selects from the candidate buffers
+    // Partly filled last wave of the persistent tensor-core kernel (only where it does not cut items at CTA
+    // boundaries, i.e. packed references larger than half of L2): every CTA executes griddepcontrol.launch_dependents
+    // once its full-wave items are done, so the re-rank of the first rows_full queries, launched right behind it with
+    // programmatic stream serialisation, runs while the last wave is still busy, on the SMs that wave leaves idle.
+    // 0: nothing to overlap.  When rows_full > 0 the pass has NOT closed the candidate stage of the timer.
+    int rows_full;
+    int launches;              // kernels the pass reports in stats_host[3]
 };
 
-// Reference half of the tensor-core operands, built once by nabo_tc_prepare_ref (prepared reference, prepared.cu):
+// Reference half of the tensor-core operands, built once by nabo_tc_prepare_ref (prepared reference, knn.cu):
 // the packed tiles in the layout the one-shot path writes, and the scale {sc, 1/sc, max scaled reference norm, cosine}.
 struct NaboTcRef {
     const void* rb;
     const double* scal;
 };
 
+// Each pass takes its regions with one carve function; the size functions run the same carve on a measuring arena.
+// With a prepared reference (plan.prepared) the reference half is not carved and those pointers stay NULL.
 struct NaboStageTimer;
 bool nabo_tc_supported(int g, int k, int drop_first);
-int nabo_tc_kprime(int k, int drop_first);
-size_t nabo_tc_ref_bytes(int n_ref, int g);
-size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first, bool with_ref = true);
+int nabo_tc_kprime(int k, int drop_first, int* cap = nullptr);    // cap: keys per candidate buffer of the plan
+int nabo_tc_split(int n_query, int n_ref, int g);
+#define NABO_TC_MAX_SPLIT 3
+struct NaboTcWork {
+    void *qa, *rb;                 // packed query and reference tiles
+    double *qnorm, *qn2, *rnorm, *scal;
+    unsigned long long* cbuf;      // per query slot and reference piece: cap keys, live count (ccnt), threshold (ctau)
+    int* ccnt;
+    float *ctau, *tau;             // tau: [n_split][n_query]
+    int32_t* cand;                 // [n_query][n_split][K']
+    unsigned int* maxbits;         // 2 norm maxima, CTA ticket, head flags
+};
+void nabo_tc_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboTcWork* w);
 size_t nabo_tc_prepared_bytes(int n_ref, int g);
 int nabo_tc_prepare_ref(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* mask, void* buffer,
                         NaboTcRef* out, cudaStream_t st);
-#define NABO_TC_MAX_SPLIT 3
-int nabo_tc_split(int n_query, int n_ref, int g);
-int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
-                       int metric, const uint8_t* mask, int drop_first, int* n_split_io, NaboArena& ar, int32_t** cand_idx_out,
-                       int* kprime_out, float** cert_tau_out, double** qn2_out, double** scal_out, int* launches,
-                       NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out = nullptr, NaboTailSplit* tail = nullptr,
-                       const NaboTcRef* pre = nullptr);
+// timed: the caller times the stages, so the candidate kernel runs alone (rows_full = 0)
+int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int metric,
+                       const uint8_t* mask, const NaboFastPlan& p, const NaboTcWork& w, bool timed, NaboStageTimer& tm,
+                       cudaStream_t st, const NaboTcRef* pre, NaboCandidates* out);
 
 bool nabo_cb_supported(int g, int k, int drop_first);
 int nabo_cb_kprime(int k, int drop_first);
 double nabo_cb_eps(int g);
 size_t nabo_cb_pretile_floats(int n, int g);
-size_t nabo_cb_extra_bytes(int n_ref, int g);
-int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
-                       double f, const uint8_t* mask, int drop_first, float* qt, float* rt, void* extra, int32_t* cand,
-                       float* tau, cudaStream_t st);
+struct NaboCbWork {
+    int32_t* cand;                 // [n_query][K']
+    float *tau, *qt, *rt, *scale;  // tau: [n_query]; FP32 tiles; per-dimension scale (of the maxima in maxbits)
+    void* rh;                      // FP16 reference tiles
+    unsigned* maxbits;
+};
+void nabo_cb_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboCbWork* w);
+int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, double f,
+                       const uint8_t* mask, const NaboFastPlan& p, const NaboCbWork& w, cudaStream_t st,
+                       NaboCandidates* out);
+void nabo_cb_result(const int32_t* cand, const float* tau, int n_cand, int g, int launches, NaboCandidates* out);
 
 int nabo_cb_pretile_launch(const double* x, int ld, int n, int g, float* out, cudaStream_t st);
 // bit-sliced Canberra pass (canberra_sliced.cu); same outputs as nabo_cb_candidates
@@ -144,27 +185,33 @@ struct NaboCbsRef {
     const float* edges;
 };
 bool nabo_cbs_supported(int g, int k, int drop_first);
-size_t nabo_cbs_extra_bytes(int n_query, int n_ref, int g, bool with_ref = true);
+int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first);
+#define NABO_CBS_MAX_SPLIT 3
+struct NaboCbsWork {
+    int32_t* cand;                 // [n_query][n_split][K']
+    float *tau, *rt, *edges, *qx;  // tau: [n_split][n_query]; reference FP32 copy and bin edges; queries' FP32 copy
+    uint32_t *planes, *ctrl;       // reference bit planes; queries' bin controls
+    unsigned long long* cbuf;      // per warp of the grid: CAP keys
+};
+void nabo_cbs_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboCbsWork* w);
 size_t nabo_cbs_prepared_bytes(int n_ref, int g);
 int nabo_cbs_prepare_ref(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, void* buffer, NaboCbsRef* out,
                          cudaStream_t st);
-#define NABO_CBS_MAX_SPLIT 3
-int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first);
-int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
-                        double f, const uint8_t* mask, int drop_first, int n_split, float* rt, void* extra,
-                        size_t extra_bytes, int32_t* cand, float* tau, cudaStream_t st, const NaboCbsRef* pre = nullptr);
+int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, double f,
+                        const uint8_t* mask, const NaboFastPlan& p, const NaboCbsWork& w, cudaStream_t st,
+                        const NaboCbsRef* pre, NaboCandidates* out);
 int nabo_tau_min_launch(float* tau, int n_query, int n_split, cudaStream_t st);
 
-// Reference-side operands of a prepared reference (prepared.cu): the tensor-core tiles (Euclidean / cosine) or the
+// Reference-side operands of a prepared reference (knn.cu): the tensor-core tiles (Euclidean / cosine) or the
 // sliced-pass state (modified Canberra); the pointers of the other engine are NULL.
 struct NaboFastRef {
     NaboTcRef tc;
     NaboCbsRef cbs;
 };
-size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric);
-// per-call workspace of nabo_knn_fast with a prepared reference (smaller by the reference's share wherever the
-// prepared operands are used for every drop_first; the full size otherwise)
-size_t nabo_fast_prepared_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, double f);
+// Workspace of nabo_knn_fast, the largest carve over drop_first: pre = false for the one-shot call (which has no
+// dist_factor: for modified Canberra both passes; f is not read), true for a prepared reference with dist_factor f
+// (the one-shot carve wherever its operands do not serve the call).
+size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, bool pre, double f);
 int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                   int metric, double f, const uint8_t* mask, int drop_first, int idx_offset, int32_t* out_idx,
                   double* out_dist, const NaboRoute& route, void* workspace, size_t workspace_bytes,

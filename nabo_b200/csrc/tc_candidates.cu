@@ -788,18 +788,13 @@ bool nabo_tc_supported(int g, int k, int drop_first) {
     return tc_plan_fits(g) && ksel <= tc::MAX_KSEL;
 }
 
-int nabo_tc_kprime(int k, int drop_first) {
+int nabo_tc_kprime(int k, int drop_first, int* cap) {
     // Extra ranks = certificate margin.  A row fails when ranks ksel..K' lie closer together than the
     // (provable, 2^-16) score error bound; measured at 100k x 100k / 200k x 1.25M, k = 30: +4 ranks ->
     // 76 / 944 uncertified rows, +6 -> 0 / 12, +8 -> 0 / 0, while the kernel time barely moves.
-    return tc::plan_k(k + (drop_first ? 1 : 0)).kprime;
-}
-
-static int tc_grid(int n_items) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return n_items < sms ? n_items : sms;
+    const tc::KPlan kpl = tc::plan_k(k + (drop_first ? 1 : 0));
+    if (cap) *cap = kpl.cap;
+    return kpl.kprime;
 }
 
 static size_t l2_bytes() {
@@ -817,7 +812,7 @@ int nabo_tc_split(int n_query, int n_ref, int g) {
     const int nq = tc::plan_smem(g).nq;
     const int n_items = (n_query + nq * tc::TILE - 1) / (nq * tc::TILE);
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
-    int s = n_items > 0 ? tc_grid(1 << 30) / n_items : 1;
+    int s = n_items > 0 ? nabo_sm_count() / n_items : 1;
     if (s > NABO_TC_MAX_SPLIT) s = NABO_TC_MAX_SPLIT;
     while (s > 1 && n_rtiles / s < 32) --s;              // keep >= 4096 references per piece
     return s < 1 ? 1 : s;
@@ -837,36 +832,28 @@ int nabo_tau_min_launch(float* tau, int n_query, int n_split, cudaStream_t st) {
     return 0;
 }
 
-size_t nabo_tc_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first, bool with_ref) {
-    const int kp = tc::kp_for(g);
-    const size_t tb = tc::tile_bytes(kp);
-    const int nq = tc::plan_smem(g).nq;
-    const int n_items = (n_query + nq * tc::TILE - 1) / (nq * tc::TILE);
-    const tc::KPlan kpl = tc::plan_k(k + (drop_first ? 1 : 0));
-    const int kprime = kpl.kprime;
-    const int max_split = kpl.cap == tc::CAP_SMALL ? NABO_TC_MAX_SPLIT : 1;
-    size_t b = 0;
-    b += nabo_align_up((size_t)n_items * nq * tb, 256);          // packed queries
-    if (with_ref) b += nabo_tc_ref_bytes(n_ref, g);                   // packed references, r norms, scale
-    b += nabo_align_up((size_t)n_query * 8, 256) * 2;                 // q norms, qn2
-    b += nabo_align_up((size_t)n_items * max_split * nq * tc::TILE * ((size_t)kpl.cap * 8 + 8), 256) + 512;   // candidate buffers, counts, thresholds
-    b += nabo_align_up((size_t)n_query * kprime * 4 * NABO_TC_MAX_SPLIT, 256);   // candidate indices (per reference range)
-    b += nabo_align_up((size_t)n_query * 4 * NABO_TC_MAX_SPLIT, 256) + nabo_align_up((size_t)n_query * 4, 256);   // cert tau, fail rows
-    b += nabo_align_up((size_t)(3 + n_items) * 4, 256);              // norm maxima, CTA ticket, head flags
-    b += 4096;
-    return b;
+void nabo_tc_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboTcWork* w) {
+    const tc::SmemPlan pl = tc::plan_smem(g);
+    const int n_items = (n_query + pl.nq * tc::TILE - 1) / (pl.nq * tc::TILE);
+    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
+    const size_t tb = tc::tile_bytes(tc::kp_for(g));
+    const size_t n_slots = (size_t)n_items * p.n_split * pl.nq * tc::TILE;
+    w->rb = nullptr; w->rnorm = nullptr; w->scal = nullptr;
+    w->qa = ar.take<char>((size_t)n_items * pl.nq * tb);
+    if (!p.prepared) w->rb = ar.take<char>((size_t)n_rtiles * tb);
+    w->qnorm = ar.take<double>(n_query);
+    w->qn2 = ar.take<double>(n_query);
+    if (!p.prepared) w->rnorm = ar.take<double>(n_ref);
+    w->cbuf = ar.take<unsigned long long>(n_slots * p.cap);
+    w->ccnt = ar.take<int>(n_slots);
+    w->ctau = ar.take<float>(n_slots);
+    w->cand = ar.take<int32_t>((size_t)n_query * p.kprime * p.n_split);
+    w->tau = ar.take<float>((size_t)n_query * p.n_split);
+    if (!p.prepared) w->scal = ar.take<double>(4);
+    w->maxbits = ar.take<unsigned int>(3 + (size_t)n_items);
 }
 
 // ------------------------------------------------------------------ reference half of the operands
-// Packed reference tiles and their norms: what the workspace holds for one call, and the first part of a prepared
-// reference's buffer (which adds the scale and the norm maximum, kTcRefTail bytes).
-size_t nabo_tc_ref_bytes(int n_ref, int g) {
-    const size_t tb = tc::tile_bytes(tc::kp_for(g));
-    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
-    return nabo_align_up((size_t)n_rtiles * tb, 256) + nabo_align_up((size_t)n_ref * 8, 256);
-}
-static const size_t kTcRefTail = 512;      // scal[4] and the reference's norm maximum, 256-aligned pieces each
-
 static void tc_ref_norms(const double* r, int ldr, int n_ref, int g, double* rnorm, unsigned int* maxr_bits, cudaStream_t st) {
     tc::norms_kernel<<<(n_ref + 255) / 256, 256, 0, st>>>(r, ldr, n_ref, g, rnorm, maxr_bits);
 }
@@ -878,75 +865,75 @@ static void tc_ref_pack(const double* r, int ldr, int n_ref, int g, const double
                                                                           rb, nullptr);
 }
 
-size_t nabo_tc_prepared_bytes(int n_ref, int g) { return nabo_tc_ref_bytes(n_ref, g) + kTcRefTail; }
+// A prepared reference's buffer: the reference half of a call's regions (tiles, norms, scale), then the reference's
+// norm maximum.
+static unsigned int* tc_prepared_carve(NaboArena& ar, int n_ref, int g, NaboTcWork* w) {
+    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
+    w->rb = ar.take<char>((size_t)n_rtiles * tc::tile_bytes(tc::kp_for(g)));
+    w->rnorm = ar.take<double>(n_ref);
+    w->scal = ar.take<double>(4);
+    return ar.take<unsigned int>(1);
+}
+
+size_t nabo_tc_prepared_bytes(int n_ref, int g) {
+    NaboArena m = NaboArena::measure();
+    NaboTcWork w;
+    tc_prepared_carve(m, n_ref, g, &w);
+    return m.off;
+}
 
 // A prepared reference's operands: the same norms and packing as a one-shot call, but the scale comes from the
 // reference's largest norm alone (cosine: 32), so that any later query batch can use the tiles.
 int nabo_tc_prepare_ref(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* mask, void* buffer,
                         NaboTcRef* out, cudaStream_t st) {
-    const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
     NaboArena ar(buffer, nabo_tc_prepared_bytes(n_ref, g));
-    __half* rb = (__half*)ar.take<char>((size_t)n_rtiles * tc::tile_bytes(tc::kp_for(g)));
-    double* rnorm = ar.take<double>(n_ref);
-    double* scal = ar.take<double>(4);
-    unsigned int* maxr = ar.take<unsigned int>(1);
+    NaboTcWork w;
+    unsigned int* maxr = tc_prepared_carve(ar, n_ref, g, &w);
     if (!ar.ok) return nabo_set_error(NABO_EINVAL, "ref_prepare: buffer layout");
     NABO_CUDA(cudaMemsetAsync(maxr, 0, sizeof(unsigned int), st));
-    tc_ref_norms(r, ldr, n_ref, g, rnorm, maxr, st);
-    tc::scale_kernel<<<1, 1, 0, st>>>(maxr, maxr, metric == NABO_COSINE ? 1 : 0, scal);
-    tc_ref_pack(r, ldr, n_ref, g, rnorm, scal, mask, rb, st);
+    tc_ref_norms(r, ldr, n_ref, g, w.rnorm, maxr, st);
+    tc::scale_kernel<<<1, 1, 0, st>>>(maxr, maxr, metric == NABO_COSINE ? 1 : 0, w.scal);
+    tc_ref_pack(r, ldr, n_ref, g, w.rnorm, w.scal, mask, (__half*)w.rb, st);
     NABO_LAUNCH_CHECK("tc reference preparation");
-    out->rb = rb;
-    out->scal = scal;
+    out->rb = w.rb;
+    out->scal = w.scal;
     return 0;
 }
 
-// Runs norms -> scale -> pack -> candidate kernel.  Outputs (device, inside the arena):
-// cand_idx [n_query][kprime], cert_tau [n_query], qn2 [n_query], scal[4].  pre != NULL: the reference half comes
-// from a prepared reference (nabo_tc_prepare_ref) and only the queries are packed, with its scale.
-int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
-                       int metric, const uint8_t* mask, int drop_first, int* n_split_io, NaboArena& ar, int32_t** cand_idx_out,
-                       int* kprime_out, float** cert_tau_out, double** qn2_out, double** scal_out, int* launches,
-                       NaboStageTimer& tm, cudaStream_t st, NaboCandBuf* raw_out, NaboTailSplit* tail, const NaboTcRef* pre) {
-    // raw_out != NULL: when every query has ONE buffer (no reference split, K' <= 64) the final selection is left to
-    // the re-rank kernel: raw_out is filled and no emit kernel runs.
-    // *n_split_io in: reference pieces per item when there are few items (nabo_tc_split), or 0 = one piece (the
-    // public candidate entry point: one K' list per query); out: K' lists per query
-    int n_split = *n_split_io;
+// Accumulation-error constant of the tensor-core score relative to (4|q||r| + |r|^2 + |q|^2);
+// measured on B200 by tests/test_gpu_tc.py::test_tc_score_error_bound, which asserts a >= 4x margin.
+static const double kCAcc = 1.52587890625e-05;   // 2^-16
+
+// Runs norms -> scale -> pack -> candidate kernel (-> emit kernel) in the regions of nabo_tc_carve.  pre != NULL: the
+// reference half comes from a prepared reference (nabo_tc_prepare_ref) and only the queries are packed, with its scale.
+// plan.fused: every query has ONE buffer (no reference split, K' <= 64) and the final selection is left to the re-rank
+// kernel (out->raw); otherwise the emit kernel writes plan.n_split K' lists per query.
+int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int metric,
+                       const uint8_t* mask, const NaboFastPlan& plan, const NaboTcWork& w, bool timed, NaboStageTimer& tm,
+                       cudaStream_t st, const NaboTcRef* pre, NaboCandidates* out) {
     const int kp = tc::kp_for(g);
     const tc::SmemPlan pl = tc::plan_smem(g);
     const size_t tb = tc::tile_bytes(kp);
     const int n_items = (n_query + pl.nq * tc::TILE - 1) / (pl.nq * tc::TILE);
     const int n_qtiles = n_items * pl.nq;
     const int n_rtiles = (n_ref + tc::TILE - 1) / tc::TILE;
-    const tc::KPlan kpl = tc::plan_k(k + (drop_first ? 1 : 0));
-    const int kprime = kpl.kprime;
-    if (n_split < 1 || n_split > NABO_TC_MAX_SPLIT || kpl.cap != tc::CAP_SMALL) n_split = 1;   // 256 keys: unsplit only
-    const int grid = tc_grid(n_items * n_split);
-
-    __half* qa = (__half*)ar.take<char>((size_t)n_qtiles * tb);
-    __half* rb = pre ? (__half*)pre->rb : (__half*)ar.take<char>((size_t)n_rtiles * tb);
-    double* qnorm = ar.take<double>(n_query);
-    double* qn2 = ar.take<double>(n_query);
-    double* rnorm = pre ? nullptr : ar.take<double>(n_ref);
+    const int kprime = plan.kprime, n_split = plan.n_split;
+    const int sms = nabo_sm_count(), grid = n_items * n_split < sms ? n_items * n_split : sms;
+    __half* qa = (__half*)w.qa;
+    __half* rb = pre ? (__half*)pre->rb : (__half*)w.rb;
+    double* scal = pre ? (double*)pre->scal : w.scal;
+    unsigned int* maxbits = w.maxbits;
     const size_t n_slots = (size_t)n_items * n_split * pl.nq * tc::TILE;
-    unsigned long long* cbuf = ar.take<unsigned long long>(n_slots * kpl.cap);
-    int* ccnt = ar.take<int>(n_slots);
-    float* ctau = ar.take<float>(n_slots);
-    int32_t* cand = ar.take<int32_t>((size_t)n_query * kprime * n_split);
-    float* tau = ar.take<float>((size_t)n_query * n_split);
-    double* scal = pre ? (double*)pre->scal : ar.take<double>(4);
-    unsigned int* maxbits = ar.take<unsigned int>(3 + (size_t)n_items);    // 2 norm maxima, CTA ticket, head flags
-    if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the tensor-core pass");
 
     NABO_CUDA(cudaMemsetAsync(maxbits, 0, (3 + (size_t)n_items) * sizeof(unsigned int), st));
-    tc::norms_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(q, ldq, n_query, g, qnorm, maxbits);
+    tc::norms_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(q, ldq, n_query, g, w.qnorm, maxbits);
     if (!pre) {
-        tc_ref_norms(r, ldr, n_ref, g, rnorm, maxbits + 1, st);
+        tc_ref_norms(r, ldr, n_ref, g, w.rnorm, maxbits + 1, st);
         tc::scale_kernel<<<1, 1, 0, st>>>(maxbits, maxbits + 1, metric == NABO_COSINE ? 1 : 0, scal);
     }
-    tc::pack_kernel<true><<<n_qtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(q, ldq, n_query, g, kp, qnorm, scal, nullptr, qa, qn2);
-    if (!pre) tc_ref_pack(r, ldr, n_ref, g, rnorm, scal, mask, rb, st);
+    tc::pack_kernel<true><<<n_qtiles, tc::TILE * tc::PACK_SPLIT, 0, st>>>(q, ldq, n_query, g, kp, w.qnorm, scal, nullptr, qa,
+                                                                         w.qn2);
+    if (!pre) tc_ref_pack(r, ldr, n_ref, g, w.rnorm, scal, mask, rb, st);
     NABO_LAUNCH_CHECK("tc pack kernels");
     tm.end(3);
 
@@ -954,9 +941,10 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     p.qa = qa; p.rb = rb;
     p.n_query = n_query; p.n_ref = n_ref; p.kp = kp; p.n_items = n_items; p.n_rtiles = n_rtiles;
     p.stages = pl.stages; p.kprime = kprime; p.kc_out = kprime; p.n_split = n_split;
-    p.cand_buf = cbuf; p.cand_cnt = ccnt; p.cand_tau = ctau; p.cand_idx = cand; p.cert_tau = tau; p.ticket = maxbits + 2;
+    p.cand_buf = w.cbuf; p.cand_cnt = w.ccnt; p.cand_tau = w.ctau; p.cand_idx = w.cand; p.cert_tau = w.tau;
+    p.ticket = maxbits + 2;
     p.a_off = pl.a_off; p.b_off = pl.b_off; p.sort_off = pl.sort_off; p.bar_off = pl.bar_off;
-    p.soft = kpl.cap - tc::CHUNK - 16 > kprime ? kpl.cap - tc::CHUNK - 16 : kprime;
+    p.soft = plan.cap - tc::CHUNK - 16 > kprime ? plan.cap - tc::CHUNK - 16 : kprime;
     // Cut items at CTA boundaries only when the last wave would be partly filled and the packed reference fits in half of
     // L2 (the running items' candidate buffers take 57 MB at g <= 52 with 128 keys; with 256 keys they take 116 MB, 78 MB
     // in the wide plan, and reference + buffers exceed L2 - yet the cuts still pay there: 100 k queries at k = 100,
@@ -969,18 +957,13 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     // line is a reasoned choice, not a measured one.  Without cuts every CTA c sweeps the items c, c + grid, ... (contiguous
     // blocks of whole items measured 2 % slower at 500 k x 2 M), as it does for a whole number of waves.
     p.cut = n_items % grid != 0 && (size_t)n_rtiles * tb <= l2_bytes() / 2 ? 1 : 0;
-    // Without cuts the last wave is partly filled (see NaboTailSplit): every CTA signals after its last full-wave item
-    // when the caller can use the gap - the fused re-rank path only, at least two waves, at least 16 SMs idle in the last
-    // one.  At 500 k x 2 M cosine (1 303 items) dropping this overlap cost 2.5 % of the kNN stage.
-    const bool fused = raw_out && n_split == 1 && kprime <= 64;
+    // Without cuts the last wave is partly filled (see NaboCandidates::rows_full): every CTA signals after its last
+    // full-wave item when the caller can use the gap - the fused re-rank path only, at least two waves, at least 16 SMs
+    // idle in the last one.  At 500 k x 2 M cosine (1 303 items) dropping this overlap cost 2.5 % of the kNN stage.
     const int rem_items = n_items % grid;
-    const bool tail_applies = tail && fused && !p.cut && n_items > grid && rem_items > 0 && grid - rem_items >= 16;
-    const bool overlap = tail_applies && !tail->dry;
+    const bool tail_applies = plan.fused && !p.cut && n_items > grid && rem_items > 0 && grid - rem_items >= 16;
+    const bool overlap = tail_applies && !timed;
     p.signal_round = overlap ? n_items / grid : 0;
-    if (tail) {
-        tail->applies = tail_applies ? 1 : 0;
-        tail->rows_full = overlap ? (n_items - rem_items) * pl.nq * tc::TILE : 0;
-    }
 #define NABO_TC_LAUNCH1(KS, SPLIT, NQ, SLAB, CAP)                                                                  \
     do {                                                                                                           \
         NABO_CUDA(cudaFuncSetAttribute(tc::candidates_kernel<KS, SPLIT, NQ, SLAB, CAP>,                            \
@@ -989,7 +972,7 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     } while (0)
 #define NABO_TC_LAUNCH(KS, NQ, SLAB)                                                                               \
     do {                                                                                                           \
-        if (kpl.cap == tc::CAP_LARGE) NABO_TC_LAUNCH1(KS, false, NQ, SLAB, tc::CAP_LARGE);                         \
+        if (plan.cap == tc::CAP_LARGE) NABO_TC_LAUNCH1(KS, false, NQ, SLAB, tc::CAP_LARGE);                        \
         else if (n_split > 1) NABO_TC_LAUNCH1(KS, true, NQ, SLAB, tc::CAP_SMALL);                                  \
         else NABO_TC_LAUNCH1(KS, false, NQ, SLAB, tc::CAP_SMALL);                                                  \
     } while (0)
@@ -1005,30 +988,27 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
     NABO_LAUNCH_CHECK("candidates_kernel");
     if (!overlap) tm.end(0);       // the final selection below is timed with the re-rank stage; with a dependent launch the
                                    // caller ends the stage after that launch (nothing may sit between the two kernels)
-    if (fused) {
-        raw_out->buf = cbuf; raw_out->cnt = ccnt; raw_out->tau = ctau; raw_out->kprime = kprime;
-        *cand_idx_out = cand; *kprime_out = kprime; *cert_tau_out = tau; *qn2_out = qn2; *scal_out = scal;
-        *launches += pre ? 3 : 6;
-        *n_split_io = 1;
+    out->cand = w.cand;
+    out->n_cand = kprime * n_split;
+    out->cert.kind = metric == NABO_COSINE ? NABO_CERT_COSINE : NABO_CERT_EUCLID;
+    out->cert.tau = w.tau; out->cert.qn2 = w.qn2; out->cert.scal = scal; out->cert.c_acc = kCAcc;
+    out->cert.abs_slack = 2.0 * sqrt((double)g) * 5.9604644775390625e-08;
+    out->raw.buf = nullptr;
+    out->rows_full = overlap ? (n_items - rem_items) * pl.nq * tc::TILE : 0;
+    // preparation kernels (3 with a prepared reference), the emit kernel and the engine's tau_min launch of a split
+    // call, and the dependent re-rank launch wherever the shape qualifies for it (timed or not)
+    out->launches = (pre ? 3 : 6) + (plan.fused ? 0 : 1) + (n_split > 1 ? 1 : 0) + (tail_applies ? 1 : 0);
+    if (plan.fused) {
+        out->raw.buf = w.cbuf; out->raw.cnt = w.ccnt; out->raw.tau = w.ctau; out->raw.kprime = kprime;
         return 0;
     }
-    if (raw_out) raw_out->buf = nullptr;
     const unsigned emit_blocks = (unsigned)((n_slots + 7) / 8);
-    if (kpl.cap == tc::CAP_LARGE) {
+    if (plan.cap == tc::CAP_LARGE) {
         if (pl.nq == 2) tc::emit_kernel<2, tc::CAP_LARGE><<<emit_blocks, 256, 0, st>>>(p);
         else tc::emit_kernel<3, tc::CAP_LARGE><<<emit_blocks, 256, 0, st>>>(p);
     } else if (pl.nq == 2) tc::emit_kernel<2><<<emit_blocks, 256, 0, st>>>(p);
     else tc::emit_kernel<3><<<emit_blocks, 256, 0, st>>>(p);
     NABO_LAUNCH_CHECK("emit_kernel");
-    *launches += 1;
-    if (n_split > 1) {
-        int rc = nabo_tau_min_launch(tau, n_query, n_split, st);
-        if (rc) return rc;
-        *launches += 1;
-    }
-    *n_split_io = n_split;
-    *cand_idx_out = cand; *kprime_out = kprime; *cert_tau_out = tau; *qn2_out = qn2; *scal_out = scal;
-    *launches += pre ? 3 : 6;
     return 0;
 }
 
@@ -1059,8 +1039,20 @@ extern "C" int nabo_knn_candidates_width(int k, int drop_first) {
     return tc::kprime_for(k + (drop_first ? 1 : 0), tc::MAX_KPRIME);
 }
 
+// One K' list per query, no reference split, no fused selection.
+static NaboFastPlan candidates_plan(int k, int drop_first) {
+    NaboFastPlan p;
+    p.path = NABO_PATH_TC;
+    p.kprime = nabo_tc_kprime(k, drop_first, &p.cap);
+    p.n_split = 1; p.fused = false; p.prepared = false;
+    return p;
+}
+
 extern "C" size_t nabo_knn_candidates_workspace_bytes(int n_query, int n_ref, int g, int k, int drop_first) {
-    return nabo_tc_workspace_bytes(n_query, n_ref, g, k, drop_first);
+    NaboArena m = NaboArena::measure();
+    NaboTcWork w;
+    nabo_tc_carve(m, n_query, n_ref, g, candidates_plan(k, drop_first), &w);
+    return m.off;
 }
 
 extern "C" int nabo_knn_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,
@@ -1073,19 +1065,20 @@ extern "C" int nabo_knn_candidates(const double* q, int ldq, const double* r, in
     NABO_ARG(q && r && out_cand && out_tau, "candidates: null pointer");
     if (!candidates_supported(g, k, drop_first))
         return nabo_set_error(NABO_EUNSUPPORTED, "candidates: g=%d k=%d outside the tensor-core tile plan", g, k);
+    const NaboFastPlan plan = candidates_plan(k, drop_first);
     NaboArena ar(workspace, workspace_bytes);
+    NaboTcWork w;
+    nabo_tc_carve(ar, n_query, n_ref, g, plan, &w);
+    if (!ar.ok) return nabo_set_error(NABO_EWORKSPACE, "knn: workspace too small for the tensor-core pass");
     NaboStageTimer tm(false, st);
-    int32_t* cand = nullptr;
-    float* tau = nullptr;
-    double *qn2 = nullptr, *scal = nullptr;
-    int kprime = 0, launches = 0;
-    int one_list = 0;
-    int rc = nabo_tc_candidates(q, ldq, r, ldr, n_query, n_ref, g, k, metric, ref_mask, drop_first, &one_list, ar, &cand,
-                                &kprime, &tau, &qn2, &scal, &launches, tm, st);
+    NaboCandidates c;
+    int rc = nabo_tc_candidates(q, ldq, r, ldr, n_query, n_ref, g, metric, ref_mask, plan, w, false, tm, st, nullptr, &c);
     if (rc) return rc;
-    NABO_CUDA(cudaMemcpyAsync(out_cand, cand, sizeof(int32_t) * (size_t)n_query * kprime, cudaMemcpyDeviceToDevice, st));
-    NABO_CUDA(cudaMemcpyAsync(out_tau, tau, sizeof(float) * (size_t)n_query, cudaMemcpyDeviceToDevice, st));
-    if (out_qn2) NABO_CUDA(cudaMemcpyAsync(out_qn2, qn2, sizeof(double) * (size_t)n_query, cudaMemcpyDeviceToDevice, st));
-    if (out_scal) NABO_CUDA(cudaMemcpyAsync(out_scal, scal, sizeof(double) * 4, cudaMemcpyDeviceToDevice, st));
+    NABO_CUDA(cudaMemcpyAsync(out_cand, c.cand, sizeof(int32_t) * (size_t)n_query * plan.kprime, cudaMemcpyDeviceToDevice,
+                              st));
+    NABO_CUDA(cudaMemcpyAsync(out_tau, c.cert.tau, sizeof(float) * (size_t)n_query, cudaMemcpyDeviceToDevice, st));
+    if (out_qn2)
+        NABO_CUDA(cudaMemcpyAsync(out_qn2, c.cert.qn2, sizeof(double) * (size_t)n_query, cudaMemcpyDeviceToDevice, st));
+    if (out_scal) NABO_CUDA(cudaMemcpyAsync(out_scal, c.cert.scal, sizeof(double) * 4, cudaMemcpyDeviceToDevice, st));
     return 0;
 }
