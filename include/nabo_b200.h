@@ -238,8 +238,12 @@ int nabo_classify_targets(const int32_t* tgt_knn, const uint8_t* counts, const d
  * reference's sum), out_pairs[t] = ordered pairs connected, out_nmapped[t] = mapped cells; the mean is
  * (out_sum / 2) / (nmapped (nmapped - 1) / 2); out_pairs < nmapped (nmapped - 1) means "no path"
  * (the reference raises NetworkXNoPath), nmapped < 2 means "no pairs" (the reference's NaN).
- * One bit-parallel multi-source BFS per target instead of one BFS per pair; k <= 64. */
+ * One bit-parallel multi-source BFS per target instead of one BFS per pair; k <= 128.
+ * nabo_specificity_workspace_bytes_k sizes the workspace for tables of width k: tables up to 64 wide take
+ * 45 bytes per reference cell and CTA, wider ones 81; 0 for k > 128.  nabo_specificity_workspace_bytes is
+ * the size for k <= 64. */
 size_t nabo_specificity_workspace_bytes(int n_ref, int n_query);
+size_t nabo_specificity_workspace_bytes_k(int n_ref, int n_query, int k);
 int nabo_mapping_specificity(const long long* indptr, const int32_t* indices, int n_ref,
                              const int32_t* tgt_knn, const uint8_t* counts, int n_query, int k,
                              long long* out_sum, int32_t* out_pairs, int32_t* out_nmapped,

@@ -66,6 +66,7 @@ SIGNATURES: Dict[str, tuple] = {
     "nabo_mapping_scores": (_i, [_p, _p, _p, _i, _i, _i, _p, _i, _d, _i, _d, _d, _p, _p, _z, _p]),
     "nabo_classify_targets": (_i, [_p, _p, _p, _i, _i, _p, _i, _d, _i, _d, _p, _p]),
     "nabo_specificity_workspace_bytes": (_z, [_i, _i]),
+    "nabo_specificity_workspace_bytes_k": (_z, [_i, _i, _i]),
     "nabo_mapping_specificity": (_i, [_p, _p, _i, _p, _p, _i, _i, _p, _p, _p, _p, _z, _p]),
     "nabo_connected_components": (_i, [_p, _p, C.c_longlong, _i, _p, _p, _z, _p]),
     "nabo_sparse_row_stats": (_i, [_p, _p, _p, _i, _i, _p, _p, C.c_longlong, _i, _p, _p, _p, _p, _p, _p]),

@@ -558,6 +558,7 @@ def mapping_specificity(indptr, indices, tgt_knn, counts):
     """Array form of ``Graph.get_mapping_specificity`` (nabo/_graph.py:794-824): per target, the mean
     unweighted shortest-path length in the reference graph (symmetric CSR ``indptr`` int64, ``indices``
     int32) between all pairs of reference cells the target has an edge to (``counts > 0``).
+    ``tgt_knn`` / ``counts`` are (N, k) with k <= 128 (every k the kNN engines take); wider tables raise.
     Returns (mean float64 (N,) with NaN where fewer than two cells are mapped, connected bool (N,) -
     False where some pair has no path, which is where the reference raises NetworkXNoPath)."""
     require_device()
@@ -571,7 +572,7 @@ def mapping_specificity(indptr, indices, tgt_knn, counts):
     osum = torch.empty(n, dtype=torch.int64, device=td.device)
     opairs = torch.empty(n, dtype=torch.int32, device=td.device)
     onm = torch.empty(n, dtype=torch.int32, device=td.device)
-    wb = lib().nabo_specificity_workspace_bytes(m, n)
+    wb = lib().nabo_specificity_workspace_bytes_k(m, n, kk)
     ws = torch.empty(max(wb, 1), dtype=torch.uint8, device=td.device)
     check(lib().nabo_mapping_specificity(_ptr(ip), _ptr(ix), m, _ptr(td), _ptr(cd), n, kk, _ptr(osum), _ptr(opairs),
                                          _ptr(onm), _ptr(ws), ws.numel(), C.c_void_p(_stream())), "mapping_specificity")
