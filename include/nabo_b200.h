@@ -83,8 +83,8 @@ int nabo_cosine_dist(const double* x, int ldx, const double* y, int ldy, double*
  *   the exact engine (same results) elsewhere; ksel = k + drop_first:
  *     Euclidean / cosine  1 <= g <= 128, ksel <= 128 (tensor-core pass: 128-key buffers for
  *                         ksel + 8 <= 96, 256-key buffers for 89 <= ksel <= 128)
- *     modified Canberra   ksel + 8 <= 64; g <= 128 with dist_factor >= 1e-6 (bit-sliced
- *                         pass), g <= 77 otherwise (FP16 two-phase pass)
+ *     modified Canberra   ksel + 8 <= 64, g <= 128, dist_factor >= 1e-6 (bit-sliced pass);
+ *                         dist_factor < 1e-6: exact engine
  */
 size_t nabo_knn_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, int mode);
 int nabo_knn(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,
@@ -151,9 +151,9 @@ int nabo_knn_routed(const double* q, int ldq, const double* r, int ldr, int n_qu
  * The tensor-core scale of a prepared reference comes from the reference's largest norm alone (cosine: 32), not
  * from the queries: a query whose scaled coordinates would overflow FP16 (about 500x the largest reference norm)
  * is sent to the exact fallback and counted in stats_host[1].
- * Calls the prepared operands do not serve run the existing path on the stored rows: mode = NABO_MODE_EXACT, k
- * beyond the fast plans (the exact engine), and modified Canberra with dist_factor < 1e-6 (the FP16 two-phase pass);
- * nabo_knn_prepared_workspace_bytes then returns the one-shot size.
+ * Calls the prepared operands do not serve run the exact engine on the stored rows: mode = NABO_MODE_EXACT, k beyond
+ * the fast plans, and modified Canberra with dist_factor < 1e-6.  A fast-mode call that runs the exact engine for
+ * every drop_first needs no workspace: nabo_knn_prepared_workspace_bytes returns 0 for it.
  * Status: a descriptor that was not filled by nabo_ref_prepare or does not match its buffer -> NABO_EINVAL; another
  * ABI version, a metric / g without a fast plan (1 <= g <= 128) or k + drop_first > 128 -> NABO_EUNSUPPORTED. */
 #define NABO_PREPARED_MAGIC 0x5250424eu   /* "NBPR" */

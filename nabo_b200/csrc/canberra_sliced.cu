@@ -12,9 +12,8 @@
 //     a superset of the unsaturated ones, for 32 references with two shared-memory loads and one LOP3;
 //   * the g flag words are summed vertically with a carry-save adder tree (Harley-Seal, 2.25 LOP3 per
 //     dimension) into a 6-bit sliced counter (8 bits for g > 56) and compared with need(tau) = min{c : g - c < tau};
-//   * the surviving pairs (about 2 % once tau is warm) go through the dense FP32 evaluation
-//     (same arithmetic and error bound nabo_cb_eps as canberra_candidates.cu) and the running top-K'
-//     selection of select.cuh.
+//   * the surviving pairs (about 2 % once tau is warm) go through the dense FP32 evaluation (a lower
+//     bound of the exact distance up to nabo_cb_eps(g)) and the running top-K' selection of select.cuh.
 //
 // Lanes are queries: a warp owns 32 queries for the whole reference sweep (their bin intervals live in
 // registers, their thresholds / counts in a private shared-memory slice); the NW warps of a CTA share the
@@ -55,13 +54,14 @@ constexpr int NBINS = 32;                 // value bins per dimension
 constexpr int NPL = NBINS + 1;            // cumulative planes per (dimension, word)
 constexpr int SLEEP_NS = 400;             // suspend-time hint of the tile waits
 constexpr int CAP = sel::CAP;
+constexpr int KP_MAX = CAP - 64;          // largest K' of the plan, which takes ksel + 8 <= KP_MAX
 constexpr int MAX_STAGES = 4;
 constexpr int EDGE_SAMPLE = 4096;
 constexpr int TRIG_EXTRA = 24;            // keys above kprime that trigger a compaction
 
 // Tile plan, a function of NB = ceil(g / 8) alone (one kernel instance per NB).
-//   narrow, g <= 56: 12 warps, 128-reference tiles, 6-bit sliced counters (count <= 63), and the FP32 reference
-//                    copy of canberra_candidates.cu ([tile64][k][64]);
+//   narrow, g <= 56: 12 warps, 128-reference tiles, 6-bit sliced counters (count <= 63), and a [tile64][k][64]
+//                    FP32 reference copy (pretile_kernel);
 //   wide, 57 <= g <= 128: the query bin intervals (4 NB registers) no longer fit 12 warps' register budget (168
 //                    per thread), so 8 warps (up to 255); 8-bit counters (count <= 128); the per-warp FP32 query
 //                    tiles (1 024 g bytes with 8 warps) leave room for two stages of 64-reference tiles up to
@@ -215,6 +215,23 @@ ctrl_kernel(const double* __restrict__ q, int ld, int n_query, int g, int nj, do
     }
     ctrl[e] = word;
 }
+
+// FP32 copy of a row-major FP64 matrix, pre-tiled k-major: out[(tile * g + k) * 64 + row_in_tile] (the narrow plan's
+// reference copy).  A tile is then a straight, contiguous copy.
+__global__ void __launch_bounds__(256)
+pretile_kernel(const double* __restrict__ x, int ld, int n, int g, float* __restrict__ out) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long total = (long long)((n + 63) / 64) * g * 64;
+    if (e >= total) return;
+    const int rl = (int)(e & 63);
+    const long long tk = e >> 6;
+    const int k = (int)(tk % g);
+    const long long tile = tk / g;
+    const long long row = tile * 64 + rl;
+    out[e] = row < n ? (float)x[row * ld + k] : 0.f;
+}
+// floats of the pretile_kernel copy; the wide plan's [tile32][k][32] copy fits in the same count
+static inline size_t pretile_floats(int n, int g) { return (size_t)((n + 63) / 64) * g * 64; }
 
 // FP32 rows, 32 per group, dimension-major: qx[(group32 * g + k) * 32 + lane] (the queries; in the wide plan the
 // reference copy too)
@@ -657,8 +674,18 @@ extern "C" int nabo_dbg_cbs_prof(unsigned long long* out_host, int reset) {
 bool nabo_cbs_supported(int g, int k, int drop_first) {
     if (g < 1 || g > 128) return false;
     const int ksel = k + (drop_first ? 1 : 0);
-    return cbs::plan_smem(g).stages >= 2 && ksel + 8 <= cbs::CAP - 64;
+    return cbs::plan_smem(g).stages >= 2 && ksel + 8 <= cbs::KP_MAX;
 }
+
+int nabo_cbs_kprime(int k, int drop_first) {
+    const int ksel = k + (drop_first ? 1 : 0);
+    const int kp = ksel + (ksel / 4 > 8 ? ksel / 4 : 8);
+    return kp < cbs::KP_MAX ? kp : cbs::KP_MAX;
+}
+
+// |FP32 score - (a lower bound of) the exact distance|: sequential FP32 sum of g terms <= 1 plus the
+// per-term rounding of the difference, the denominator and the approximate division.
+static double nabo_cb_eps(int g) { return 1.2e-7 * (double)g * g + 2e-6 * g + 4e-7 * g; }
 
 // CTAs of the sweep: whole query blocks, each cut into the plan's reference pieces (nabo_fast_plan keeps n_split at
 // most the SM count)
@@ -678,16 +705,16 @@ int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first) {
     const int per_cta = (n_groups + sms - 1) / sms;
     int s = per_cta > 0 ? pl.nw / per_cta : 1;
     if (s > NABO_CBS_MAX_SPLIT) s = NABO_CBS_MAX_SPLIT;
-    while (s > 1 && (n_tiles / s < 8192 / pl.rt || s * nabo_cb_kprime(k, drop_first) > 128)) --s;
+    while (s > 1 && (n_tiles / s < 8192 / pl.rt || s * nabo_cbs_kprime(k, drop_first) > 128)) --s;
     return s < 1 ? 1 : s;
 }
 
-// The reference half: FP32 copy (nabo_cb_pretile_floats(n_ref, g) floats: [tile64][k][64], or [tile32][k][32] in the
-// wide plan), cumulative planes, bin edges.  The regions of a prepared reference's buffer, and of a call without one.
+// The reference half: FP32 copy ([tile64][k][64], or [tile32][k][32] in the wide plan), cumulative planes, bin edges.
+// The regions of a prepared reference's buffer, and of a call without one.
 static void cbs_ref_carve(NaboArena& ar, int n_ref, int g, NaboCbsWork* w) {
     const cbs::SmemPlan pl = cbs::plan_smem(g);
     const size_t n_tiles = (n_ref + pl.rt - 1) / pl.rt;
-    w->rt = ar.take<float>(nabo_cb_pretile_floats(n_ref, g));
+    w->rt = ar.take<float>(cbs::pretile_floats(n_ref, g));
     w->planes = (uint32_t*)ar.take<char>(n_tiles * cbs::plane_tile_bytes(g, pl.rt));
     w->edges = ar.take<float>((size_t)g * (cbs::NBINS - 1));
 }
@@ -705,14 +732,14 @@ void nabo_cbs_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFast
 }
 
 // The reference half of the sliced pass.  None of it depends on the queries or on dist_factor.
-static int cbs_ref_launch(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, float* rt, float* edges,
-                          uint32_t* planes, cudaStream_t st) {
+static void cbs_ref_launch(const double* r, int ldr, int n_ref, int g, const uint8_t* mask, float* rt, float* edges,
+                           uint32_t* planes, cudaStream_t st) {
     const cbs::SmemPlan pl = cbs::plan_smem(g);
     const int n_tiles = (n_ref + pl.rt - 1) / pl.rt;
     const int n_yblk = (n_ref + pl.yw - 1) / pl.yw;
     if (pl.yw == 64) {
-        int rc = nabo_cb_pretile_launch(r, ldr, n_ref, g, rt, st);
-        if (rc) return rc;
+        const size_t tr = cbs::pretile_floats(n_ref, g);
+        cbs::pretile_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, rt);
     } else {
         const long long tr = (long long)n_yblk * g * 32;
         cbs::pretile32_kernel<<<(unsigned)((tr + 255) / 256), 256, 0, st>>>(r, ldr, n_ref, g, rt, tr);
@@ -723,7 +750,6 @@ static int cbs_ref_launch(const double* r, int ldr, int n_ref, int g, const uint
         case 64: cbs::planes_kernel<64, 32><<<dim3(n_tiles, g), 64, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
         default: cbs::planes_kernel<32, 32><<<dim3(n_tiles, g), 32, 0, st>>>(rt, edges, mask, n_ref, g, planes); break;
     }
-    return 0;
 }
 
 size_t nabo_cbs_prepared_bytes(int n_ref, int g) {
@@ -740,8 +766,7 @@ int nabo_cbs_prepare_ref(const double* r, int ldr, int n_ref, int g, const uint8
     NaboCbsWork w;
     cbs_ref_carve(ar, n_ref, g, &w);
     if (!ar.ok) return nabo_set_error(NABO_EINVAL, "ref_prepare: buffer layout");
-    int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, w.rt, w.edges, w.planes, st);
-    if (rc) return rc;
+    cbs_ref_launch(r, ldr, n_ref, g, mask, w.rt, w.edges, w.planes, st);
     NABO_LAUNCH_CHECK("cbs reference preparation");
     out->rt = w.rt;
     out->planes = w.planes;
@@ -765,10 +790,7 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     uint32_t* planes = pre ? (uint32_t*)pre->planes : w.planes;
     float* edges = pre ? (float*)pre->edges : w.edges;
 
-    if (!pre) {
-        int rc = cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
-        if (rc) return rc;
-    }
+    if (!pre) cbs_ref_launch(r, ldr, n_ref, g, mask, rt, edges, planes, st);
     const long long tc = (long long)n_groups * nj * 32;
     cbs::ctrl_kernel<<<(unsigned)((tc + 255) / 256), 256, 0, st>>>(q, ldq, n_query, g, nj, f, edges, w.ctrl, tc);
     const long long tq = (long long)n_groups * g * 32;
@@ -779,7 +801,10 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     p.planes = planes; p.rt = rt; p.qx = w.qx; p.ctrl = w.ctrl;
     p.n_query = n_query; p.n_ref = n_ref; p.g = g; p.n_tiles = n_tiles; p.n_yblk = n_yblk;
     p.n_groups = (int)n_groups; p.kprime = kprime; p.stages = pl.stages; p.nj = nj; p.n_split = n_split;
-    const double delta = fmax(1e-5, 4e-7 * (2.0 + f) / f);      // same optimistic margin as canberra_candidates.cu
+    // Optimistic margin of the saturation predicate: whenever the exact FP64 test |x-y| < f|x| holds, the FP32 test on
+    // the rounded inputs must hold too.  Near the threshold |y| <= (1+f)|x|, so the FP32 difference is off by at most
+    // ~1.2e-7 (2+f)|x|; delta covers it with a 3x reserve.
+    const double delta = fmax(1e-5, 4e-7 * (2.0 + f) / f);
     p.fm = (float)(f * (1.0 + delta));
     p.cand_buf = w.cbuf; p.cand = w.cand; p.tau_out = w.tau;
     p.trig_extra = cbs::TRIG_EXTRA;
@@ -807,6 +832,9 @@ int nabo_cbs_candidates(const double* q, int ldq, const double* r, int ldr, int 
     }
 #undef NABO_CBS_LAUNCH
     NABO_LAUNCH_CHECK("cbs::sliced_kernel");
-    nabo_cb_result(w.cand, w.tau, kprime * n_split, g, 6, out);    // 6 launches reported, prepared or not
+    // the score is a lower bound of the distance up to nabo_cb_eps(g); 6 launches reported, prepared or not
+    out->cand = w.cand; out->n_cand = kprime * n_split; out->raw.buf = nullptr; out->rows_full = 0; out->launches = 6;
+    out->cert.kind = NABO_CERT_LINEAR; out->cert.tau = w.tau; out->cert.qn2 = nullptr; out->cert.scal = nullptr;
+    out->cert.c_acc = nabo_cb_eps(g); out->cert.abs_slack = 0.0;
     return 0;
 }

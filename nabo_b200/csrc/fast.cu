@@ -2,8 +2,7 @@
 // for the rows the certificate could not clear.  Results are identical to the exact engine
 // (and hence to the reference) by construction; only the amount of FP64 work changes.
 //   Euclidean / cosine : tensor-core candidate pass (tc_candidates.cu)
-//   modified Canberra  : bit-sliced count bound + FP32 evaluation (canberra_sliced.cu, g <= 128), or the two-phase
-//                        FP16 / FP32 CUDA-core pass (canberra_candidates.cu, g <= 77) for a vanishing dist_factor
+//   modified Canberra  : bit-sliced count bound + FP32 evaluation (canberra_sliced.cu, g <= 128, dist_factor >= 1e-6)
 #include "knn_internal.cuh"
 
 NaboFastPlan nabo_fast_plan(int n_query, int n_ref, int g, int k, int metric, double f, int drop_first, bool pre) {
@@ -25,17 +24,16 @@ NaboFastPlan nabo_fast_plan(int n_query, int n_ref, int g, int k, int metric, do
     }
     if (metric != NABO_MOD_CANBERRA) return p;
     // the interval ends of the sliced pass carry a 1e-6 relative margin over f|x|; it must dominate the FP64
-    // rounding of x -+ f|x| (~1e-16 |x|), so a vanishing dist_factor goes to the FP16 two-phase pass instead
-    const bool sliced = nabo_cbs_supported(g, k, drop_first) && f >= 1e-6;
-    const int kprime = nabo_cb_kprime(k, drop_first);
-    if (!(sliced || nabo_cb_supported(g, k, drop_first)) || n_ref <= kprime) return p;
-    p.path = sliced ? NABO_PATH_SLICED : NABO_PATH_TWO_PHASE;
+    // rounding of x -+ f|x| (~1e-16 |x|), so a vanishing dist_factor runs on the exact engine.  No candidate pass would
+    // help there: nearly every pair is at d = g, so the K'-th candidate ties the threshold and the certificate fails.
+    if (!nabo_cbs_supported(g, k, drop_first) || f < 1e-6) return p;
+    const int kprime = nabo_cbs_kprime(k, drop_first);
+    if (n_ref <= kprime) return p;
+    p.path = NABO_PATH_SLICED;
     p.kprime = kprime;
-    if (sliced) {
-        p.n_split = nabo_cbs_split(n_query, n_ref, g, k, drop_first);
-        if (nabo_sm_count() < p.n_split) p.n_split = 1;     // the pieces of a query block run on CTAs of their own
-        p.prepared = pre;
-    }
+    p.n_split = nabo_cbs_split(n_query, n_ref, g, k, drop_first);
+    if (nabo_sm_count() < p.n_split) p.n_split = 1;     // the pieces of a query block run on CTAs of their own
+    p.prepared = pre;
     return p;
 }
 
@@ -45,7 +43,6 @@ struct FastWork {
     NaboExactSplit split, few;
     NaboTcWork tc;
     NaboCbsWork cbs;
-    NaboCbWork cb;
 };
 
 // The regions of one call: the failure list first (the re-rank of the full waves may start while the tensor-core pass
@@ -57,22 +54,20 @@ static void fast_carve(NaboArena& ar, int n_query, int n_ref, int g, int k, int 
     w->fail_count = ar.take<int>(1);
     nabo_exact_split_carve(ar, n_ref, k + (drop_first ? 1 : 0), &w->split, &w->few);
     if (p.path == NABO_PATH_TC) nabo_tc_carve(ar, n_query, n_ref, g, p, &w->tc);
-    else if (p.path == NABO_PATH_SLICED) nabo_cbs_carve(ar, n_query, n_ref, g, p, &w->cbs);
-    else nabo_cb_carve(ar, n_query, n_ref, g, p, &w->cb);
+    else nabo_cbs_carve(ar, n_query, n_ref, g, p, &w->cbs);
 }
 
 size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, bool pre, double f) {
-    // the one-shot size has no dist_factor: for modified Canberra it covers both passes (f >= 1e-6 and below)
-    const double fs[2] = {pre ? f : 1.0, pre ? f : 0.0};
+    // the one-shot size has no dist_factor: the sliced carve, the same for every f >= 1e-6
+    const double fv = pre ? f : 1.0;
     size_t need = 0;
-    for (int drop_first = 0; drop_first <= 1; ++drop_first)
-        for (double fv : fs) {
-            NaboArena m = NaboArena::measure();
-            FastWork w;
-            fast_carve(m, n_query, n_ref, g, k, drop_first, nabo_fast_plan(n_query, n_ref, g, k, metric, fv, drop_first, pre),
-                       &w);
-            if (m.off > need) need = m.off;
-        }
+    for (int drop_first = 0; drop_first <= 1; ++drop_first) {
+        NaboArena m = NaboArena::measure();
+        FastWork w;
+        fast_carve(m, n_query, n_ref, g, k, drop_first, nabo_fast_plan(n_query, n_ref, g, k, metric, fv, drop_first, pre),
+                   &w);
+        if (m.off > need) need = m.off;
+    }
     return need;
 }
 
@@ -99,11 +94,9 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
     if (p.path == NABO_PATH_TC)        // stage timing asked for: the candidate kernel is timed on its own
         rc = nabo_tc_candidates(q, ldq, r, ldr, n_query, n_ref, g, metric, mask, p, w.tc, stats_host != nullptr, tm, st,
                                 p.prepared ? &pre->tc : nullptr, &c);
-    else if (p.path == NABO_PATH_SLICED)
+    else
         rc = nabo_cbs_candidates(q, ldq, r, ldr, n_query, n_ref, g, f, mask, p, w.cbs, st, p.prepared ? &pre->cbs : nullptr,
                                  &c);
-    else
-        rc = nabo_cb_candidates(q, ldq, r, ldr, n_query, n_ref, g, f, mask, p, w.cb, st, &c);
     if (rc) return rc;
     if (p.n_split > 1) {               // the re-rank certifies against the smallest threshold of the pieces
         rc = nabo_tau_min_launch(const_cast<float*>(c.cert.tau), n_query, p.n_split, st);

@@ -102,7 +102,6 @@ int nabo_rerank_launch(const double* q, int ldq, const double* r, int ldr, int n
 #define NABO_PATH_EXACT 0        // the exact engine on every row
 #define NABO_PATH_TC 1           // tensor-core candidate pass (Euclidean / cosine)
 #define NABO_PATH_SLICED 2       // bit-sliced modified-Canberra pass
-#define NABO_PATH_TWO_PHASE 3    // FP16 / FP32 two-phase modified-Canberra pass
 struct NaboFastPlan {
     int path;
     int kprime;       // K': candidates per list
@@ -160,24 +159,7 @@ int nabo_tc_candidates(const double* q, int ldq, const double* r, int ldr, int n
                        const uint8_t* mask, const NaboFastPlan& p, const NaboTcWork& w, bool timed, NaboStageTimer& tm,
                        cudaStream_t st, const NaboTcRef* pre, NaboCandidates* out);
 
-bool nabo_cb_supported(int g, int k, int drop_first);
-int nabo_cb_kprime(int k, int drop_first);
-double nabo_cb_eps(int g);
-size_t nabo_cb_pretile_floats(int n, int g);
-struct NaboCbWork {
-    int32_t* cand;                 // [n_query][K']
-    float *tau, *qt, *rt, *scale;  // tau: [n_query]; FP32 tiles; per-dimension scale (of the maxima in maxbits)
-    void* rh;                      // FP16 reference tiles
-    unsigned* maxbits;
-};
-void nabo_cb_carve(NaboArena& ar, int n_query, int n_ref, int g, const NaboFastPlan& p, NaboCbWork* w);
-int nabo_cb_candidates(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, double f,
-                       const uint8_t* mask, const NaboFastPlan& p, const NaboCbWork& w, cudaStream_t st,
-                       NaboCandidates* out);
-void nabo_cb_result(const int32_t* cand, const float* tau, int n_cand, int g, int launches, NaboCandidates* out);
-
-int nabo_cb_pretile_launch(const double* x, int ld, int n, int g, float* out, cudaStream_t st);
-// bit-sliced Canberra pass (canberra_sliced.cu); same outputs as nabo_cb_candidates
+// bit-sliced modified-Canberra pass (canberra_sliced.cu)
 // Reference half of the sliced pass, built once by nabo_cbs_prepare_ref: FP32 copy, cumulative planes, bin edges.
 struct NaboCbsRef {
     const float* rt;
@@ -185,6 +167,7 @@ struct NaboCbsRef {
     const float* edges;
 };
 bool nabo_cbs_supported(int g, int k, int drop_first);
+int nabo_cbs_kprime(int k, int drop_first);
 int nabo_cbs_split(int n_query, int n_ref, int g, int k, int drop_first);
 #define NABO_CBS_MAX_SPLIT 3
 struct NaboCbsWork {
@@ -208,9 +191,9 @@ struct NaboFastRef {
     NaboTcRef tc;
     NaboCbsRef cbs;
 };
-// Workspace of nabo_knn_fast, the largest carve over drop_first: pre = false for the one-shot call (which has no
-// dist_factor: for modified Canberra both passes; f is not read), true for a prepared reference with dist_factor f
-// (the one-shot carve wherever its operands do not serve the call).
+// Workspace of nabo_knn_fast, the largest carve over drop_first: pre = false for the one-shot call, which has no
+// dist_factor (f is not read; modified Canberra is sized for the sliced pass), true for a prepared reference with
+// dist_factor f.  0 when every drop_first runs the exact engine.
 size_t nabo_fast_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, bool pre, double f);
 int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g, int k,
                   int metric, double f, const uint8_t* mask, int drop_first, int idx_offset, int32_t* out_idx,

@@ -201,10 +201,10 @@ def test_cb_wide_mapping_drop_in(core, tmp_path):
 
 
 def test_cb_wide_vanishing_dist_factor(core):
-    """f = 1e-9 is below the sliced pass's interval margin and g = 100 above the two-phase pass's limit: the call
-    runs on the exact engine, as before."""
+    """f = 1e-9 is below the sliced pass's interval margin: the call runs on the exact engine at every width."""
     from nabo_b200 import synth
-    q = synth.pc_mixture(300, 100, seed=7)
-    r = synth.pc_mixture(3000, 100, seed=8)
-    _, _, st = fast_vs_exact(core, q, r, 8, 1e-9)
-    assert st["rows_exact_fallback"] == len(q) and st["kernel_launches"] == 1, st
+    for g in (20, 50, 100):
+        q = synth.pc_mixture(300, g, seed=7)
+        r = synth.pc_mixture(3000, g, seed=8)
+        _, _, st = fast_vs_exact(core, q, r, 8, 1e-9)
+        assert st["rows_exact_fallback"] == len(q) and st["kernel_launches"] == 1, (g, st)

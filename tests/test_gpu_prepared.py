@@ -1,8 +1,9 @@
 """Prepared references (core.prepare_reference / nabo_ref_prepare + nabo_knn_prepared): one reference packed once
 serves many query batches, and every result is bit-identical to core.knn with the raw rows and to the exact engine -
-indices, FP64 distances, tie and NaN order - across both tensor-core tile plans, the sliced and the two-phase
-Canberra passes, the exact-engine branch, every batch schedule (reference split, one wave, balanced cuts, several
-waves), masks, drop_first, idx_offset, routed output, and queries far outside the reference's scale."""
+indices, FP64 distances, tie and NaN order - across both tensor-core tile plans, the sliced Canberra pass, the
+exact-engine branches (k beyond the fast plans, a vanishing dist_factor), every batch schedule (reference split, one
+wave, balanced cuts, several waves), masks, drop_first, idx_offset, routed output, and queries far outside the
+reference's scale."""
 import ctypes as C
 
 import numpy as np
@@ -72,12 +73,12 @@ def test_canberra_prepared_serves_several_batches(core, synth, g):
     mask = np.random.default_rng(g).random(m) < 0.1
     for msk in (None, mask):
         pr = core.prepare_reference(r, "mod_canberra", msk)
-        for f in (0.25, 1e-7):                                       # sliced pass / FP16 two-phase pass
+        for f in (0.25, 1e-7):                                       # sliced pass / exact engine
             for i, (n, k) in enumerate([(1, 30), (500, 1), (2500, 30), (1200, 88)]):
                 q = queries(synth, n, g, 200 + i)
                 st = check_batch(core, q, r, pr, k, "mod_canberra", f=f, mask=msk)
-                if k == 88:
-                    assert st["rows_exact_fallback"] == n, st         # past the fast plan: the exact engine
+                if k == 88 or f < 1e-6:
+                    assert st["rows_exact_fallback"] == n, st         # past the fast plan or its f: the exact engine
             check_batch(core, r[:300], r, pr, 30, "mod_canberra", f=f, mask=msk, drop_first=True, idx_offset=7)
 
 

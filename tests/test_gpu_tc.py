@@ -175,8 +175,8 @@ def test_fallback_paths(core, n_bad):
 
 @pytest.mark.parametrize("f", [0.05, 0.25, 1.5])
 def test_canberra_threshold_adversarial(core, f):
-    """Modified Canberra fast path: phase 1 counts unsaturated dimensions in FP16 with a widened threshold and
-    phase 2 scores in FP32; both must stay LOWER bounds.  References are built so that, for their query, most
+    """Modified Canberra fast path: the sliced pass over-counts unsaturated dimensions over widened bin intervals
+    and scores the survivors in FP32; both must stay LOWER bounds.  References are built so that, for their query, most
     dimensions sit within 1e-3 .. 1e-7 (relative) of the saturation boundary |x-y| = f|x|, with column
     magnitudes from 1e-6 to 1e5 and a few zeros / tiny values; a violated bound would drop a true neighbour."""
     rng = np.random.default_rng(int(f * 100))
@@ -209,10 +209,10 @@ def test_canberra_threshold_adversarial(core, f):
     (5000, 30000, 25, 10, 0.25),       # config-1 width
     (4800, 20000, 50, 30, 0.5),        # 150 query groups: every SM gets one or two
     (700, 9000, 56, 20, 0.25),         # widest g of the sliced pass
-    (700, 9000, 64, 20, 0.25),         # past it: FP16 two-phase pass
-    (300, 3000, 80, 8, 2.0),           # g > 64: exact engine; f > 1 (intervals straddle zero)
+    (700, 9000, 64, 20, 0.25),         # past it: the wide plan
+    (300, 3000, 80, 8, 2.0),           # wide plan; f > 1 (intervals straddle zero)
     (300, 3000, 40, 8, 2.0),
-    (300, 3000, 20, 8, 1e-9),          # vanishing dist_factor: FP16 two-phase pass (margin of the sliced pass too thin)
+    (300, 3000, 20, 8, 1e-9),          # vanishing dist_factor: exact engine (margin of the sliced pass too thin)
     (300, 3000, 20, 8, 1e-4),
 ])
 def test_canberra_sliced_shapes(core, n, m, g, k, f):

@@ -13,16 +13,17 @@ EWORKSPACE = -2
 
 # (name, metric, g, n_query, n_ref, k, dist_factor, kernel launches per drop_first (one-shot, prepared)).  The launch
 # counts tell the paths apart: the tensor-core pass counts its preparation (6, or 3 with a prepared reference), the
-# emit kernel and the threshold reduction of a split call; the sliced pass reports 10, the two-phase pass 11 and the
-# exact engine 1.
+# emit kernel and the threshold reduction of a split call; the sliced pass reports 10 and the exact engine 1.  A call
+# that runs the exact engine for every drop_first needs no workspace, so its prepared size is 0.
 CASES = [
     ("tc_fused", "euclidean", 50, 3001, 6000, 30, 0.25, {0: (10, 7), 1: (10, 7)}),
     ("tc_emit", "cosine", 50, 3001, 20011, 60, 0.25, {0: (11, 8), 1: (11, 8)}),
     ("tc_split", "euclidean", 50, 300, 100000, 30, 0.25, {0: (12, 9), 1: (12, 9)}),
     ("sliced", "mod_canberra", 50, 3001, 6000, 30, 0.25, {0: (10, 10), 1: (10, 10)}),
     ("sliced_split", "mod_canberra", 50, 300, 100000, 30, 0.25, {0: (10, 10), 1: (10, 10)}),
-    ("two_phase", "mod_canberra", 50, 3001, 20011, 30, 1e-7, {0: (11, 11), 1: (11, 11)}),
-    # k + drop_first = 57 is past both Canberra passes: drop_first runs the exact engine on a workspace sized for the
+    # dist_factor < 1e-6 runs the exact engine; the one-shot size (which has no dist_factor) is still the sliced carve
+    ("vanishing_f", "mod_canberra", 50, 3001, 20011, 30, 1e-7, {0: (1, 1), 1: (1, 1)}),
+    # k + drop_first = 57 is past the sliced pass: drop_first runs the exact engine on a workspace sized for the
     # sliced pass that the same k takes without it
     ("exact", "mod_canberra", 50, 2001, 20011, 56, 0.25, {0: (10, 10), 1: (1, 1)}),
 ]
@@ -49,8 +50,11 @@ def test_workspace_is_exact_on_every_path(core, case):
     st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
     full = int(L.nabo_knn_workspace_bytes(n, m, g, k, mi, 1))
     prep = int(L.nabo_knn_prepared_workspace_bytes(n, C.byref(pr.desc), k, f, 1))
-    assert 0 < prep <= full
-    if case[0] not in ("two_phase", "exact"):
+    if case[0] == "vanishing_f":
+        assert prep == 0 and full > 0
+    else:
+        assert 0 < prep <= full
+    if case[0] not in ("vanishing_f", "exact"):
         assert prep < full                              # the prepared operands replace the reference's share
     ws = torch.empty(full, dtype=torch.uint8, device="cuda")
     stats = (C.c_int64 * 8)()
@@ -75,4 +79,5 @@ def test_workspace_is_exact_on_every_path(core, case):
             assert stats[3] == nl, (call.__name__, drop_first, list(stats))
             assert torch.equal(idx, ei) and torch.equal(dst.view(torch.int64), ed.view(torch.int64)), \
                 (call.__name__, drop_first)
-            assert call(nbytes - 1, drop_first) == EWORKSPACE, (call.__name__, drop_first)
+            if nbytes > 0:
+                assert call(nbytes - 1, drop_first) == EWORKSPACE, (call.__name__, drop_first)
