@@ -36,10 +36,27 @@ extern "C" {
 
 /* metric ids.  Reference dispatch: euclidean when the query set IS the reference
  * (intra_ref), modified Canberra otherwise (nabo/_mapping.py:119-124, 433-440).
- * Cosine and query!=reference Euclidean are extensions (BASELINE.json). */
+ * Cosine, correlation and query!=reference Euclidean are extensions (BASELINE.json).
+ *
+ * NABO_CORRELATION is Pearson correlation distance (scipy's and scanpy's `correlation`): the cosine distance of the
+ * row-centred vectors.  For a row x (its first g columns):
+ *   s   = x_0 + x_1 + ... + x_{g-1}     sequential, ascending k, from 0.0
+ *   mu  = s / g
+ *   c_k = x_k - mu
+ *   d(x, y) = 1 - dot(c_x, c_y) / (sqrt(|c_x|^2) * sqrt(|c_y|^2)), dot and norms in ascending k with separate
+ *             multiplies and adds (the cosine arithmetic, on the centred rows)
+ * Range [0, 2] up to rounding (parallel rows can land a few ulps below 0, as under cosine).  A NaN or +-inf
+ * coordinate makes the row's centred copy non-finite, so every distance from it is NaN.
+ * A constant row whose sum is exact (every row at g = 1) centres to zero and every distance from it is NaN, like a
+ * zero row under cosine; NaN distances sort last.  scipy sums in another order and agrees to rounding only.
+ * The kNN entry points centre the queries and the reference once per call into the head of the workspace (a
+ * prepared reference keeps its centred copy in its buffer) and then run the cosine engines on the copies.
+ * nabo_knn_candidates and nabo_rerank_exact take rows as given and refuse NABO_CORRELATION: pass centred rows with
+ * NABO_COSINE instead. */
 #define NABO_EUCLIDEAN 0
 #define NABO_MOD_CANBERRA 1
 #define NABO_COSINE 2
+#define NABO_CORRELATION 3
 
 /* kNN engines */
 #define NABO_MODE_EXACT 0 /* FP64 brute force in the reference's arithmetic order */
@@ -62,6 +79,9 @@ int nabo_mod_canberra_dist(const double* x, int ldx, const double* y, int ldy, d
                            int m, int n, int g, double f, void* stream);
 int nabo_cosine_dist(const double* x, int ldx, const double* y, int ldy, double* d, int ldd,
                      int m, int n, int g, void* stream);
+/* Pearson correlation distance (NABO_CORRELATION above); same contract as nabo_cosine_dist. */
+int nabo_correlation_dist(const double* x, int ldx, const double* y, int ldy, double* d, int ldd,
+                          int m, int n, int g, void* stream);
 
 /* ---- (2) fused distance + per-query top-k: replaces _calc_dist ------------------
  * nabo/_mapping.py:48-148, restricted to what _calc_snn consumes ([:k] of every
@@ -78,13 +98,17 @@ int nabo_cosine_dist(const double* x, int ldx, const double* y, int ldy, double*
  *              brute-force engine, [2] candidates kept per row, [3] kernels launched,
  *              [4] ns spent in the dominant distance/top-k kernel (CUDA events on
  *              `stream`), [5] ns in the exact re-rank, [6] ns in the exact fallback,
- *              [7] ns in operand preparation.
+ *              [7] ns in operand preparation (correlation adds its centring launches to
+ *              [7] and counts them in [3]).
  *   mode = NABO_MODE_FAST runs the candidate pass + re-rank where a fast plan exists, and
  *   the exact engine (same results) elsewhere; ksel = k + drop_first:
  *     Euclidean / cosine  1 <= g <= 128, ksel <= 128 (tensor-core pass: 128-key buffers for
- *                         ksel + 8 <= 96, 256-key buffers for 89 <= ksel <= 128)
+ *     / correlation       ksel + 8 <= 96, 256-key buffers for 89 <= ksel <= 128)
  *     modified Canberra   ksel + 8 <= 64, g <= 128, dist_factor >= 1e-6 (bit-sliced pass);
  *                         dist_factor < 1e-6: exact engine
+ *   Workspace: nabo_knn_workspace_bytes.  Correlation adds the centred copies of the queries and the
+ *   reference (n_query * g + n_ref * g doubles, each region 256-byte aligned) to the cosine size, in
+ *   exact mode too (the exact mode of every other metric needs 256 bytes).
  */
 size_t nabo_knn_workspace_bytes(int n_query, int n_ref, int g, int k, int metric, int mode);
 int nabo_knn(const double* q, int ldq, const double* r, int ldr, int n_query, int n_ref, int g,
@@ -147,6 +171,10 @@ int nabo_knn_routed(const double* q, int ldq, const double* r, int ldr, int n_qu
  * is bit-identical to nabo_knn / nabo_knn_routed on the same inputs (the exact re-rank, the certificate and the
  * exact fallback decide every row).  The descriptor keeps the caller's FP64 rows and mask by address (the re-rank
  * and the fallback read them): both, and the buffer, must stay allocated and unchanged while it is in use.
+ * Correlation is the exception for the rows: the buffer starts with their centred FP64 copy (n_ref x g), which the
+ * descriptor's r points at (ldr = g), followed by the tensor-core operands of that copy as cosine; the caller's
+ * rows are not read after nabo_ref_prepare.  A call then centres only the queries (workspace: their copy + the
+ * cosine size).
  *
  * The tensor-core scale of a prepared reference comes from the reference's largest norm alone (cosine: 32), not
  * from the queries: a query whose scaled coordinates would overflow FP16 (about 500x the largest reference norm)
@@ -157,13 +185,14 @@ int nabo_knn_routed(const double* q, int ldq, const double* r, int ldr, int n_qu
  * Status: a descriptor that was not filled by nabo_ref_prepare or does not match its buffer -> NABO_EINVAL; another
  * ABI version, a metric / g without a fast plan (1 <= g <= 128) or k + drop_first > 128 -> NABO_EUNSUPPORTED. */
 #define NABO_PREPARED_MAGIC 0x5250424eu   /* "NBPR" */
-#define NABO_PLAN_TC 1                     /* tensor-core operands (Euclidean, cosine)   */
+#define NABO_PLAN_TC 1                     /* tensor-core operands (Euclidean, cosine, correlation) */
 #define NABO_PLAN_SLICED 2                 /* bit-sliced operands (modified Canberra)    */
 typedef struct nabo_prepared_ref {
     uint32_t magic;            /* NABO_PREPARED_MAGIC                                        */
     int abi_version;           /* NABO_ABI_VERSION of the library that prepared it           */
     int n_ref, g, metric, plan;
-    const double* r;           /* the caller's FP64 rows (n_ref x g, row stride ldr)         */
+    const double* r;           /* the caller's FP64 rows (n_ref x g, row stride ldr); correlation: the centred copy
+                                  at the start of buffer (ldr = g)                              */
     int ldr;
     const uint8_t* ref_mask;   /* the caller's mask or NULL                                  */
     void* buffer;              /* the caller's buffer (nabo_ref_prepared_bytes)              */
@@ -172,7 +201,8 @@ typedef struct nabo_prepared_ref {
 } nabo_prepared_ref;
 
 /* device bytes of the prepared operands; 0 when metric / g have no fast plan.  Tensor-core plan: 128-row tiles of
- * 2 * ceil16(3g + 3) bytes per row (320 B per row at g = 50) + 8 B per row. */
+ * 2 * ceil16(3g + 3) bytes per row (320 B per row at g = 50) + 8 B per row; correlation adds the centred copy
+ * (8g bytes per row, 256-byte aligned) in front. */
 size_t nabo_ref_prepared_bytes(int n_ref, int g, int metric);
 int nabo_ref_prepare(const double* r, int ldr, int n_ref, int g, int metric, const uint8_t* ref_mask, void* buffer,
                      size_t buffer_bytes, nabo_prepared_ref* prepared_host, void* stream);

@@ -16,8 +16,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("NABO_B200_LIB") or os.path.join(HERE, "libnabo_b200.so")   # override: A/B builds (tools/)
 HEADER = os.path.join(os.path.dirname(HERE), "include", "nabo_b200.h")
 
-EUCLIDEAN, MOD_CANBERRA, COSINE = 0, 1, 2
-METRICS = {"euclidean": EUCLIDEAN, "mod_canberra": MOD_CANBERRA, "cosine": COSINE}
+EUCLIDEAN, MOD_CANBERRA, COSINE, CORRELATION = 0, 1, 2, 3
+METRICS = {"euclidean": EUCLIDEAN, "mod_canberra": MOD_CANBERRA, "cosine": COSINE, "correlation": CORRELATION}
 MODE_EXACT, MODE_FAST = 0, 1
 
 _p = C.c_void_p
@@ -42,6 +42,7 @@ SIGNATURES: Dict[str, tuple] = {
     "nabo_euclidean_dist": (_i, [_p, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
     "nabo_mod_canberra_dist": (_i, [_p, _i, _p, _i, _p, _i, _i, _i, _i, _d, _p]),
     "nabo_cosine_dist": (_i, [_p, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
+    "nabo_correlation_dist": (_i, [_p, _i, _p, _i, _p, _i, _i, _i, _i, _p]),
     "nabo_knn_workspace_bytes": (_z, [_i, _i, _i, _i, _i, _i]),
     "nabo_knn": (_i, [_p, _i, _p, _i, _i, _i, _i, _i, _i, _d, _p, _i, _i, _i, _p, _p, _p, _z,
                       C.POINTER(C.c_int64), _p]),

@@ -16,7 +16,7 @@ import torch
 
 from ._lib import METRICS, MODE_EXACT, MODE_FAST, PreparedDesc, check, lib, require_device
 
-__all__ = ["euclidean_dist", "mod_canberra_dist", "cosine_dist", "knn", "prepare_reference", "PreparedReference", "knn_candidates", "rerank_exact", "merge_topk",
+__all__ = ["euclidean_dist", "mod_canberra_dist", "cosine_dist", "correlation_dist", "knn", "prepare_reference", "PreparedReference", "knn_candidates", "rerank_exact", "merge_topk",
            "merge_topk_parts", "snn_int_weights", "score_accumulate", "scores_finalize", "snn_weight_lut", "fix_weight", "snn_weights", "mapping_scores", "classify_targets", "mapping_specificity", "sparse_row_stats", "connected_components",
            "project", "project_csr", "scale_counts", "map_cells", "map_cells_host", "resolve_metric"]
 
@@ -124,6 +124,13 @@ def cosine_dist(x, y, d=None):
     return _dist("nabo_cosine_dist", x, y, d, None)
 
 
+def correlation_dist(x, y, d=None):
+    """Extension metric: Pearson correlation distance, the cosine distance of the row-centred vectors (each row
+    minus its mean, summed sequentially in FP64; see NABO_CORRELATION in include/nabo_b200.h).  Constant rows give
+    NaN, like zero rows under cosine."""
+    return _dist("nabo_correlation_dist", x, y, d, None)
+
+
 # ----------------------------------------------------------------------------- (2) kNN
 PREPARED_MAX_G = 128      # widest PCA space with a prepared form (the fast plans' limit, nabo_ref_prepared_bytes)
 
@@ -133,7 +140,8 @@ class PreparedReference:
     of the fast engine for one (rows, g, metric, mask) in a device buffer this object owns, plus the FP64 rows and
     the mask it keeps on the device (the exact re-rank and fallback read them).  Results are bit-identical to
     ``knn`` with the raw rows.  Device memory: the packed tensor-core tiles take 2 * ceil16(3g + 3) bytes per
-    reference (about 31 MB per 100 k references at g = 50); see ``nbytes``.
+    reference (about 31 MB per 100 k references at g = 50); correlation adds the centred FP64 copy of the rows
+    (8g bytes per reference), which the calls read instead of ``r``; see ``nbytes``.
 
     The rows must not change while the object is in use: a CUDA tensor passed in (or the float64 copy made of
     it) that is modified in place afterwards makes every later call raise ``ValueError``.  NumPy input is copied
@@ -310,9 +318,17 @@ def _knn_routed(qd, rd, n, m, g, k, metric, dist_factor, md, drop_first, idx_off
     return (None, None, _stats_dict(stats)) if return_stats else (None, None)
 
 
+def _rows_as_given(metric: str, what: str) -> None:
+    if metric == "correlation":
+        raise ValueError("ERROR: %s takes rows as given and has no correlation form; centre the rows and pass "
+                         "metric='cosine'" % what)
+
+
 def knn_candidates(q, r, k: int, metric: str = "euclidean", ref_mask=None, drop_first: bool = False):
     """Tensor-core candidate pass alone (Euclidean / cosine).  Returns dict(cand int32 (N,K'),
-    tau float32 (N,), qn2 float64 (N,), scal float64 (4,)); see include/nabo_b200.h."""
+    tau float32 (N,), qn2 float64 (N,), scal float64 (4,)); see include/nabo_b200.h.  Rows are taken as
+    given: for correlation, pass row-centred rows with ``metric="cosine"``."""
+    _rows_as_given(metric, "knn_candidates")
     require_device()
     host = _is_host(q, r)
     qd, rd = _dev(q, torch.float64), _dev(r, torch.float64)
@@ -335,7 +351,9 @@ def knn_candidates(q, r, k: int, metric: str = "euclidean", ref_mask=None, drop_
 
 def rerank_exact(q, r, cand, k: int, metric: str = "euclidean", dist_factor: float = 0.25, ref_mask=None,
                  drop_first: bool = False, idx_offset: int = 0):
-    """Exact FP64 re-rank (reference arithmetic order) of caller-supplied candidates."""
+    """Exact FP64 re-rank (reference arithmetic order) of caller-supplied candidates.  Rows are taken as given:
+    for correlation, pass row-centred rows with ``metric="cosine"``."""
+    _rows_as_given(metric, "rerank_exact")
     require_device()
     host = _is_host(q, r, cand)
     qd, rd = _dev(q, torch.float64), _dev(r, torch.float64)

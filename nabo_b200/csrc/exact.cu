@@ -106,7 +106,17 @@ __global__ void __launch_bounds__(NT) dist_tile_kernel(const double* __restrict_
     load_tile_kmajor(xs, x, ldx, q0, m, g, nullptr);
     load_tile_kmajor(ys, y, ldy, r0, n, g, nullptr);
     __syncthreads();
-    if (METRIC == NABO_COSINE) {
+    // correlation = cosine of the centred rows: one thread per tile row (padding rows included) centres it in place
+    constexpr bool COS_LIKE = METRIC == NABO_COSINE || METRIC == NABO_CORRELATION;
+    if (METRIC == NABO_CORRELATION && threadIdx.x < TQ + TR) {
+        double* col = threadIdx.x < TQ ? xs + threadIdx.x : ys + (threadIdx.x - TQ);
+        double s = 0.0;
+        for (int k = 0; k < g; ++k) s = __dadd_rn(s, col[k * LDS_T]);
+        const double mu = __ddiv_rn(s, (double)g);
+        for (int k = 0; k < g; ++k) col[k * LDS_T] = __dsub_rn(col[k * LDS_T], mu);
+    }
+    if (METRIC == NABO_CORRELATION) __syncthreads();
+    if (COS_LIKE) {
         if (threadIdx.x < TQ) {
             double s = 0.0;
             for (int k = 0; k < g; ++k) { double v = xs[k * LDS_T + threadIdx.x]; s = __dadd_rn(s, __dmul_rn(v, v)); }
@@ -144,8 +154,8 @@ __global__ void __launch_bounds__(NT) dist_tile_kernel(const double* __restrict_
         for (int b = 0; b < 4; ++b) {
             int rj = r0 + tr * 4 + b;
             if (rj < n) {
-                double nq = METRIC == NABO_COSINE ? nqs[tq * 4 + a] : 0.0;
-                double nr = METRIC == NABO_COSINE ? nrs[tr * 4 + b] : 0.0;
+                double nq = COS_LIKE ? nqs[tq * 4 + a] : 0.0;
+                double nr = COS_LIKE ? nrs[tr * 4 + b] : 0.0;
                 d[(long long)qi * ldd + rj] = Pair<METRIC>::finish(acc[a][b], nq, nr);
             }
         }
@@ -180,6 +190,10 @@ extern "C" int nabo_mod_canberra_dist(const double* x, int ldx, const double* y,
 extern "C" int nabo_cosine_dist(const double* x, int ldx, const double* y, int ldy, double* d, int ldd,
                                 int m, int n, int g, void* stream) {
     return launch_dist_tiles<NABO_COSINE>(x, ldx, y, ldy, d, ldd, m, n, g, 0.0, (cudaStream_t)stream);
+}
+extern "C" int nabo_correlation_dist(const double* x, int ldx, const double* y, int ldy, double* d, int ldd,
+                                     int m, int n, int g, void* stream) {
+    return launch_dist_tiles<NABO_CORRELATION>(x, ldx, y, ldy, d, ldd, m, n, g, 0.0, (cudaStream_t)stream);
 }
 
 // ------------------------------------------------------------------ (2) brute force + fused top-k
@@ -644,15 +658,17 @@ __device__ __forceinline__ double cert_lower_bound(const NaboCert& c, int qi, fl
     const double qn = sqrt(qn2);
     const double eps = c.c_acc * (4.0 * qn * rmax + rmax * rmax + qn2);       // accumulation error (scaled^2)
     const double l2 = (double)tau + qn2 - eps;
-    if (!(l2 > 0.0)) return 0.0;
     if (c.kind == NABO_CERT_EUCLID) {
+        if (!(l2 > 0.0)) return 0.0;
         // |d~ - d| <= 2^-21 (|q| + |r|) from the two-term FP16 split of the inputs
         return sqrt(l2) * sc_inv * (1.0 - 1e-7) - (9.6e-7 * (qn + rmax) + c.abs_slack) * sc_inv;
     }
-    // cosine: unit vectors, chord e -> distance e^2 / 2
-    double e = sqrt(l2) * sc_inv - 1.0e-6;
-    if (!(e > 0.0)) return 0.0;
-    return 0.5 * e * e * (1.0 - 1e-9);
+    // cosine: unit vectors, chord e -> distance e^2 / 2.  The FP64 distance 1 - dot / (|q| |r|) itself lies up to
+    // (g + 5) 2^-53 below the true one (below zero for parallel vectors, e.g. every centred row at g = 2 under
+    // correlation), so the bound keeps 1e-12 below it: a non-candidate at a rounded-down distance cannot pass.
+    double e = l2 > 0.0 ? sqrt(l2) * sc_inv - 1.0e-6 : 0.0;
+    if (!(e > 0.0)) e = 0.0;
+    return 0.5 * e * e * (1.0 - 1e-9) - 1e-12;
 }
 
 // acc[u] = sum over the dimensions of the pair terms of (x, row jj[u] of r), u < NU, all slots in one sweep over the

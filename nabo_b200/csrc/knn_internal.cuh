@@ -200,6 +200,10 @@ int nabo_knn_fast(const double* q, int ldq, const double* r, int ldr, int n_quer
                   double* out_dist, const NaboRoute& route, void* workspace, size_t workspace_bytes,
                   int64_t* stats_host, cudaStream_t st, const NaboFastRef* pre = nullptr);
 
+// Correlation metric (correlation.cu): out (n x g, contiguous) = the rows of x (stride ld) minus their means, in the
+// arithmetic the header pins.  One launch.
+int nabo_centre_rows(const double* x, int ld, int n, int g, double* out, cudaStream_t st);
+
 // CUDA-event stage timer, active only when the caller asked for stats (stats_host != NULL).
 // Usage: begin(); <launch stage 0>; end(0); <launch stage 1>; end(1); ... sync; ns(i).
 struct NaboStageTimer {

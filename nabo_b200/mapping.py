@@ -17,8 +17,9 @@ same exceptions, same mapping-file group names (``name_stash``, ``ref_cells``,
 * ``chunk_size`` is accepted and validated but has no effect (results never depended on
   it, :106-128);
 * new keyword-only extensions with reference-preserving defaults: ``metric`` (None ->
-  Euclidean for the reference graph, modified Canberra for targets, :433-440) and
-  ``mode`` ('fast' | 'exact').
+  Euclidean for the reference graph, modified Canberra for targets, :433-440; or any of
+  'euclidean', 'mod_canberra', 'cosine', 'correlation' - Pearson correlation distance, scanpy's
+  and scipy's ``correlation``) and ``mode`` ('fast' | 'exact').
 """
 from __future__ import annotations
 
@@ -192,7 +193,8 @@ class Mapping:
     def _prepared_ref(self, metric: str, ignore_ref_cells: List[str], mask) -> Optional["core.PreparedReference"]:
         """The reference packed for (use_comps, metric, ignore_ref_cells), kept between calc_dist calls so that
         mapping several targets uploads and packs the reference once.  One is kept at a time (its device memory:
-        the FP64 rows plus about 31 MB per 100 k references at use_comps = 50).  None where no prepared form
+        the FP64 rows plus about 31 MB per 100 k references at use_comps = 50, and for correlation the centred
+        copy of the rows, 40 MB per 100 k references at use_comps = 50).  None where no prepared form
         exists (use_comps > core.PREPARED_MAX_G): the call then takes the host matrix."""
         key = (self._useComps, metric, frozenset(ignore_ref_cells))
         if self._refPrepCache is not None and self._refPrepCache[0] == key:
